@@ -2,7 +2,7 @@
 """bench.py -- ARF-filtered frames/s of the B200 temporal filter (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload 4k10_n15|1080p10_n11|1080p8_n7]
-                    [--mode windows|slab] [--impl tfgpu|reference]
+                    [--mode windows|slab] [--impl tfgpu|reference] [--dump-outputs DIR]
 
 A step = one pass of the hot path over one ARF window = one filtered output frame
 per GPU (mode windows, weak scaling: independent windows per GPU, no collective) or
@@ -22,6 +22,14 @@ slab, strong scaling).  Prints ONE JSON line (rank 0).
 
 --impl reference times the reference's own CPU implementation on all host cores (row
 sharding across processes, the reference's own MT axis: av1/encoder/ethread.c:2062-2189).
+
+--dump-outputs DIR writes, after the timed steps, what every context's last timed step returned:
+DIR/ctx<c>_{y,u,v}.npy (the filtered planes, whole 32x32 blocks, float32) and DIR/ctx<c>_frame_diff.npy
+(FRAME_DIFF sum and sse, float64); with several ranks the names start with rank<r>_.  In slab mode on several
+GPUs rank 0 writes the frame the gather assembled and the all-reduced FRAME_DIFF: DIR/frame_{y,u,v,diff}.npy
+(--impl tfgpu only: the reference arm times block-row samples and returns no frame).  The inputs are seeded,
+so two builds run with the same arguments can be compared file for file.  Above 64 MB in all, each plane is
+cut to the same fixed sample of its samples in every run (see write_outputs).
 """
 import argparse
 import importlib.util
@@ -81,6 +89,32 @@ def make_window(width, height, bd, n, seed):
 def plane_bytes(width, height, bd):
     es = 2 if bd > 8 else 1
     return (width * height + 2 * ((width + 1) // 2) * ((height + 1) // 2)) * es
+
+
+DUMP_LIMIT_BYTES = 64_000_000
+SMALL = 4096  # arrays of at most this many elements are always written whole
+
+
+def write_outputs(path, arrays, limit=DUMP_LIMIT_BYTES):
+    """Writes {name: integer array} as path/<name>.npy: 8- and 16-bit samples in float32, wider integers
+    (FRAME_DIFF) in float64, both exact.  When that would exceed `limit` bytes in all, every larger array
+    is cut to the same share of its elements, flattened: sorted flat indices drawn by
+    numpy.random.default_rng(0), so every run with the same arguments keeps the same positions."""
+    out = {}
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        out[name] = a.astype(np.float32 if a.dtype.itemsize <= 2 else np.float64)
+    small = sum(a.nbytes for a in out.values() if a.size <= SMALL)
+    big = sum(a.nbytes for a in out.values() if a.size > SMALL)
+    if small + big > limit:
+        share = (limit - small - 256 * len(out)) / big  # 256: room for each .npy header
+        for name, a in out.items():
+            if a.size > SMALL:
+                idx = np.sort(np.random.default_rng(0).choice(a.size, int(a.size * share), replace=False))
+                out[name] = a.ravel()[idx]
+    os.makedirs(path, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 # ---------------------------------------------------------------------------------------
@@ -355,7 +389,12 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--concurrent", type=int, default=0,
                     help="independent windows in flight per GPU (contexts); 0 = auto: 3 for 4K, 4 below")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned as DIR/*.npy (--impl tfgpu; "
+                         "the reference arm times block-row samples in worker processes and returns no frame)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "tfgpu":
+        ap.error("--dump-outputs needs --impl tfgpu: the reference arm times block-row samples and returns no frame")
     args.warmup = max(args.warmup, 3) if args.impl == "tfgpu" else args.warmup
     wl = args.workload
     if args.impl == "reference":
@@ -435,12 +474,13 @@ def main():
             dist.barrier()
 
     slab_win = sharding.SlabWindow(mb_rows, world, rank) if slab else None
+    last_gather = [None, None]  # slab mode: rank 0's gathered slabs and the all-reduced FRAME_DIFF of the last step
 
     def slab_gather(diff):
         """NCCL gather of the disjoint output row slabs to rank 0 and a 16-byte all-reduce of
         FRAME_DIFF (SURVEY 8e; integer sums, so order independent like ethread.c:2161-2173)."""
         d = torch.from_numpy(diff.copy()).to(f"cuda:{local}")
-        slab_win.gather(slab_win.device_slabs(ctx, torch, f"cuda:{local}"), d, dist, torch)
+        last_gather[:] = slab_win.gather(slab_win.device_slabs(ctx, torch, f"cuda:{local}"), d, dist, torch)
         torch.cuda.current_stream().synchronize()
 
     ids = [[b.frame_id for b in bufs] for _, bufs in windows]
@@ -449,11 +489,13 @@ def main():
 
     pending = [False] * conc
     call_ms = [0.0] * conc
+    last_diff = [None] * conc
 
     def harvest(ci):
         nonlocal launches
         m, diff = ctxs[ci].filter_resident_result()
         pending[ci] = False
+        last_diff[ci] = diff
         call_ms[ci] += m
         launches += ctxs[ci].last_stats()[0]
         if ci == 0:
@@ -506,6 +548,27 @@ def main():
     # flight, must equal the same window filtered synchronously on an otherwise idle device --------------
     import hashlib
     vout = pkg.Yv12Buffer(width, height, 1, 1, use_hbd, p["border"])
+
+    if args.dump_outputs and slab:
+        if rank == 0:  # the frame the gather assembled, as measure_slab() reads it back
+            pitches = [ctx.output_device_plane(pl)[1] for pl in range(3)]
+            planes = slab_win.assemble(last_gather[0], pitches, torch.cat)
+            dumped = {}
+            for pl, plane in enumerate("yuv"):
+                want = vout.full_blocks(pl)
+                rows = planes[pl].cpu().numpy()[:, :want.shape[1] * want.itemsize]
+                dumped[f"frame_{plane}"] = np.ascontiguousarray(rows).view(want.dtype)
+            dumped["frame_diff"] = last_gather[1].cpu().numpy()
+            write_outputs(args.dump_outputs, dumped)
+    elif args.dump_outputs:
+        dumped = {}
+        prefix = f"rank{rank}_" if world > 1 else ""
+        for ci, c in enumerate(ctxs):
+            c.download_output(vout)
+            for pl, plane in enumerate("yuv"):
+                dumped[f"{prefix}ctx{ci}_{plane}"] = vout.full_blocks(pl).copy()
+            dumped[f"{prefix}ctx{ci}_frame_diff"] = last_diff[ci]
+        write_outputs(args.dump_outputs, dumped, DUMP_LIMIT_BYTES // world)  # every rank writes its share
 
     def out_hash(c):
         c.download_output(vout)
@@ -716,7 +779,7 @@ def main():
 
     slab_section = None
     if world > 1 and not slab and width >= 3000:
-        slab_section = measure_slab(max(args.steps, 30))
+        slab_section = measure_slab(args.steps)
 
     if rank != 0:
         if world > 1:

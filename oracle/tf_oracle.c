@@ -124,6 +124,27 @@ int tfo_get_plane_with_border(tfo_ctx *c, int idx, int plane, uint16_t *dst, int
   if (dst) memcpy(dst, f->alloc[plane], (size_t)f->rows[k] * f->stride[k] * 2);
   return f->stride[k];
 }
+/* aom_extend_frame_borders_c -> extend_frame(ybf, ybf->border) (yv12extend.c): every plane replicated from
+ * its crop area, top/left by the border, bottom/right by the border plus aligned - crop */
+void tfo_extend_output_borders(tfo_ctx *c) {
+  frame_t *f = &c->out;
+  for (int pl = 0; pl < c->num_planes; pl++) {
+    const int k = pl > 0;
+    const int w = f->crop_w[k], h = f->crop_h[k], st = f->stride[k];
+    const int et = f->bh[k], el = f->bw[k];
+    const int eb = et + f->ah[k] - h, er = el + f->aw[k] - w;
+    uint16_t *dst = f->buf[pl];
+    for (int y = 0; y < h; y++) {
+      uint16_t *row = dst + (size_t)y * st;
+      for (int x = 1; x <= el; x++) row[-x] = row[0];
+      for (int x = 0; x < er; x++) row[w + x] = row[w - 1];
+    }
+    const int linesize = el + er + w;
+    for (int y = 1; y <= et; y++) memcpy(dst - (size_t)y * st - el, dst - el, linesize * 2);
+    for (int y = 0; y < eb; y++)
+      memcpy(dst + (size_t)(h + y) * st - el, dst + (size_t)(h - 1) * st - el, linesize * 2);
+  }
+}
 int tfo_plane_alloc_size(tfo_ctx *c, int plane) {
   const int k = plane > 0;
   return c->frames[0].rows[k] * c->frames[0].stride[k];
@@ -842,9 +863,9 @@ static unsigned subpel_search(const search_t *s, mv_t start_full, mv_t *best) {
 
 /* av1_set_mv_{row,col}_limits mcomp.h:216-240 + av1_set_mv_search_range
  * mcomp.c:196-215 with ref_mv = 0 */
-static void set_limits(const tfo_ctx *c, int mb_row, int mb_col, limits_t *l) {
+static void set_limits(const tfo_ctx *c, int mi_row, int mi_col, int mi_size, limits_t *l) {
   const int border = c->p.border;
-  const int mi_row = mb_row * 8, mi_col = mb_col * 8, mih = 8, miw = 8;
+  const int mih = mi_size, miw = mi_size;
   l->row_min = MAXI(-(mi_row * 4 + border - 8), -(((mi_row + mih) * 4) + 8));
   l->row_max = MINI((c->mi_rows - mi_row - mih) * 4 + border - 8, (c->mi_rows - mi_row) * 4 + 8);
   l->col_min = MAXI(-(mi_col * 4 + border - 8), -(((mi_col + miw) * 4) + 8));
@@ -852,6 +873,47 @@ static void set_limits(const tfo_ctx *c, int mb_row, int mb_col, limits_t *l) {
   /* ref_mv = 0: [-1023, 1023] intersect (MV_LOW/8+1.. never binds) */
   l->col_min = MAXI(l->col_min, -1023); l->col_max = MINI(l->col_max, 1023);
   l->row_min = MAXI(l->row_min, -1023); l->row_max = MINI(l->row_max, 1023);
+}
+
+/* tf_motion_search temporal_filter.c:94-130: the search state of one frame pair; returns step_param */
+static int search_setup(const tfo_ctx *c, const sites_t *sites, int stride, search_t *s, int *skip) {
+  const tfo_params *p = &c->p;
+  const int min_frame_size = MINI(p->width, p->height);
+  memset(s, 0, sizeof(*s));
+  s->p = p;
+  s->stride = stride;
+  s->sites = sites;
+  s->min_frame_size = min_frame_size;
+  if (min_frame_size >= 720) { s->sad_lambda = 8; s->sse_lambda = 1; }
+  else if (min_frame_size >= 480) { s->sad_lambda = 15; s->sse_lambda = 0; }
+  else { s->sad_lambda = 32; s->sse_lambda = 2; }
+  /* use_downsampled_sad && block_size_high >= 16: true for both sizes */
+  *skip = p->use_downsampled_sad ? 1 : 0;
+  /* av1_init_search_range mcomp.c:217-226 */
+  int size = MAXI(16, MAXI(p->width, p->height));
+  int step_param = 0;
+  while ((size << step_param) < 1023) step_param++;
+  return MINI(step_param, 9);
+}
+
+void tfo_full_pixel_search(tfo_ctx *c, int src_idx, int ref_idx, int bsize, int x, int y,
+                           int start_row, int start_col, int *out) {
+  sites_t sites;
+  init_nstep(&sites);
+  const frame_t *cur = &c->frames[src_idx], *ref = &c->frames[ref_idx];
+  const int st = cur->stride[0];
+  search_t s;
+  int skip;
+  const int step_param = search_setup(c, &sites, st, &s, &skip);
+  set_limits(c, y >> 2, x >> 2, bsize >> 2, &s.lim);
+  s.src = cur->buf[0] + (size_t)y * st + x;
+  s.ref = ref->buf[0] + (size_t)y * st + x;
+  s.w = s.h = bsize;
+  const mv_t start = { start_row, start_col };
+  mv_t best;
+  out[2] = full_pixel_search(&s, start, step_param, skip, &best);
+  out[0] = best.row;
+  out[1] = best.col;
 }
 
 /* tf_motion_search temporal_filter.c:87-253 */
@@ -862,22 +924,9 @@ static void motion_search(const tfo_ctx *c, const sites_t *sites, const frame_t 
   const int y_offset = mb_row * 32 * st + mb_col * 32;
   const int min_frame_size = MINI(p->width, p->height);
   search_t s;
-  memset(&s, 0, sizeof(s));
-  s.p = p;
-  s.stride = st;
-  s.sites = sites;
-  s.min_frame_size = min_frame_size;
-  if (min_frame_size >= 720) { s.sad_lambda = 8; s.sse_lambda = 1; }
-  else if (min_frame_size >= 480) { s.sad_lambda = 15; s.sse_lambda = 0; }
-  else { s.sad_lambda = 32; s.sse_lambda = 2; }
-  set_limits(c, mb_row, mb_col, &s.lim);
-  /* av1_init_search_range mcomp.c:217-226 */
-  int size = MAXI(16, MAXI(p->width, p->height));
-  int step_param = 0;
-  while ((size << step_param) < 1023) step_param++;
-  step_param = MINI(step_param, 9);
-  /* use_downsampled_sad && block_size_high >= 16: true for both sizes */
-  const int skip = p->use_downsampled_sad ? 1 : 0;
+  int skip;
+  const int step_param = search_setup(c, sites, st, &s, &skip);
+  set_limits(c, mb_row * 8, mb_col * 8, 8, &s.lim);
 
   mv_t start = { rawpel(ref_mv->row), rawpel(ref_mv->col) };
   s.src = cur->buf[0] + y_offset;

@@ -53,6 +53,13 @@ void tfo_get_output(tfo_ctx *c, int plane, uint16_t *dst, int w, int h);
 int tfo_get_plane_with_border(tfo_ctx *c, int idx, int plane, uint16_t *dst, int *rows,
                               int *bw, int *bh);
 int tfo_plane_alloc_size(tfo_ctx *c, int plane);
+/* aom_extend_frame_borders on the output frame (what the caller runs after the filter) */
+void tfo_extend_output_borders(tfo_ctx *c);
+/* av1_full_pixel_search as tf_motion_search() configures it, on the bsize x bsize (16 or 32) luma block
+ * at (x, y) of frame src_idx against frame ref_idx from full-pel start (start_row, start_col):
+ * out = best row, best col, returned variance cost */
+void tfo_full_pixel_search(tfo_ctx *c, int src_idx, int ref_idx, int bsize, int x, int y,
+                           int start_row, int start_col, int *out);
 
 /* av1_apply_temporal_filter_c on caller supplied block data
  * (the call test/temporal_filter_test.cc:210-221 makes). */

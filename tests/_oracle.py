@@ -52,6 +52,8 @@ def lib():
         l.tfo_get_plane_with_border.restype = C.c_int
         l.tfo_get_plane_with_border.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p] + [C.POINTER(C.c_int)] * 3
         l.tfo_plane_alloc_size.argtypes = [C.c_void_p, C.c_int]
+        l.tfo_extend_output_borders.argtypes = [C.c_void_p]
+        l.tfo_full_pixel_search.argtypes = [C.c_void_p] + [C.c_int] * 7 + [C.POINTER(C.c_int)]
         l.tfo_apply_block.argtypes = (
             [C.c_int] * 7 + [C.c_void_p] * 3 + [C.c_int] * 4 + [C.c_void_p] * 3 + [C.c_int] * 2 + [C.c_void_p] * 3)
         l.tfo_sad.restype = C.c_uint
@@ -133,6 +135,16 @@ class OracleFilter:
         assert buf.size == n
         lib().tfo_get_plane_with_border(self.h, idx, plane, _ptr(buf), rows, bw, bh)
         return buf, dict(stride=stride, bw=bw.value, bh=bh.value)
+
+    def extend_output_borders(self):
+        """aom_extend_frame_borders on the output frame; plane_with_border(-1, plane) reads it back."""
+        lib().tfo_extend_output_borders(self.h)
+
+    def full_pixel_search(self, src_idx, ref_idx, bsize, x, y, start_row, start_col):
+        """av1_full_pixel_search() on one block as tf_motion_search() configures it -> (row, col, var)."""
+        out = (C.c_int * 3)()
+        lib().tfo_full_pixel_search(self.h, src_idx, ref_idx, bsize, x, y, start_row, start_col, out)
+        return out[0], out[1], out[2]
 
     def close(self):
         if self.h:

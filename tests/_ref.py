@@ -1,5 +1,5 @@
 """ctypes binding for oracle/_ref/libtf_ref.so (the UNMODIFIED reference compiled
-from /root/reference by oracle/Makefile).  TEST INFRASTRUCTURE ONLY."""
+from the upstream source tree by oracle/Makefile).  TEST INFRASTRUCTURE ONLY."""
 import ctypes as C
 import os
 import numpy as np
@@ -48,8 +48,24 @@ def avx2_lib():
     return _avx2
 
 
+# the upstream source tree oracle/Makefile compiles oracle/_ref from (make REF=<dir>); unset: not available
+SOURCE_DIR = os.environ.get("REF", "")
+
+
 def available():
     return os.path.exists(LIB)
+
+
+def reference_or_oracle(p, frames):
+    """The compiled reference where oracle/_ref is built, else the oracle (oracle/tf_oracle.c).  Both give
+    estimate_noise, run, extend_output_borders, plane_with_border(idx, plane)[0] (the whole padded plane, same
+    layout) and full_pixel_search.  tests/golden/ holds reference outputs of the filter pipeline only: the
+    oracle's per-block search and border extension are pinned to them only where the pipeline exercises them
+    (tests/test_oracle_golden.py), so where oracle/_ref is built these tests compare with the reference."""
+    if available():
+        return RefFilter(p, frames)
+    import _oracle
+    return _oracle.OracleFilter(p, frames)
 
 
 def seam_available():

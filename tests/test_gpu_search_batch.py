@@ -2,8 +2,9 @@
 consumer beyond the temporal filter) -- against the reference's own av1_full_pixel_search() (mcomp.c:1693-1832) run
 per block through the compiled, unmodified reference (oracle/_ref, tfref_full_pixel_search: configured as
 tf_motion_search() configures it, the same NSTEP search first_pass_motion_search(), firstpass.c:261-300, and TPL's
-motion_estimation(), tpl_model.c:285, run per 16x16 / 32x32 block).  Best MV and returned variance cost must be
-equal for every block: 16x16 and 32x32 blocks on the macroblock grid, zero and random start MVs, frame edges."""
+motion_estimation(), tpl_model.c:285, run per 16x16 / 32x32 block); where oracle/_ref is not built, the oracle's
+restatement of that search (tfo_full_pixel_search).  Best MV and returned variance cost must be equal for every
+block: 16x16 and 32x32 blocks on the macroblock grid, zero and random start MVs, frame edges."""
 import numpy as np
 import pytest
 
@@ -11,7 +12,7 @@ import _clips
 import _params
 import _ref
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not _ref.available(), reason="oracle/_ref/libtf_ref.so not built")]
+pytestmark = pytest.mark.gpu
 
 CASES = [  # name, W, H, bit depth, clip motion, params
     ("cif8_s4", 352, 288, 8, (1, 2), {}),
@@ -30,7 +31,7 @@ def test_batch_search_equals_reference_full_pixel_search(pkg, tfgpu, case, bsize
     name, W, H, bd, motion, pkw = case
     frames = _clips.moving_texture(W, H, 2, bd, motion=motion)
     p = _params.tf_params(W, H, 2, bit_depth=bd, **pkw)
-    r = _ref.RefFilter(p, frames)
+    r = _ref.reference_or_oracle(p, frames)
     bufs = [pkg.Yv12Buffer(W, H, 1, 1, bd > 8, p["border"], frame_id=880000 + 10 * CASES.index(case) + i).set_planes(*f, extend=False)
             for i, f in enumerate(frames)]
     rng = np.random.default_rng(1234 + bsize)

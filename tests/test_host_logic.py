@@ -68,8 +68,8 @@ def test_int_roofline_work_matches_survey():
     assert w["subpel"] == 16 * 2048 * 6
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/av1/encoder/temporal_filter.c"),
-                    reason="reference tree not present (GPU box)")
+@pytest.mark.skipif(not (_ref.SOURCE_DIR and os.path.exists(os.path.join(_ref.SOURCE_DIR, "av1/encoder/temporal_filter.c"))),
+                    reason="upstream source tree not given (REF=<dir>)")
 def test_seam_patch_applies_to_the_reference(tmp_path):
     """integration/tf_gpu_seam.patch is a well-formed unified diff against the reference tree."""
     import re
@@ -83,7 +83,7 @@ def test_seam_patch_applies_to_the_reference(tmp_path):
                              "build/cmake/aom_config_defaults.cmake"]
     for rel in files:
         os.makedirs(os.path.dirname(tmp_path / rel), exist_ok=True)
-        shutil.copyfile(os.path.join("/root/reference", rel), tmp_path / rel)
+        shutil.copyfile(os.path.join(_ref.SOURCE_DIR, rel), tmp_path / rel)
     r = subprocess.run(["patch", "-p1", "-s", "-i", patch], cwd=tmp_path, capture_output=True, text=True)
     assert r.returncode == 0, r.stdout + r.stderr
     patched = open(tmp_path / "av1/encoder/temporal_filter.c").read()

@@ -72,6 +72,24 @@ def test_apply_filter_block_vectors(bd, ss, extreme):
     assert (count == G[key + "/count"]).all()
 
 
+def test_full_pixel_search_matches_reference_fixture():
+    """With force_integer_mv the filter's MV of a block is its 32x32 full-pel search from a zero start
+    (temporal_filter.c:94-176), so the reference's stored MVs of that case pin the oracle's per-block
+    av1_full_pixel_search entry point (tfo_full_pixel_search) on every block, frame edges included."""
+    name, W, H, N, bd, kind, ckw, pkw = next(c for c in PIPELINE_CASES if c[0] == "intmv8")
+    frames = make_frames(kind, W, H, N, bd, ckw, pkw)
+    p = _params.tf_params(W, H, N, bit_depth=bd, **pkw)
+    o = _oracle.OracleFilter(p, frames)
+    fi, mb_cols = p["filter_frame_idx"], (W + 31) // 32
+    mvs = G[f"{name}/mvs"]
+    for b in range(mvs.shape[0]):
+        y, x = (b // mb_cols) * 32, (b % mb_cols) * 32
+        for f in (f for f in range(N) if f != fi):
+            row, col, _ = o.full_pixel_search(fi, f, 32, x, y, 0, 0)
+            assert (row * 8, col * 8) == tuple(mvs[b, f, 0]), (b, f)
+    o.close()
+
+
 def test_od_divu_is_plain_division():
     # the exhaustive proof against the reference's table lives in test_oracle_vs_ref.py
     assert _oracle.lib().tfo_od_divu(21000 * 4095 + 10500, 21000) == (21000 * 4095 + 10500) // 21000
