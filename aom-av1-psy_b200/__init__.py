@@ -32,7 +32,7 @@ EXPORTS = [
     "tf_gpu_host_register", "tf_gpu_host_unregister", "tf_gpu_last_stats", "tf_gpu_event_record",
     "tf_gpu_event_elapsed_ms", "tf_gpu_synchronize", "tf_gpu_microbench", "tf_gpu_last_kernel_times", "tf_gpu_filter_resident_async", "tf_gpu_filter_resident_result", "tf_gpu_collect_counters", "tf_gpu_read_counters",
     "tf_gpu_cache_frame_async", "tf_gpu_debug_read_plane", "tf_gpu_device_border", "tf_gpu_fullpel_search_batch",
-    "tf_gpu_output_ipc_export", "tf_gpu_output_ipc_import",
+    "tf_gpu_output_ipc_export", "tf_gpu_output_ipc_import", "tf_gpu_cache_frame_device",
 ]
 
 
@@ -108,6 +108,7 @@ def load_library():
     lib.tf_gpu_cache_frame.argtypes = [vp, C.POINTER(Frame)]
     lib.tf_gpu_evict_frame.argtypes = [vp, u64]
     lib.tf_gpu_cache_frame_async.argtypes = [vp, C.POINTER(Frame)]
+    lib.tf_gpu_cache_frame_device.argtypes = [vp, C.POINTER(Frame), vp]
     lib.tf_gpu_debug_read_plane.argtypes = [vp, u64, i, vp, i, i, i, i, i]
     lib.tf_gpu_device_border.restype = i
     lib.tf_gpu_output_ipc_export.argtypes = [vp, i, C.c_char_p, C.POINTER(C.c_size_t), C.POINTER(C.c_size_t)]
@@ -212,6 +213,64 @@ class Yv12Buffer:
         return self.plane(p)[:h, :w]
 
 
+def tensor_frame(frame_id, y, u=None, v=None):
+    """tf_gpu_frame over 2-D CUDA tensors (the descriptor tf_gpu_cache_frame_device reads): uint8 for 8-bit,
+    int16 / uint16 for high bit depth, unit column stride, any row stride.  The geometry is derived as Yv12Buffer
+    derives it: crop = tensor shape, aligned = align8(luma) >> ss, ss_x / ss_y from the chroma shapes (no chroma:
+    monochrome).  Returns (Frame, torch.device).  Malformed input raises ValueError."""
+    import torch
+    if (u is None) != (v is None):
+        raise ValueError("give both chroma planes or neither")
+    planes = [y] if u is None else [y, u, v]
+    for t in planes:
+        if not isinstance(t, torch.Tensor) or t.dim() != 2 or t.numel() == 0:
+            raise ValueError("planes must be non-empty 2-D torch tensors")
+    hbd_types = (torch.int16, getattr(torch, "uint16", torch.int16))
+    if y.dtype == torch.uint8:
+        hbd = False
+    elif y.dtype in hbd_types:
+        hbd = True
+    else:
+        raise ValueError(f"luma dtype {y.dtype}: uint8 for 8-bit, int16 or uint16 for high bit depth")
+    if any(t.dtype != y.dtype for t in planes):
+        raise ValueError(f"planes of one frame must share a dtype, got {[str(t.dtype) for t in planes]}")
+    H, W = y.shape
+    ss_x = ss_y = 1
+    if u is not None:
+        if u.shape != v.shape:
+            raise ValueError(f"chroma planes differ in shape: {tuple(u.shape)} vs {tuple(v.shape)}")
+        ch, cw = u.shape
+        ss_x = next((s for s in (1, 0) if (W + s) >> s == cw), None)
+        ss_y = next((s for s in (1, 0) if (H + s) >> s == ch), None)
+        if ss_x is None or ss_y is None:
+            raise ValueError(f"chroma shape {tuple(u.shape)} matches no subsampling of a {H}x{W} luma plane")
+    def row_stride(t):
+        return t.stride(0) if t.shape[0] > 1 else t.shape[1]
+
+    for t in planes:
+        if t.shape[1] > 1 and t.stride(1) != 1:
+            raise ValueError("planes need a unit column stride (rows may have any stride)")
+    if u is not None and row_stride(u) != row_stride(v):
+        # tf_gpu_frame has one uv stride: the kernel would read one chroma plane with the other's row stride
+        raise ValueError(f"the chroma planes differ in row stride ({row_stride(u)} vs {row_stride(v)} samples); "
+                         "tf_gpu_frame has one uv stride: give them the same layout (e.g. .contiguous() both)")
+    for t in planes:
+        if not t.is_cuda:
+            raise ValueError("planes must be CUDA tensors (host frames go through Yv12Buffer / cache_frame)")
+        if t.device != y.device:
+            raise ValueError("planes of one frame must be on one device")
+    aw, ah = _align(W, 8), _align(H, 8)
+    f = Frame()
+    for p, t in enumerate(planes):
+        f.plane[p] = t.data_ptr()
+    for k, (t, sx, sy) in enumerate(((y, 0, 0), (planes[-1], ss_x, ss_y))):
+        f.stride[k] = row_stride(t)
+        f.crop_w[k], f.crop_h[k] = (W + sx) >> sx, (H + sy) >> sy
+        f.aligned_w[k], f.aligned_h[k] = aw >> sx, ah >> sy
+    f.border, f.ss_x, f.ss_y, f.is_hbd, f.frame_id = 0, ss_x, ss_y, int(hbd), frame_id
+    return f, y.device
+
+
 def make_params(p):
     """dict (tests/_params.tf_params) -> tf_gpu_params."""
     c = Params()
@@ -240,6 +299,7 @@ class TemporalFilterGpu:
 
     def __init__(self, device=-1, max_cached_frames=0):
         self.lib = load_library()
+        self.device = device
         self.h = C.c_void_p()
         cfg = DeviceCfg(device=device, max_cached_frames=max_cached_frames)
         rc = self.lib.tf_gpu_create(C.byref(self.h), C.byref(cfg))
@@ -315,6 +375,62 @@ class TemporalFilterGpu:
         """Upload without waiting (at most one outstanding; see tf_gpu.h)."""
         cf = frame.c_frame()
         self._check(self.lib.tf_gpu_cache_frame_async(self.h, C.byref(cf)))
+
+    # ---- frames that already live in device memory (torch CUDA tensors) ---------------------------------------
+    def cache_frame_tensor(self, frame_id, y, u=None, v=None):
+        """Put a frame held in CUDA tensors into the device cache (tf_gpu_cache_frame_device): see tensor_frame()
+        for what the tensors may be.  Ordered on the tensors' current torch stream: the ingest runs after what is
+        already enqueued there, and later work on that stream runs after the ingest, so the tensors may be
+        overwritten on that stream right after the call.  They may also be freed: the tensors are recorded as in use
+        on that stream (Tensor.record_stream), so the caching allocator does not hand their memory out again, on
+        the stream they were allocated on or any other, before the ingest has read it.  Does not block the host."""
+        import torch
+        f, dev = tensor_frame(frame_id, y, u, v)
+        s = torch.cuda.current_stream(dev)
+        self._check(self.lib.tf_gpu_cache_frame_device(self.h, C.byref(f), s.cuda_stream))
+        for t in (y, u, v):
+            if t is not None:
+                t.record_stream(s)
+
+    def _torch_device(self, torch):
+        return torch.device("cuda", self.device if self.device >= 0 else torch.cuda.current_device())
+
+    def filter_tensors(self, params, frame_ids):
+        """filter_resident() over cached frames, returning the crop area of every output plane as new CUDA tensors
+        (uint8 for 8-bit, int16 for high bit depth) and FRAME_DIFF.  params: the dict form (_params.tf_params),
+        which carries the crop size.  The copies out of the library's output planes (the zero-copy views
+        sharding.SlabWindow.device_planes builds) run on the current torch stream and have finished on return,
+        so the next filter call of this context may overwrite the planes."""
+        import torch
+        _, diff = self.filter_resident(params, frame_ids)
+        dev = self._torch_device(torch)
+        W, H = params["width"], params["height"]
+        out = []
+        for pl in range(1 if params["monochrome"] else 3):
+            sx, sy = (params["ss_x"], params["ss_y"]) if pl else (0, 0)
+            es = 2 if params["use_hbd"] else 1
+            ptr, pitch, rows, _ = self.output_device_plane(pl)
+
+            class _View:  # __cuda_array_interface__ holder
+                pass
+            view = _View()
+            view.__cuda_array_interface__ = {"shape": (rows, pitch), "typestr": "|u1", "data": (ptr, False),
+                                             "version": 3}
+            t = torch.as_tensor(view, device=dev)[:(H + sy) >> sy, :((W + sx) >> sx) * es]
+            out.append(t.view(torch.int16).clone() if es == 2 else t.clone())
+        torch.cuda.current_stream(dev).synchronize()
+        return out, diff
+
+    def estimate_noise_tensor(self, frame_id, tensors, plane, bit_depth,
+                              edge_thresh=NOISE_ESTIMATION_EDGE_THRESHOLD):
+        """av1_estimate_noise_from_single_plane on a frame held in CUDA tensors (y,) or (y, u, v): ingests it under
+        frame_id (nothing is read when that id is resident), then estimates from the cached slot."""
+        y, u, v = (tuple(tensors) + (None, None))[:3]
+        self.cache_frame_tensor(frame_id, y, u, v)
+        f, _ = tensor_frame(frame_id, y, u, v)
+        out = C.c_double()
+        self._check(self.lib.tf_gpu_estimate_noise(self.h, C.byref(f), plane, bit_depth, edge_thresh, C.byref(out)))
+        return out.value
 
     def debug_read_plane(self, frame, plane, x0, y0, w, h):
         """Rectangle of a cached device plane, border included (test hook for the upload path)."""

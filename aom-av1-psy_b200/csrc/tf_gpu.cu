@@ -93,6 +93,7 @@ struct tf_gpu_ctx {
   cudaStream_t noise_stream = nullptr;        // noise estimates do not queue behind a submitted window
   cudaEvent_t ev_async_upload = nullptr;      // last tf_gpu_cache_frame_async upload
   bool async_upload_pending = false;
+  cudaEvent_t ev_ingest_src = nullptr;        // producer's stream at a tf_gpu_cache_frame_device call
   cudaEvent_t user_ev[4] = { nullptr, nullptr, nullptr, nullptr };
   std::vector<DevFrame> cache;
   DevFrame out;
@@ -206,6 +207,20 @@ EncodeTiledFn encode_tiled_fn() {
   }
   return fn;
 }
+// cuMemGetAddressRange (allocation base and size of a device pointer), for the extent check of device frames
+typedef CUresult (*AddressRangeFn)(CUdeviceptr *, size_t *, CUdeviceptr);
+AddressRangeFn address_range_fn() {
+  static AddressRangeFn fn = nullptr;
+  static bool tried = false;
+  if (!tried) {
+    tried = true;
+    void *p = nullptr;
+    cudaDriverEntryPointQueryResult q;
+    if (cudaGetDriverEntryPoint("cuMemGetAddressRange", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
+      fn = (AddressRangeFn)p;
+  }
+  return fn;
+}
 int make_tensor_maps(tf_gpu_ctx *ctx, DevFrame *d) {
   EncodeTiledFn enc = encode_tiled_fn();
   if (!enc) return fail(ctx, TF_GPU_ERR_CUDA, "cuTensorMapEncodeTiled is not available in this driver");
@@ -279,6 +294,42 @@ int upload_frame(tf_gpu_ctx *ctx, DevFrame *d, const tf_gpu_frame *f) {
   return TF_GPU_OK;
 }
 
+// Fill a slot from device planes (tf_gpu_cache_frame_device, validated there): after the work already enqueued on
+// the producer's stream, one ingest_plane_kernel per plane on the copy stream writes the same rectangle
+// upload_frame() defines.
+int ingest_frame(tf_gpu_ctx *ctx, DevFrame *d, const tf_gpu_frame *f, cudaStream_t src_stream) {
+  const Geometry &g = d->g;
+  CU(cudaEventRecord(ctx->ev_ingest_src, src_stream));
+  CU(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_ingest_src, 0));
+  for (int p = 0; p < g.num_planes; p++) {
+    const int k = p > 0;
+    const int ext_w = g.aligned_w[k] + g.bx[k], ext_h = g.aligned_h[k] + g.by[k];
+    const int groups = (g.bx[k] + ext_w + (g.is_hbd ? 8 : 16) - 1) / (g.is_hbd ? 8 : 16);
+    const dim3 grid((groups + INGEST_THREADS - 1) / INGEST_THREADS, (g.by[k] + ext_h + INGEST_ROWS - 1) / INGEST_ROWS);
+    if (g.is_hbd)
+      ingest_plane_kernel<uint16_t><<<grid, INGEST_THREADS, 0, ctx->copy_stream>>>(
+          (uint16_t *)d->p00[p], g.pitch[k], (const uint16_t *)f->plane[p], f->stride[k], g.crop_w[k], g.crop_h[k],
+          g.bx[k], g.by[k], ext_w, ext_h);
+    else
+      ingest_plane_kernel<uint8_t><<<grid, INGEST_THREADS, 0, ctx->copy_stream>>>(
+          (uint8_t *)d->p00[p], g.pitch[k], (const uint8_t *)f->plane[p], f->stride[k], g.crop_w[k], g.crop_h[k],
+          g.bx[k], g.by[k], ext_w, ext_h);
+    ctx->last_launches++;
+  }
+  CU(cudaGetLastError());
+  CU(cudaEventRecord(d->ready, ctx->copy_stream));
+  d->frame_id = f->frame_id;
+  d->valid = true;
+  return TF_GPU_OK;
+}
+
+// Where a frame that is not resident comes from: the host (upload_frame) or device memory written on `stream`
+// (ingest_frame).
+struct FrameSource {
+  bool device = false;
+  cudaStream_t stream = nullptr;
+};
+
 DevFrame *find_cached(tf_gpu_ctx *ctx, uint64_t id, const Geometry *g) {
   if (!id) return nullptr;
   for (auto &d : ctx->cache)
@@ -288,7 +339,8 @@ DevFrame *find_cached(tf_gpu_ctx *ctx, uint64_t id, const Geometry *g) {
 
 // Returns a slot holding the frame (uploading if needed); the slot is pinned
 // for the current epoch so that one window never evicts its own frames.
-int get_frame(tf_gpu_ctx *ctx, const tf_gpu_frame *f, int num_planes, DevFrame **out) {
+int get_frame(tf_gpu_ctx *ctx, const tf_gpu_frame *f, int num_planes, DevFrame **out,
+              const FrameSource &src = FrameSource()) {
   Geometry g;
   if (!make_geometry(f, num_planes, &g)) return fail(ctx, TF_GPU_ERR_INVALID, "bad frame geometry");
   DevFrame *d = find_cached(ctx, f->frame_id, &g);
@@ -324,7 +376,7 @@ int get_frame(tf_gpu_ctx *ctx, const tf_gpu_frame *f, int num_planes, DevFrame *
       if (victim->pinned_epoch > 0 && ctx->done_valid[idx])
         CU(cudaStreamWaitEvent(ctx->copy_stream, ctx->done_ev[idx], 0));
     }
-    rc = upload_frame(ctx, victim, f);
+    rc = src.device ? ingest_frame(ctx, victim, f, src.stream) : upload_frame(ctx, victim, f);
     if (rc) return rc;
     d = victim;
   }
@@ -907,6 +959,7 @@ int tf_gpu_create(tf_gpu_ctx **out, const tf_gpu_device_cfg *cfg) {
   for (int i = 0; i < 8; i++) make_call_events(ctx->tickets[i].te);
   if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&ctx->noise_stream, cudaStreamNonBlocking);
   if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ctx->ev_async_upload, cudaEventDisableTiming);
+  if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ctx->ev_ingest_src, cudaEventDisableTiming);
   for (int i = 0; i < 4 && e == cudaSuccess; i++) e = cudaEventCreate(&ctx->user_ev[i]);
   for (int i = 0; i < 8 && e == cudaSuccess; i++) e = cudaEventCreateWithFlags(&ctx->tickets[i].ev, cudaEventDisableTiming);
   if (e == cudaSuccess) e = cudaMalloc(&ctx->d_diff, 18 * sizeof(unsigned long long));
@@ -977,6 +1030,7 @@ void tf_gpu_destroy(tf_gpu_ctx *ctx) {
     cudaStreamDestroy(ctx->noise_stream);
   }
   if (ctx->ev_async_upload) cudaEventDestroy(ctx->ev_async_upload);
+  if (ctx->ev_ingest_src) cudaEventDestroy(ctx->ev_ingest_src);
   if (ctx->ev0) cudaEventDestroy(ctx->ev0);
   if (ctx->ev1) cudaEventDestroy(ctx->ev1);
   for (int i = 0; i < TF_GPU_MAX_FRAMES; i++)
@@ -1020,6 +1074,73 @@ int tf_gpu_cache_frame_async(tf_gpu_ctx *ctx, const tf_gpu_frame *frame) {
   if (rc) return rc;
   CU(cudaEventRecord(ctx->ev_async_upload, ctx->copy_stream));
   ctx->async_upload_pending = true;
+  return TF_GPU_OK;
+}
+
+int tf_gpu_cache_frame_device(tf_gpu_ctx *ctx, const tf_gpu_frame *frame, void *stream) {
+  if (!ctx || !frame) return TF_GPU_ERR_INVALID;
+  ctx->last_launches = 0;
+  if (!frame->frame_id) return fail(ctx, TF_GPU_ERR_INVALID, "frame_id 0 cannot be cached");
+  const int num_planes = frame->plane[1] ? 3 : 1;
+  Geometry g;
+  if (!make_geometry(frame, num_planes, &g)) return fail(ctx, TF_GPU_ERR_INVALID, "bad frame geometry");
+  CU(cudaSetDevice(ctx->device));
+  const AddressRangeFn range = address_range_fn();
+  if (!range) return fail(ctx, TF_GPU_ERR_CUDA, "cuMemGetAddressRange is not available in this driver");
+  // Everything the ingest kernels will read is checked here, before anything is enqueued: a plane is device (or
+  // managed) memory of this context's device, and its crop area, rows `stride` samples apart, lies inside the
+  // allocation the pointer belongs to (or in allocations mapped contiguously after it).
+  const size_t es = g.is_hbd ? 2 : 1;
+  for (int p = 0; p < num_planes; p++) {
+    const int k = p > 0;
+    const void *ptr = frame->plane[p];
+    if (!ptr) return fail(ctx, TF_GPU_ERR_INVALID, "frame plane %d is NULL", p);
+    if (g.crop_w[k] <= 0 || g.crop_h[k] <= 0 || g.aligned_w[k] < g.crop_w[k] || g.aligned_h[k] < g.crop_h[k])
+      return fail(ctx, TF_GPU_ERR_INVALID, "plane %d: bad crop / aligned size", p);
+    if (frame->stride[k] < g.crop_w[k])
+      return fail(ctx, TF_GPU_ERR_INVALID, "plane %d: stride %d is smaller than the crop width %d", p, frame->stride[k], g.crop_w[k]);
+    if ((uintptr_t)ptr % es) return fail(ctx, TF_GPU_ERR_INVALID, "plane %d is not aligned to its %zu-byte samples", p, es);
+    cudaPointerAttributes at;
+    if (cudaPointerGetAttributes(&at, ptr) != cudaSuccess) {
+      cudaGetLastError();
+      return fail(ctx, TF_GPU_ERR_INVALID, "plane %d is not a CUDA pointer", p);
+    }
+    if ((at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged) || at.device != ctx->device)
+      return fail(ctx, TF_GPU_ERR_INVALID, "plane %d is not device memory of device %d", p, ctx->device);
+    CUdeviceptr base = 0;
+    size_t size = 0;
+    const CUdeviceptr dp = (CUdeviceptr)(uintptr_t)ptr;
+    if (range(&base, &size, dp) != CUDA_SUCCESS || dp < base || dp - base > size)
+      return fail(ctx, TF_GPU_ERR_INVALID, "plane %d: no device allocation at this address", p);
+    const size_t need = ((size_t)(g.crop_h[k] - 1) * frame->stride[k] + g.crop_w[k]) * es;
+    // Allocators that map memory in chunks (the virtual-memory API behind torch's expandable segments, stream-ordered
+    // pools) may report one chunk per call: the extent may go on into chunks mapped right after it, each device
+    // memory of this device, so the walk follows the ranges as long as they are contiguous.
+    CUdeviceptr end = base + size;
+    while (end - dp < need) {
+      CUdeviceptr nb = 0;
+      size_t ns = 0;
+      cudaPointerAttributes na;
+      if (range(&nb, &ns, end) != CUDA_SUCCESS || nb != end || ns == 0 ||
+          cudaPointerGetAttributes(&na, (const void *)(uintptr_t)end) != cudaSuccess ||
+          (na.type != cudaMemoryTypeDevice && na.type != cudaMemoryTypeManaged) || na.device != ctx->device) {
+        cudaGetLastError();
+        return fail(ctx, TF_GPU_ERR_INVALID,
+                    "plane %d: its crop area (%zu bytes from pixel (0,0)) runs past its allocation (%zu bytes)", p,
+                    need, (size_t)(end - dp));
+      }
+      end = nb + ns;
+    }
+  }
+  CallScope scope(ctx);
+  FrameSource src;
+  src.device = true;
+  src.stream = (cudaStream_t)stream;
+  DevFrame *d;
+  int rc = get_frame(ctx, frame, num_planes, &d, src);
+  if (rc) return rc;
+  // the producer may overwrite or free the planes in its stream order (a resident frame: its last load)
+  CU(cudaStreamWaitEvent(src.stream, d->ready, 0));
   return TF_GPU_OK;
 }
 

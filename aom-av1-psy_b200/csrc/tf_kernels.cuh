@@ -2313,6 +2313,62 @@ __global__ void extend_borders_kernel(T *plane /* pixel (0,0) */, int pitch, int
 }
 
 // ---------------------------------------------------------------------------
+// Device ingest: a caller's device plane (any row stride, any base alignment)
+// copied into a cache slot together with the border replication, in one pass.
+// Writes rows [-by, aligned_h + by) x columns [-bx, aligned_w + bx) -- the
+// rectangle upload + extend_borders_kernel define -- with
+// dst[y][x] = src[clamp(y, 0, crop_h - 1)][clamp(x, 0, crop_w - 1)].
+// One thread per 16-byte group of a slot row, counted from the row start
+// (column -bx; slot rows are 128-sample aligned), so every store is one
+// st.global.v4; the last group of a row may run into the pitch padding,
+// which nothing reads.  Loads are as wide as the source address allows
+// (16 / 8 / 4 bytes) for groups inside the crop columns, single samples with
+// clamping otherwise.  INGEST_ROWS rows per thread for independent loads.
+// ---------------------------------------------------------------------------
+constexpr int INGEST_THREADS = 128, INGEST_ROWS = 4;
+
+template <typename T>
+__global__ void __launch_bounds__(INGEST_THREADS) ingest_plane_kernel(
+    T *__restrict__ dst /* slot pixel (0,0) */, int pitch, const T *__restrict__ src /* pixel (0,0) */, int stride,
+    int crop_w, int crop_h, int bx, int by, int ext_w /* aligned_w + bx */, int ext_h /* aligned_h + by */) {
+  constexpr int V = 16 / sizeof(T);  // samples per group
+  constexpr int PER_WORD = 4 / sizeof(T);
+  const int groups = (bx + ext_w + V - 1) / V;
+  const int g = blockIdx.x * INGEST_THREADS + threadIdx.x;
+  if (g >= groups) return;
+  const int x0 = g * V - bx;
+  const bool inside = x0 >= 0 && x0 + V <= crop_w;
+#pragma unroll
+  for (int r = 0; r < INGEST_ROWS; r++) {
+    const int y = (blockIdx.y * INGEST_ROWS + r) - by;
+    if (y >= ext_h) break;
+    const T *row = src + (long long)iclamp(y, 0, crop_h - 1) * stride;
+    uint32_t w[4];
+    const uintptr_t a = (uintptr_t)(row + x0);
+    if (inside && (a & 15) == 0) {
+      const uint4 q = __ldg((const uint4 *)a);
+      w[0] = q.x, w[1] = q.y, w[2] = q.z, w[3] = q.w;
+    } else if (inside && (a & 7) == 0) {
+      const uint2 q0 = __ldg((const uint2 *)a), q1 = __ldg((const uint2 *)a + 1);
+      w[0] = q0.x, w[1] = q0.y, w[2] = q1.x, w[3] = q1.y;
+    } else if (inside && (a & 3) == 0) {
+#pragma unroll
+      for (int j = 0; j < 4; j++) w[j] = __ldg((const uint32_t *)a + j);
+    } else {
+#pragma unroll
+      for (int j = 0; j < 4; j++) {
+        uint32_t v = 0;
+#pragma unroll
+        for (int i = 0; i < PER_WORD; i++)
+          v |= (uint32_t)__ldg(row + iclamp(x0 + j * PER_WORD + i, 0, crop_w - 1)) << (8 * sizeof(T) * i);
+        w[j] = v;
+      }
+    }
+    *(uint4 *)(dst + (long long)y * pitch + x0) = make_uint4(w[0], w[1], w[2], w[3]);
+  }
+}
+
+// ---------------------------------------------------------------------------
 // av1_estimate_noise_from_single_plane (temporal_filter.c:1150-1194):
 // integer accumulate / count; the final double division is done on the host.
 // ---------------------------------------------------------------------------

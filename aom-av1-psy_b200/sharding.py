@@ -9,7 +9,8 @@ Two independent axes, no exchange during compute:
     rank 0 straight from the library's device output planes, plus a 16-byte
     all-reduce for FRAME_DIFF (integer sums: order independent); or, without any
     gather, every rank stores its rows straight into rank 0's planes over NVLink
-    (CUDA IPC peer mapping, `connect_peer_output`).
+    (CUDA IPC peer mapping, `connect_peer_output`).  When only one rank holds the window's frames,
+    `replicate_frames` broadcasts them over NVLink and every rank ingests them from device memory.
 The reference's counterpart is the row job queue of av1/encoder/ethread.c:2062-2189
 (workers share tf_ctx->output_frame and add their FRAME_DIFF under a mutex, :2161-2173).
 
@@ -52,6 +53,7 @@ class SlabWindow:
         self.pad_rows = max_slab_rows(mb_rows, world)
         self.block_h = [32] + [32 >> ss_y] * (num_planes - 1)
         self._recv = None
+        self._stage, self._stage_meta = None, None  # replicate_frames' staging tensors and what they were made for
 
     def params(self, p):
         """The window's parameters restricted to this rank's rows."""
@@ -119,6 +121,48 @@ class SlabWindow:
         rank's rows are in the owner's planes."""
         dist.all_reduce(diff)
         return diff
+
+    # ---- frame replication: the window's pixels cross PCIe once per box ---------------------------------------
+    def replicate_frames(self, ctx, dist, torch, frames, ids, owner=0, device=None):
+        """Put the window's frames into every rank's frame cache when only `owner` holds them.  frames / ids:
+        on the owner, per frame (y, u, v) (u, v None for monochrome) as host arrays or CUDA tensors, and the frame
+        ids; ignored elsewhere.  The owner stages each plane in a device tensor, dist.broadcast sends it to every
+        rank's staging tensor (shapes, dtypes and ids go first with broadcast_object_list, so the other ranks need
+        no pixels), and every rank, owner included, ingests it with ctx.cache_frame_tensor.  The staging tensors
+        are reused by the next window of the same geometry.  device: where staging lives (default: the current
+        CUDA device under NCCL, the CPU otherwise).  Returns the ids."""
+        if device is None:
+            device = (torch.device("cuda", torch.cuda.current_device()) if dist.get_backend() == "nccl"
+                      else torch.device("cpu"))
+        def as_tensor(a):  # collectives carry 16-bit samples as int16 (the ingest takes int16 and uint16 alike)
+            if not isinstance(a, torch.Tensor):
+                return torch.from_numpy(a.view("int16") if a.dtype.itemsize == 2 else a)
+            return a.view(torch.int16) if a.dtype == getattr(torch, "uint16", None) else a
+
+        src = []
+        box = [None]
+        if self.rank == owner:
+            src = [[as_tensor(a) for a in planes if a is not None] for planes in frames]
+            box = [([int(i) for i in ids], [[(tuple(t.shape), str(t.dtype)) for t in ts] for ts in src])]
+        dist.broadcast_object_list(box, src=owner)
+        out_ids, meta = box[0]
+        if self._stage is None or self._stage_meta != (meta, device):
+            # byte tensors on the wire (NCCL and gloo have no 16-bit integer type), sample-typed views for the ingest
+            self._stage = []
+            for planes in meta:
+                views = []
+                for (h, w), dt in planes:
+                    dt = getattr(torch, dt.split(".")[-1])
+                    views.append(torch.empty((h, w * dt.itemsize), dtype=torch.uint8, device=device).view(dt))
+                self._stage.append(views)
+            self._stage_meta = (meta, device)
+        for f, planes in enumerate(self._stage):
+            for p, t in enumerate(planes):
+                if self.rank == owner:
+                    t.copy_(src[f][p])
+                dist.broadcast(t.view(torch.uint8), src=owner)
+            ctx.cache_frame_tensor(out_ids[f], *planes)
+        return out_ids
 
     # ---- collective ---------------------------------------------------------------------------
     def gather(self, slabs, diff, dist, torch):

@@ -155,7 +155,11 @@ int tf_gpu_wait(tf_gpu_ctx *ctx, uint64_t ticket);
 /* Step before / after the path (SURVEY 8f rank 1-2): upload a source frame
  * into the device cache when it enters the lookahead (av1_lookahead_push,
  * lookahead.c:101-163) so that tf_gpu_filter never waits on PCIe; drop it when
- * it leaves. */
+ * it leaves.  A cache slot is filled from host memory (tf_gpu_cache_frame,
+ * tf_gpu_cache_frame_async, or any call taking tf_gpu_frame) or from device
+ * memory (tf_gpu_cache_frame_device); both leave sample-identical slots (crop
+ * area plus the replicated device border), so the resident calls cannot tell
+ * them apart and one window may mix them. */
 int tf_gpu_cache_frame(tf_gpu_ctx *ctx, const tf_gpu_frame *frame);
 /* Same without waiting for the copy: the call first waits for the PREVIOUS asynchronous upload of
  * this context, then enqueues this one and returns.  So at most one upload is outstanding and a
@@ -163,6 +167,19 @@ int tf_gpu_cache_frame(tf_gpu_ctx *ctx, const tf_gpu_frame *frame);
  * tf_gpu_synchronize / tf_gpu_wait that covers it) has returned -- which is what a lookahead ring
  * needs: a slot is only rewritten by a later av1_lookahead_push (lookahead.c:126,150). */
 int tf_gpu_cache_frame_async(tf_gpu_ctx *ctx, const tf_gpu_frame *frame);
+/* Same as tf_gpu_cache_frame, but frame->plane[] are DEVICE pointers on the context's device (stride in
+ * samples, crop/aligned sizes and frame_id as for host frames; frame->border is ignored: only the crop area is
+ * read).  `stream` (a cudaStream_t; NULL = the legacy default stream) is the stream the producer wrote the
+ * planes on: the ingest starts after the work already enqueued there, and before returning the call makes
+ * `stream` wait for the ingest, so the caller may overwrite or free the planes in stream order.  Never blocks
+ * the host.  A frame_id that is already resident with the same geometry is not re-read (same id => same pixels).
+ * TF_GPU_ERR_INVALID, with nothing enqueued, for frame_id 0, a NULL plane, bad geometry, a plane that is not
+ * device or managed memory of the context's device, or one whose crop area
+ * ((crop_h - 1) * stride + crop_w samples from pixel (0,0)) runs past its allocation.  Allocations are those
+ * cuMemGetAddressRange reports; where an allocator maps its memory in chunks (virtual-memory mappings, stream-ordered
+ * pools), an extent may continue into chunks mapped contiguously after the first one on the same device.  Both
+ * chroma planes are read with the one uv stride. */
+int tf_gpu_cache_frame_device(tf_gpu_ctx *ctx, const tf_gpu_frame *frame, void *stream);
 int tf_gpu_evict_frame(tf_gpu_ctx *ctx, uint64_t frame_id);
 /* Test hook for the upload path (av1_copy_and_extend_frame, extend.c:113-163): copies the rectangle
  * [x0, x0+w) x [y0, y0+h) of a cached device plane (coordinates relative to pixel (0,0); negative =
