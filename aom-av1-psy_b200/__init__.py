@@ -20,6 +20,7 @@ LIB_PATH = os.path.join(_HERE, "libtf_gpu.so")
 LIB_PATH = os.environ.get("TF_GPU_LIB", LIB_PATH)
 
 TF_GPU_MAX_FRAMES = 24
+TF_GPU_MAX_BATCH = 16
 NOISE_ESTIMATION_EDGE_THRESHOLD = 50  # temporal_filter.h:79
 TF_BLOCK = 32  # TF_BLOCK_SIZE = BLOCK_32X32, temporal_filter.h:31
 
@@ -33,6 +34,8 @@ EXPORTS = [
     "tf_gpu_event_elapsed_ms", "tf_gpu_synchronize", "tf_gpu_microbench", "tf_gpu_last_kernel_times", "tf_gpu_filter_resident_async", "tf_gpu_filter_resident_result", "tf_gpu_collect_counters", "tf_gpu_read_counters",
     "tf_gpu_cache_frame_async", "tf_gpu_debug_read_plane", "tf_gpu_device_border", "tf_gpu_fullpel_search_batch",
     "tf_gpu_output_ipc_export", "tf_gpu_output_ipc_import", "tf_gpu_cache_frame_device",
+    "tf_gpu_filter_batch_async", "tf_gpu_filter_batch_result", "tf_gpu_download_batch_output",
+    "tf_gpu_batch_output_device_plane",
 ]
 
 
@@ -131,6 +134,11 @@ def load_library():
     lib.tf_gpu_microbench.argtypes = [vp, i, C.POINTER(C.c_double)]
     lib.tf_gpu_last_kernel_times.argtypes = [vp, C.POINTER(C.c_float)]
     lib.tf_gpu_collect_counters.argtypes = [vp, i]
+    lib.tf_gpu_filter_batch_async.argtypes = [vp, i, C.POINTER(Params), C.POINTER(C.POINTER(u64))]
+    lib.tf_gpu_filter_batch_result.argtypes = [vp, C.POINTER(C.c_int64 * 2), C.POINTER(C.c_float)]
+    lib.tf_gpu_download_batch_output.argtypes = [vp, i, C.POINTER(Frame)]
+    lib.tf_gpu_batch_output_device_plane.argtypes = [vp, i, i, C.POINTER(vp), C.POINTER(C.c_size_t), C.POINTER(i),
+                                                     C.POINTER(i)]
     lib.tf_gpu_read_counters.argtypes = [vp, C.POINTER(u64)]
     _lib = lib
     return lib
@@ -294,6 +302,29 @@ def make_params(p):
     return c
 
 
+def batch_args(params_list, frame_ids_list):
+    """Arguments of tf_gpu_filter_batch_async for a list of windows: (n, tf_gpu_params[n], uint64_t *[n], keep-alive).
+    params_list holds dicts (tests/_params.tf_params) or Params; frame_ids_list one id list per window.  Raises
+    ValueError, before anything reaches the library, for lists of different lengths, an empty batch or one of more
+    than TF_GPU_MAX_BATCH windows, and a window whose id count differs from its num_frames."""
+    params_list, frame_ids_list = list(params_list), list(frame_ids_list)
+    if len(params_list) != len(frame_ids_list):
+        raise ValueError(f"{len(params_list)} params for {len(frame_ids_list)} id lists")
+    n = len(params_list)
+    if not 1 <= n <= TF_GPU_MAX_BATCH:
+        raise ValueError(f"a batch holds 1 to {TF_GPU_MAX_BATCH} windows, got {n}")
+    cps = [make_params(p) if isinstance(p, dict) else p for p in params_list]
+    ids = []
+    for w, (cp, fl) in enumerate(zip(cps, frame_ids_list)):
+        fl = [int(i) for i in fl]
+        if len(fl) != cp.num_frames:
+            raise ValueError(f"window {w}: {len(fl)} frame ids for num_frames {cp.num_frames}")
+        ids.append((C.c_uint64 * len(fl))(*fl))
+    params = (Params * n)(*cps)
+    ptrs = (C.POINTER(C.c_uint64) * n)(*[C.cast(a, C.POINTER(C.c_uint64)) for a in ids])
+    return n, params, ptrs, ids
+
+
 class TemporalFilterGpu:
     """One tf_gpu_ctx (CUDA device + stream + frame cache)."""
 
@@ -403,13 +434,19 @@ class TemporalFilterGpu:
         so the next filter call of this context may overwrite the planes."""
         import torch
         _, diff = self.filter_resident(params, frame_ids)
+        out = self._clone_planes(torch, params, self.output_device_plane)
+        torch.cuda.current_stream(self._torch_device(torch)).synchronize()
+        return out, diff
+
+    def _clone_planes(self, torch, params, device_plane):
+        """Crop area of every output plane that device_plane(plane) describes, cloned on the current torch stream."""
         dev = self._torch_device(torch)
         W, H = params["width"], params["height"]
         out = []
         for pl in range(1 if params["monochrome"] else 3):
             sx, sy = (params["ss_x"], params["ss_y"]) if pl else (0, 0)
             es = 2 if params["use_hbd"] else 1
-            ptr, pitch, rows, _ = self.output_device_plane(pl)
+            ptr, pitch, rows, _ = device_plane(pl)
 
             class _View:  # __cuda_array_interface__ holder
                 pass
@@ -418,8 +455,52 @@ class TemporalFilterGpu:
                                              "version": 3}
             t = torch.as_tensor(view, device=dev)[:(H + sy) >> sy, :((W + sx) >> sx) * es]
             out.append(t.view(torch.int16).clone() if es == 2 else t.clone())
-        torch.cuda.current_stream(dev).synchronize()
-        return out, diff
+        return out
+
+    # ---- several windows over one frame cache in one call (tf_gpu_filter_batch_async) -------------------------
+    def filter_batch_async(self, params_list, frame_ids_list):
+        """Enqueue a batch of windows over resident frames (see batch_args for the checks made here)."""
+        n, params, ptrs, _ = batch_args(params_list, frame_ids_list)
+        self._check(self.lib.tf_gpu_filter_batch_async(self.h, n, params, ptrs))
+        self._batch_n = n
+        return n
+
+    def filter_batch_result(self, n=None):
+        """Wait for the last batch: (kernel ms, FRAME_DIFF int64[n, 2]), n = its window count unless given (at most
+        that).  The library writes one entry per window of the last batch, so the buffer holds TF_GPU_MAX_BATCH."""
+        last = getattr(self, "_batch_n", 0)
+        n = last if n is None else min(int(n), last)
+        diffs = (C.c_int64 * 2 * TF_GPU_MAX_BATCH)()
+        ms = C.c_float()
+        self._check(self.lib.tf_gpu_filter_batch_result(self.h, diffs, C.byref(ms)))
+        return ms.value, np.array([[d[0], d[1]] for d in diffs[:n]], np.int64).reshape(n, 2)
+
+    def filter_batch(self, params_list, frame_ids_list):
+        """Filter several windows over cached frames in one call: (kernel ms, FRAME_DIFF int64[n, 2]).  Each window's
+        output stays on the device (download_batch_output, batch_output_device_plane) until the next batch."""
+        return self.filter_batch_result(self.filter_batch_async(params_list, frame_ids_list))
+
+    def download_batch_output(self, window, out):
+        co = out.c_frame()
+        self._check(self.lib.tf_gpu_download_batch_output(self.h, window, C.byref(co)))
+
+    def batch_output_device_plane(self, window, plane):
+        p, pitch, rows, rb = C.c_void_p(), C.c_size_t(), C.c_int(), C.c_int()
+        self._check(self.lib.tf_gpu_batch_output_device_plane(self.h, window, plane, C.byref(p), C.byref(pitch),
+                                                              C.byref(rows), C.byref(rb)))
+        return p.value, pitch.value, rows.value, rb.value
+
+    def filter_batch_tensors(self, params_list, frame_ids_list):
+        """filter_batch() returning, per window, (output planes as new CUDA tensors, FRAME_DIFF) as filter_tensors
+        does.  params_list: dicts (_params.tf_params).  The copies run on the current torch stream and have
+        finished on return."""
+        import torch
+        _, diffs = self.filter_batch(params_list, frame_ids_list)
+        res = []
+        for w, p in enumerate(params_list):
+            res.append((self._clone_planes(torch, p, lambda pl, w=w: self.batch_output_device_plane(w, pl)), diffs[w]))
+        torch.cuda.current_stream(self._torch_device(torch)).synchronize()
+        return res
 
     def estimate_noise_tensor(self, frame_id, tensors, plane, bit_depth,
                               edge_thresh=NOISE_ESTIMATION_EDGE_THRESHOLD):

@@ -119,6 +119,14 @@ struct tf_gpu_ctx {
   uint64_t next_ticket = 1;
   int last_launches = 0;
   float last_kernel_ms = 0.f;
+  // batched windows (tf_gpu_filter_batch_async): one output frame and one FRAME_DIFF slot per window, separate from
+  // `out` and the ticket / resident slots; allocated by the first batch that needs them
+  DevFrame bout[TF_GPU_MAX_BATCH];
+  unsigned long long *d_bdiff = nullptr;  // [TF_GPU_MAX_BATCH][2]
+  unsigned long long *h_bdiff = nullptr;  // pinned mirror
+  int batch_n = 0;                        // windows of the last batch enqueued (0: none, or it failed)
+  int batch_planes[TF_GPU_MAX_BATCH] = {}; // planes each window writes (its num_planes; bout[w] may hold more)
+  CallEvents batch_ev;
   // dump buffers (device), grown on demand
   void *d_dump[12] = {};
   size_t d_dump_sz[12] = {};
@@ -543,11 +551,11 @@ void fill_kparams(const tf_gpu_ctx *ctx, const tf_gpu_params *p, const Geometry 
   K.hbd_shift = g.is_hbd ? (p->bit_depth == 10 ? 2 : (p->bit_depth == 12 ? 4 : 0)) : 0;
 }
 
-// Build kernel parameters and launch the block kernel over rows [rb, re).
-int launch_filter(tf_gpu_ctx *ctx, const tf_gpu_params *p, DevFrame *const *frames, const Geometry &g,
-                  unsigned long long *d_diff, const tf_gpu_dump *dump, const CallEvents *te) {
-  const bool timed = te != nullptr;
-  KParams K;
+// The KParams of one window writing into `out`, all rows: fill_kparams, the decay factors of the weights and the
+// frame planes.  Shared by the single-window and the batched launches; each adds where its scratch and
+// FRAME_DIFF go.
+void window_kparams(const tf_gpu_ctx *ctx, const tf_gpu_params *p, DevFrame *const *frames, const Geometry &g,
+                    const DevFrame &out, KParams &K) {
   fill_kparams(ctx, p, g, K);
   const int min_frame_size = K.width < K.height ? K.width : K.height;  // av1_apply_temporal_filter_c: the source size (:603)
   {  // decay factors, temporal_filter.c:583-597 (host libm, as the reference)
@@ -567,8 +575,20 @@ int launch_filter(tf_gpu_ctx *ctx, const tf_gpu_params *p, DevFrame *const *fram
     for (int pl = 0; pl < p->num_planes; pl++) K.frm[f][pl] = frames[f]->p00[pl];
     K.tmap[f] = frames[f]->d_tmap;
   }
+  for (int k = 0; k < 2; k++) K.out_pitch[k] = out.g.pitch[k];
+  for (int pl = 0; pl < p->num_planes; pl++) K.out[pl] = out.p00[pl];
+  K.num_pels = 1024 + (p->num_planes > 1 ? 2 * (1024 >> (g.ss_x + g.ss_y)) : 0);
+  K.row_begin = 0;
+  K.row_end = K.mb_rows;
+}
+
+// Build kernel parameters and launch the block kernel over rows [rb, re).
+int launch_filter(tf_gpu_ctx *ctx, const tf_gpu_params *p, DevFrame *const *frames, const Geometry &g,
+                  unsigned long long *d_diff, const tf_gpu_dump *dump, const CallEvents *te) {
+  const bool timed = te != nullptr;
+  KParams K;
+  window_kparams(ctx, p, frames, g, ctx->out, K);
   for (int pl = 0; pl < p->num_planes; pl++) {
-    K.out[pl] = ctx->out.p00[pl];
     if (ctx->peer_out[pl]) {  // the owner rank's plane: same geometry, hence the same pitch
       if (ctx->peer_pitch[pl] != (size_t)ctx->out.g.pitch[pl > 0] * (g.is_hbd ? 2 : 1))
         return fail(ctx, TF_GPU_ERR_INVALID, "imported output plane %d has a different pitch than this context's", pl);
@@ -581,9 +601,6 @@ int launch_filter(tf_gpu_ctx *ctx, const tf_gpu_params *p, DevFrame *const *fram
     K.ctr = ctx->d_ctr;
     CU(cudaMemsetAsync(ctx->d_ctr, 0, 4 * sizeof(unsigned long long), ctx->stream));
   }
-  K.num_pels = 1024 + (p->num_planes > 1 ? 2 * (1024 >> (g.ss_x + g.ss_y)) : 0);
-  K.row_begin = 0;
-  K.row_end = K.mb_rows;
   if (p->out_row_end > p->out_row_begin) {
     K.row_begin = p->out_row_begin < 0 ? 0 : p->out_row_begin;
     K.row_end = p->out_row_end > K.mb_rows ? K.mb_rows : p->out_row_end;
@@ -726,6 +743,88 @@ int launch_filter(tf_gpu_ctx *ctx, const tf_gpu_params *p, DevFrame *const *fram
   return TF_GPU_OK;
 }
 
+// The batched form of launch_filter: n windows over one geometry, every block row, each window into its own
+// output frame (ctx->bout[w]) and FRAME_DIFF slot.  Three launches on the main stream: the fused 32x32 chain
+// (every frame of a (window, block) in one warp) over the windows that have a reference frame, the 16x16 tasks over
+// the windows that have any, the filter over all.  Each kernel gets only the windows that have work for it, so
+// grid y never holds a window whose blocks would all exit.
+int launch_filter_batch(tf_gpu_ctx *ctx, int n, const tf_gpu_params *params,
+                        DevFrame *const (*frames)[TF_GPU_MAX_FRAMES], const Geometry &g, const CallEvents *te) {
+  const int mb_cols = (g.crop_w[0] + 31) / 32, nblk = ((g.crop_h[0] + 31) / 32) * mb_cols;
+  // search scratch: window w's [blocks][num_frames] slices follow those of the windows before it
+  size_t bf_total = 0;
+  for (int w = 0; w < n; w++) bf_total += (size_t)nblk * params[w].num_frames;
+  int rc = ensure_dump(ctx, 5, bf_total * 2 * sizeof(int16_t));
+  if (!rc) rc = ensure_dump(ctx, 6, bf_total * sizeof(int32_t));
+  if (!rc) rc = ensure_dump(ctx, 7, bf_total * 8 * sizeof(int16_t));
+  if (!rc) rc = ensure_dump(ctx, 8, bf_total * 4 * sizeof(int32_t));
+  if (!rc) rc = ensure_dump(ctx, 9, (size_t)n * nblk * 2 * sizeof(int16_t));
+  if (rc) return rc;
+  KParamsBatch all, s32, s16;
+  int n32 = 0, n16 = 0, max_nref16 = 0, max_pels = 0;
+  size_t bf = 0;
+  for (int w = 0; w < n; w++) {
+    const tf_gpu_params *p = &params[w];
+    KParams &K = all.w[w];
+    window_kparams(ctx, p, frames[w], g, ctx->bout[w], K);
+    K.diff = ctx->d_bdiff + 2 * w;
+    K.s_blk_mv = (int16_t *)ctx->d_dump[5] + bf * 2;
+    K.s_blk_mse = (int32_t *)ctx->d_dump[6] + bf;
+    K.s_sub_mv = (int16_t *)ctx->d_dump[7] + bf * 8;
+    K.s_sub_mse = (int32_t *)ctx->d_dump[8] + bf * 4;
+    K.s_ref_mv = (int16_t *)ctx->d_dump[9] + (size_t)w * nblk * 2;
+    K.frame_begin = 0;
+    K.frame_end = p->num_frames;
+    bf += (size_t)nblk * p->num_frames;
+    if (K.num_pels > max_pels) max_pels = K.num_pels;
+    const int nref = p->num_frames - 1;
+    if (nref > 0) {  // the same rules as launch_filter: no reference frame, no search; integer MVs, no 16x16 search
+      s32.w[n32++] = K;
+      if (!p->force_integer_mv) {
+        s16.w[n16++] = K;
+        if (nref > max_nref16) max_nref16 = nref;
+      }
+    }
+  }
+  CU(cudaMemsetAsync(ctx->d_bdiff, 0, (size_t)n * 2 * sizeof(unsigned long long), ctx->stream));
+  CU(cudaEventRecord(te->ev0, ctx->stream));
+  int nlaunch = 0;
+  if (n32) {
+    // the register build as launch_filter picks it for its per-frame grids, from the grid of the whole batch: the
+    // denser one only where it makes the grid resident in one wave
+    const long long total = (long long)nblk * n32;
+    const int hi = g.is_hbd ? S32_WARPS_HI_HBD : S32_WARPS_HI;
+    const bool one_wave = total <= (long long)ctx->num_sms * hi && total > (long long)ctx->num_sms * S32_WARPS_LO;
+    const dim3 grid(nblk, n32);
+    if (g.is_hbd) {
+      if (one_wave) tf_search32_batch_kernel<uint16_t, S32_WARPS_HI_HBD><<<grid, 32, SearchSmem<uint16_t, 32>::TOTAL_BASE, ctx->stream>>>(s32);
+      else tf_search32_batch_kernel<uint16_t, S32_WARPS_LO><<<grid, 32, SearchSmem<uint16_t, 32>::TOTAL, ctx->stream>>>(s32);
+    } else {
+      if (one_wave) tf_search32_batch_kernel<uint8_t, S32_WARPS_HI><<<grid, 32, SearchSmem<uint8_t, 32>::TOTAL_BASE, ctx->stream>>>(s32);
+      else tf_search32_batch_kernel<uint8_t, S32_WARPS_LO><<<grid, 32, SearchSmem<uint8_t, 32>::TOTAL, ctx->stream>>>(s32);
+    }
+    nlaunch++;
+  }
+  CU(cudaEventRecord(te->evk[0], ctx->stream));
+  if (n16) {
+    const dim3 grid(nblk * 4 * max_nref16, n16);
+    if (g.is_hbd) tf_search16_batch_kernel<uint16_t><<<grid, 32, SearchSmem<uint16_t, 16>::TOTAL, ctx->stream>>>(s16);
+    else tf_search16_batch_kernel<uint8_t><<<grid, 32, SearchSmem<uint8_t, 16>::TOTAL, ctx->stream>>>(s16);
+    nlaunch++;
+  }
+  CU(cudaEventRecord(te->evk[1], ctx->stream));
+  const dim3 grid(nblk, n);
+  if (g.is_hbd) tf_filter_batch_kernel<uint16_t><<<grid, FILT_THREADS, filter_smem_bytes(max_pels), ctx->stream>>>(all);
+  else tf_filter_batch_kernel<uint8_t><<<grid, FILT_THREADS, filter_smem_bytes(max_pels), ctx->stream>>>(all);
+  nlaunch++;
+  CU(cudaGetLastError());
+  CU(cudaEventRecord(te->ev1, ctx->stream));
+  ctx->last_launches += nlaunch;
+  ctx->split_valid = n32 > 0;
+  ctx->last_ev = te;
+  return TF_GPU_OK;
+}
+
 int download_dump(tf_gpu_ctx *ctx, const tf_gpu_params *p, const Geometry &g, const tf_gpu_dump *dump) {
   const int mb_rows = (g.crop_h[0] + 31) / 32, mb_cols = (g.crop_w[0] + 31) / 32;
   const size_t nb = (size_t)mb_rows * mb_cols, bf = nb * p->num_frames;
@@ -738,12 +837,15 @@ int download_dump(tf_gpu_ctx *ctx, const tf_gpu_params *p, const Geometry &g, co
   return TF_GPU_OK;
 }
 
-// Copy block rows [rb, re) of the device output into the caller's planes.
-int download_rows(tf_gpu_ctx *ctx, tf_gpu_frame *out, int rb, int re, cudaStream_t os) {
-  const Geometry &g = ctx->out.g;
+// Copy block rows [rb, re) of the first num_planes planes of a device output frame (ctx->out or a batch output)
+// into the caller's planes (num_planes < 0: all planes of the frame).
+int download_rows(tf_gpu_ctx *ctx, const DevFrame &dev, tf_gpu_frame *out, int rb, int re, cudaStream_t os,
+                  int num_planes = -1) {
+  const Geometry &g = dev.g;
   const size_t es = g.is_hbd ? 2 : 1;
   const int mb_cols = (g.crop_w[0] + 31) / 32;
-  for (int pl = 0; pl < g.num_planes; pl++) {
+  const int np = num_planes < 0 || num_planes > g.num_planes ? g.num_planes : num_planes;
+  for (int pl = 0; pl < np; pl++) {
     const int k = pl > 0;
     const int bh = 32 >> (pl ? g.ss_y : 0), bw = 32 >> (pl ? g.ss_x : 0);
     if (!out->plane[pl]) return fail(ctx, TF_GPU_ERR_INVALID, "output plane %d is NULL", pl);
@@ -757,7 +859,7 @@ int download_rows(tf_gpu_ctx *ctx, tf_gpu_frame *out, int rb, int re, cudaStream
     if (y1 > max_rows) y1 = max_rows;
     if (y1 <= y0) continue;
     char *dst = (char *)out->plane[pl] + (size_t)y0 * out->stride[k] * es;
-    const char *src = (const char *)ctx->out.p00[pl] + (size_t)y0 * g.pitch[k] * es;
+    const char *src = (const char *)dev.p00[pl] + (size_t)y0 * g.pitch[k] * es;
     CU(cudaMemcpy2DAsync(dst, (size_t)out->stride[k] * es, src, (size_t)g.pitch[k] * es, (size_t)cols * es, y1 - y0,
                          cudaMemcpyDeviceToHost, os));
   }
@@ -798,6 +900,17 @@ int extend_and_download_output(tf_gpu_ctx *ctx, tf_gpu_frame *out, cudaStream_t 
                          hb_y + ext_h, cudaMemcpyDeviceToHost, os));
   }
   return TF_GPU_OK;
+}
+
+// Pointer, pitch and full-block extent of a plane of a device output frame.
+void device_plane(const DevFrame &d, int plane, void **dptr, size_t *pitch_bytes, int *rows, int *row_bytes) {
+  const Geometry &g = d.g;
+  const int k = plane > 0;
+  const size_t es = g.is_hbd ? 2 : 1;
+  if (dptr) *dptr = d.p00[plane];
+  if (pitch_bytes) *pitch_bytes = (size_t)g.pitch[k] * es;
+  if (rows) *rows = ((g.crop_h[0] + 31) / 32) * (32 >> (plane ? g.ss_y : 0));
+  if (row_bytes) *row_bytes = (int)(((g.crop_w[0] + 31) / 32) * (32 >> (plane ? g.ss_x : 0)) * es);
 }
 
 int submit_impl(tf_gpu_ctx *ctx, const tf_gpu_params *params, const tf_gpu_frame *frames, tf_gpu_frame *out,
@@ -863,7 +976,7 @@ int submit_impl(tf_gpu_ctx *ctx, const tf_gpu_params *params, const tf_gpu_frame
       CU(cudaEventRecord(ctx->ev_out_ready, ctx->stream));
       CU(cudaStreamWaitEvent(os, ctx->ev_out_ready, 0));
     }
-    rc = download_rows(ctx, out, rb, re, os);
+    rc = download_rows(ctx, ctx->out, out, rb, re, os);
     if (rc) return rc;
   }
   if (dump) {
@@ -956,6 +1069,7 @@ int tf_gpu_create(tf_gpu_ctx **out, const tf_gpu_device_cfg *cfg) {
     if (e == cudaSuccess) e = cudaEventCreate(&te.evk[1]);
   };
   make_call_events(ctx->res_ev);
+  make_call_events(ctx->batch_ev);
   for (int i = 0; i < 8; i++) make_call_events(ctx->tickets[i].te);
   if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&ctx->noise_stream, cudaStreamNonBlocking);
   if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ctx->ev_async_upload, cudaEventDisableTiming);
@@ -976,6 +1090,8 @@ int tf_gpu_create(tf_gpu_ctx **out, const tf_gpu_device_cfg *cfg) {
   if (e == cudaSuccess) e = cudaMemcpyToSymbol(c_k8, K8, sizeof(K8));
   if (e == cudaSuccess) e = cudaFuncSetAttribute(tf_filter_kernel<uint8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)filter_smem_bytes(3072));
   if (e == cudaSuccess) e = cudaFuncSetAttribute(tf_filter_kernel<uint16_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)filter_smem_bytes(3072));
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(tf_filter_batch_kernel<uint8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)filter_smem_bytes(3072));
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(tf_filter_batch_kernel<uint16_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)filter_smem_bytes(3072));
   if (e != cudaSuccess) {
     tf_gpu_destroy(ctx);
     return e == cudaErrorMemoryAllocation ? TF_GPU_ERR_MEM : TF_GPU_ERR_CUDA;
@@ -1004,6 +1120,11 @@ void tf_gpu_destroy(tf_gpu_ctx *ctx) {
   if (ctx->ev_out_done) cudaEventDestroy(ctx->ev_out_done);
   for (int p = 0; p < 3; p++)
     if (ctx->out.base[p]) cudaFree(ctx->out.base[p]);
+  for (auto &b : ctx->bout)
+    for (int p = 0; p < 3; p++)
+      if (b.base[p]) cudaFree(b.base[p]);
+  if (ctx->d_bdiff) cudaFree(ctx->d_bdiff);
+  if (ctx->h_bdiff) cudaFreeHost(ctx->h_bdiff);
   for (int i = 0; i < 12; i++)
     if (ctx->d_dump[i]) cudaFree(ctx->d_dump[i]);
   for (int p = 0; p < 3; p++)
@@ -1024,6 +1145,7 @@ void tf_gpu_destroy(tf_gpu_ctx *ctx) {
     if (te.evk[1]) cudaEventDestroy(te.evk[1]);
   };
   drop_call_events(ctx->res_ev);
+  drop_call_events(ctx->batch_ev);
   for (int i = 0; i < 8; i++) drop_call_events(ctx->tickets[i].te);
   if (ctx->noise_stream) {
     cudaStreamSynchronize(ctx->noise_stream);
@@ -1300,6 +1422,114 @@ int tf_gpu_filter_resident(tf_gpu_ctx *ctx, const tf_gpu_params *params, const u
   return tf_gpu_filter_resident_result(ctx, diff_sum_sse, time_ms);
 }
 
+int tf_gpu_filter_batch_async(tf_gpu_ctx *ctx, int n, const tf_gpu_params *params, const uint64_t *const *frame_ids) {
+  static_assert(MAXB == TF_GPU_MAX_BATCH, "device batch size and ABI batch size must agree");
+  if (!ctx) return TF_GPU_ERR_INVALID;
+  // every check comes before anything is enqueued or pinned: a rejected batch leaves the context as it was
+  if (n < 1 || n > TF_GPU_MAX_BATCH) return fail(ctx, TF_GPU_ERR_INVALID, "batch of %d windows out of [1,%d]", n, TF_GPU_MAX_BATCH);
+  if (!params || !frame_ids) return fail(ctx, TF_GPU_ERR_INVALID, "params / frame_ids is NULL");
+  for (int w = 0; w < n; w++) {
+    const tf_gpu_params *p = &params[w];
+    if (!frame_ids[w]) return fail(ctx, TF_GPU_ERR_INVALID, "frame_ids[%d] is NULL", w);
+    int rc = validate_params(ctx, p);
+    if (rc) return rc;
+    if (p->out_row_end > p->out_row_begin)
+      return fail(ctx, TF_GPU_ERR_INVALID, "window %d: a batch filters whole frames (no out_row_begin / out_row_end)", w);
+    if (p->extend_output_borders)
+      return fail(ctx, TF_GPU_ERR_INVALID, "window %d: a batch does not extend output borders", w);
+  }
+  if (ctx->peer_out[0] || ctx->peer_out[1] || ctx->peer_out[2])
+    return fail(ctx, TF_GPU_ERR_INVALID, "an output plane is imported from another rank: a batch writes only its own outputs");
+  if (ctx->collect_counters) return fail(ctx, TF_GPU_ERR_INVALID, "work counters are not collected for batches");
+  {
+    uint64_t ids[TF_GPU_MAX_BATCH * TF_GPU_MAX_FRAMES];
+    int nd = 0;
+    for (int w = 0; w < n; w++)
+      for (int i = 0; i < params[w].num_frames; i++) {
+        int j = 0;
+        while (j < nd && ids[j] != frame_ids[w][i]) j++;
+        if (j == nd) ids[nd++] = frame_ids[w][i];
+      }
+    if (nd > (int)ctx->cache.size())
+      return fail(ctx, TF_GPU_ERR_INVALID, "the batch reads %d distinct frames, the frame cache holds %d", nd, (int)ctx->cache.size());
+  }
+  CU(cudaSetDevice(ctx->device));
+  DevFrame *devf[TF_GPU_MAX_BATCH][TF_GPU_MAX_FRAMES];
+  for (int w = 0; w < n; w++)
+    for (int i = 0; i < params[w].num_frames; i++) {
+      devf[w][i] = find_cached(ctx, frame_ids[w][i], nullptr);
+      if (!devf[w][i])
+        return fail(ctx, TF_GPU_ERR_INVALID, "window %d: frame id %llu is not resident", w, (unsigned long long)frame_ids[w][i]);
+      if (!(devf[w][i]->g == devf[0][0]->g)) return fail(ctx, TF_GPU_ERR_INVALID, "window %d: the frames of a batch must share one geometry", w);
+    }
+  const Geometry &g = devf[0][0]->g;
+  for (int w = 0; w < n; w++) {
+    const int rc = validate_geometry(ctx, &params[w], g);
+    if (rc) return rc;
+  }
+  CallScope scope(ctx);
+  ctx->last_launches = 0;
+  ctx->batch_n = 0;
+  for (int w = 0; w < n; w++)
+    for (int i = 0; i < params[w].num_frames; i++) {
+      DevFrame *d = devf[w][i];
+      if (d->pinned_epoch != ctx->epoch) CU(cudaStreamWaitEvent(ctx->stream, d->ready, 0));
+      d->last_use = ++ctx->use_counter;
+      d->pinned_epoch = ctx->epoch;
+    }
+  for (int w = 0; w < n; w++) {
+    const int rc = alloc_dev_frame(ctx, &ctx->bout[w], g);
+    if (rc) return rc;
+  }
+  if (!ctx->d_bdiff) CU(cudaMalloc(&ctx->d_bdiff, TF_GPU_MAX_BATCH * 2 * sizeof(unsigned long long)));
+  if (!ctx->h_bdiff) CU(cudaMallocHost(&ctx->h_bdiff, TF_GPU_MAX_BATCH * 2 * sizeof(unsigned long long)));
+  const int rc = launch_filter_batch(ctx, n, params, devf, g, &ctx->batch_ev);
+  if (rc) return rc;
+  CU(cudaMemcpyAsync(ctx->h_bdiff, ctx->d_bdiff, (size_t)n * 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
+  for (int w = 0; w < n; w++) ctx->batch_planes[w] = params[w].num_planes;
+  ctx->batch_n = n;
+  return TF_GPU_OK;
+}
+
+int tf_gpu_filter_batch_result(tf_gpu_ctx *ctx, int64_t (*diff_sum_sse)[2], float *time_ms) {
+  if (!ctx) return TF_GPU_ERR_INVALID;
+  if (!ctx->batch_n) return fail(ctx, TF_GPU_ERR_INVALID, "no batch has been enqueued");
+  CU(cudaSetDevice(ctx->device));
+  CU(cudaStreamSynchronize(ctx->stream));
+  if (diff_sum_sse)
+    for (int w = 0; w < ctx->batch_n; w++) {
+      diff_sum_sse[w][0] = (int64_t)ctx->h_bdiff[2 * w];
+      diff_sum_sse[w][1] = (int64_t)ctx->h_bdiff[2 * w + 1];
+    }
+  float ms = 0.f;
+  CU(cudaEventElapsedTime(&ms, ctx->batch_ev.ev0, ctx->batch_ev.ev1));
+  ctx->last_ev = &ctx->batch_ev;
+  ctx->last_kernel_ms = ms;
+  if (time_ms) *time_ms = ms;
+  return TF_GPU_OK;
+}
+
+int tf_gpu_download_batch_output(tf_gpu_ctx *ctx, int window, tf_gpu_frame *out) {
+  if (!ctx || !out) return TF_GPU_ERR_INVALID;
+  if (window < 0 || window >= ctx->batch_n) return fail(ctx, TF_GPU_ERR_INVALID, "window %d is not in the last batch (%d windows)", window, ctx->batch_n);
+  CU(cudaSetDevice(ctx->device));
+  const DevFrame &d = ctx->bout[window];
+  int rc = download_rows(ctx, d, out, 0, (d.g.crop_h[0] + 31) / 32, ctx->stream, ctx->batch_planes[window]);
+  if (rc) return rc;
+  CU(cudaStreamSynchronize(ctx->stream));
+  return TF_GPU_OK;
+}
+
+int tf_gpu_batch_output_device_plane(tf_gpu_ctx *ctx, int window, int plane, void **dptr, size_t *pitch_bytes,
+                                     int *rows, int *row_bytes) {
+  if (!ctx || plane < 0 || plane > 2) return TF_GPU_ERR_INVALID;
+  if (window < 0 || window >= ctx->batch_n) return fail(ctx, TF_GPU_ERR_INVALID, "window %d is not in the last batch (%d windows)", window, ctx->batch_n);
+  if (plane >= ctx->batch_planes[window] || !ctx->bout[window].p00[plane])
+    return fail(ctx, TF_GPU_ERR_INVALID, "window %d filters %d plane(s): no plane %d", window, ctx->batch_planes[window], plane);
+  device_plane(ctx->bout[window], plane, dptr, pitch_bytes, rows, row_bytes);
+  return TF_GPU_OK;
+}
+
 int tf_gpu_download_output(tf_gpu_ctx *ctx, tf_gpu_frame *out, int row_begin, int row_end) {
   if (!ctx || !out) return TF_GPU_ERR_INVALID;
   if (!ctx->out.base[0]) return fail(ctx, TF_GPU_ERR_INVALID, "no output on the device yet");
@@ -1311,7 +1541,7 @@ int tf_gpu_download_output(tf_gpu_ctx *ctx, tf_gpu_frame *out, int row_begin, in
   }
   if (row_begin < 0) row_begin = 0;
   if (row_end > mb_rows) row_end = mb_rows;
-  int rc = download_rows(ctx, out, row_begin, row_end, ctx->stream);
+  int rc = download_rows(ctx, ctx->out, out, row_begin, row_end, ctx->stream);
   if (rc) return rc;
   CU(cudaStreamSynchronize(ctx->stream));
   return TF_GPU_OK;
@@ -1320,13 +1550,7 @@ int tf_gpu_download_output(tf_gpu_ctx *ctx, tf_gpu_frame *out, int row_begin, in
 int tf_gpu_output_device_plane(tf_gpu_ctx *ctx, int plane, void **dptr, size_t *pitch_bytes, int *rows,
                                int *row_bytes) {
   if (!ctx || plane < 0 || plane > 2 || !ctx->out.p00[plane]) return TF_GPU_ERR_INVALID;
-  const Geometry &g = ctx->out.g;
-  const int k = plane > 0;
-  const size_t es = g.is_hbd ? 2 : 1;
-  if (dptr) *dptr = ctx->out.p00[plane];
-  if (pitch_bytes) *pitch_bytes = (size_t)g.pitch[k] * es;
-  if (rows) *rows = ((g.crop_h[0] + 31) / 32) * (32 >> (plane ? g.ss_y : 0));
-  if (row_bytes) *row_bytes = (int)(((g.crop_w[0] + 31) / 32) * (32 >> (plane ? g.ss_x : 0)) * es);
+  device_plane(ctx->out, plane, dptr, pitch_bytes, rows, row_bytes);
   return TF_GPU_OK;
 }
 

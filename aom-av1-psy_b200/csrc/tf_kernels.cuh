@@ -1608,11 +1608,11 @@ constexpr int S32_WARPS_HI = TF_S32_HI, S32_WARPS_HI_HBD = TF_S32_HI_HBD, S32_WA
 #endif
 constexpr int S16_WARPS = TF_S16_WARPS;
 template <typename T, int MINB>
-__global__ void __launch_bounds__(32, MINB) tf_search32_kernel(const __grid_constant__ KParams P) {
+__device__ __forceinline__ void search32_block(const KParams &P, const unsigned bid) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   const int lane = lane_id();
-  const int mb_row = P.row_begin + blockIdx.x / P.mb_cols;
-  const int mb_col = blockIdx.x % P.mb_cols;
+  const int mb_row = P.row_begin + bid / P.mb_cols;
+  const int mb_col = bid % P.mb_cols;
   const int blk = mb_row * P.mb_cols + mb_col;
   const int st = P.pitch[0];
   const int y_offset = mb_row * 32 * st + mb_col * 32;
@@ -1670,17 +1670,20 @@ __global__ void __launch_bounds__(32, MINB) tf_search32_kernel(const __grid_cons
     P.s_ref_mv[blk * 2 + 1] = (int16_t)ref_mv.col;
   }
 }
+template <typename T, int MINB>
+__global__ void __launch_bounds__(32, MINB) tf_search32_kernel(const __grid_constant__ KParams P) {
+  search32_block<T, MINB>(P, blockIdx.x);
+}
 
 // Kernel 2: every 16x16 sub-block search is an independent task
 // (frame, block, sub-block); it starts from the full-pel rounding of the
 // 32x32 result (temporal_filter.c:194) and reuses the 32x32 block's MV limits
 // (:202-205).  One warp per task, frame-major task order for L2 locality.
 template <typename T>
-__global__ void __launch_bounds__(32, S16_WARPS) tf_search16_kernel(const __grid_constant__ KParams P) {
+__device__ __forceinline__ void search16_task(const KParams &P, const int task) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   const int lane = lane_id();
   const int nblk = (P.row_end - P.row_begin) * P.mb_cols;
-  const int task = blockIdx.x;
   const int fidx = task / (nblk * 4);
   const int rem = task - fidx * nblk * 4;
   const int bl = rem >> 2, sub = rem & 3;
@@ -1710,6 +1713,10 @@ __global__ void __launch_bounds__(32, S16_WARPS) tf_search16_kernel(const __grid
     P.s_sub_mv[(bf * 4 + sub) * 2 + 1] = (int16_t)best.col;
     P.s_sub_mse[bf * 4 + sub] = (int)((err + 128u) / 256u);
   }
+}
+template <typename T>
+__global__ void __launch_bounds__(32, S16_WARPS) tf_search16_kernel(const __grid_constant__ KParams P) {
+  search16_task<T>(P, blockIdx.x);
 }
 
 // Batched full-pixel search (tf_gpu_fullpel_search_batch): one warp per item, the engine of the two
@@ -2130,13 +2137,13 @@ __device__ __forceinline__ WarpSmem carve_smem(unsigned char *raw, int num_pels)
 }
 
 template <typename T>
-__global__ void __launch_bounds__(FILT_THREADS, TF_FILT_MINB) tf_filter_kernel(const __grid_constant__ KParams P) {
+__device__ __forceinline__ void filter_block(const KParams &P, const unsigned bid) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   constexpr int NT = FILT_THREADS;
   const WarpSmem sm = carve_smem(smem_raw, P.num_pels);
   const int tid = threadIdx.x;
-  const int mb_row = P.row_begin + blockIdx.x / P.mb_cols;
-  const int mb_col = blockIdx.x % P.mb_cols;
+  const int mb_row = P.row_begin + bid / P.mb_cols;
+  const int mb_col = bid % P.mb_cols;
   const int blk = mb_row * P.mb_cols + mb_col;
   T *pred = reinterpret_cast<T *>(sm.pred);
 
@@ -2280,6 +2287,43 @@ __global__ void __launch_bounds__(FILT_THREADS, TF_FILT_MINB) tf_filter_kernel(c
       atomicAdd(&P.diff[1], (unsigned long long)((long long)sse32 * (long long)sse32));
     }
   }
+}
+template <typename T>
+__global__ void __launch_bounds__(FILT_THREADS, TF_FILT_MINB) tf_filter_kernel(const __grid_constant__ KParams P) {
+  filter_block<T>(P, blockIdx.x);
+}
+
+// ---------------------------------------------------------------------------
+// Batched windows (tf_gpu_filter_batch_async): several windows over one frame geometry in one grid per kernel,
+// blockIdx.y = window.  Each window's KParams carries its own frames, search scratch, output planes and FRAME_DIFF
+// slot, so the bodies above run unchanged.  The per-window parameters are the kernel parameter itself
+// (__grid_constant__): the window index is warp-uniform, so the window's fields are read with LDCU at a uniform-register
+// offset (blockIdx.y * sizeof(KParams)), constant-bank loads like the single-window kernels' immediate-offset ones, no
+// extra global traffic.  The host fills only the entries of the windows that have work for the kernel.
+// ---------------------------------------------------------------------------
+constexpr int MAXB = 16;  // TF_GPU_MAX_BATCH
+struct KParamsBatch {
+  KParams w[MAXB];
+};
+static_assert(sizeof(KParamsBatch) <= 32764, "the per-window parameters of a full batch must fit the kernel-parameter limit");
+
+// The 32x32 search of every frame of each window in one launch (the fused chain: the warp walks frames
+// [0, num_frames) of its (window, block)).
+template <typename T, int MINB>
+__global__ void __launch_bounds__(32, MINB) tf_search32_batch_kernel(const __grid_constant__ KParamsBatch B) {
+  search32_block<T, MINB>(B.w[blockIdx.y], blockIdx.x);
+}
+// The 16x16 tasks of every window: grid x covers the window with the most reference frames; the tasks beyond a
+// window's own reference frames exit at once.
+template <typename T>
+__global__ void __launch_bounds__(32, S16_WARPS) tf_search16_batch_kernel(const __grid_constant__ KParamsBatch B) {
+  const KParams &P = B.w[blockIdx.y];
+  if ((int)blockIdx.x >= (P.row_end - P.row_begin) * P.mb_cols * 4 * (P.num_frames - 1)) return;
+  search16_task<T>(P, blockIdx.x);
+}
+template <typename T>
+__global__ void __launch_bounds__(FILT_THREADS, TF_FILT_MINB) tf_filter_batch_kernel(const __grid_constant__ KParamsBatch B) {
+  filter_block<T>(B.w[blockIdx.y], blockIdx.x);
 }
 
 // ---------------------------------------------------------------------------

@@ -201,6 +201,32 @@ int tf_gpu_filter_resident(tf_gpu_ctx *ctx, const tf_gpu_params *params,
 int tf_gpu_filter_resident_async(tf_gpu_ctx *ctx, const tf_gpu_params *params, const uint64_t *frame_ids);
 int tf_gpu_filter_resident_result(tf_gpu_ctx *ctx, int64_t diff_sum_sse[2], float *time_ms);
 int tf_gpu_download_output(tf_gpu_ctx *ctx, tf_gpu_frame *out, int row_begin, int row_end);
+/* Batched windows: n windows over frames that are already resident, in one call and three kernel launches in all.
+ * A frame that several windows read -- the windows centred on every frame of a clip, the KF and ARF windows of one
+ * GOP -- is cached once, where one context per window (SURVEY 8e) caches it once per context.  Throughput
+ * (DESIGN.md §5): at 640x360 a batch is faster than several contexts in flight (up to +44 % at 16 windows); at
+ * 1080p and 4K it is faster than one window after another but 1-17 % slower than several contexts in flight.  Every window has
+ * its own params (num_frames, filter_frame_idx, noise levels, q_factor, strength, search settings,
+ * compute_frame_diff) and its own device output frame; all frames of a batch share one geometry.
+ * frame_ids[w] lists params[w].num_frames ids.  TF_GPU_ERR_INVALID, with nothing enqueued and the context unchanged,
+ * for: n outside [1, TF_GPU_MAX_BATCH]; a NULL array; a window that fails the checks of
+ * tf_gpu_filter_resident_async (params, ids resident, geometry); frames of different geometry; more distinct
+ * frames than the cache holds; a window with out_row_begin / out_row_end or extend_output_borders; an output
+ * plane imported with tf_gpu_output_ipc_import; counters enabled (tf_gpu_collect_counters).
+ * The batch's outputs are separate from the output of the single-window calls: neither overwrites the other.
+ * _result waits for the batch and returns each window's FRAME_DIFF (diff_sum_sse[w], nullable) and the device
+ * time of its three kernels.  The outputs stay valid until the next batch of this context. */
+#define TF_GPU_MAX_BATCH 16
+int tf_gpu_filter_batch_async(tf_gpu_ctx *ctx, int n, const tf_gpu_params *params /*[n]*/,
+                              const uint64_t *const *frame_ids /*[n][params[i].num_frames]*/);
+int tf_gpu_filter_batch_result(tf_gpu_ctx *ctx, int64_t (*diff_sum_sse)[2] /*[n], nullable*/, float *time_ms);
+/* Full blocks of window `window` of the last batch into `out` (as tf_gpu_download_output with all rows); only the
+ * window's own params.num_planes planes are written, so a luma-only window needs only out->plane[0]. */
+int tf_gpu_download_batch_output(tf_gpu_ctx *ctx, int window, tf_gpu_frame *out);
+/* As tf_gpu_output_device_plane, for window `window` of the last batch; TF_GPU_ERR_INVALID for a plane the window
+ * does not filter (plane >= its num_planes). */
+int tf_gpu_batch_output_device_plane(tf_gpu_ctx *ctx, int window, int plane, void **dptr, size_t *pitch_bytes,
+                                     int *rows, int *row_bytes);
 /* Raw device pointer + pitch (bytes) of an output plane, for NCCL gathers in
  * slab mode (the reference's counterpart is the shared tf_ctx->output_frame
  * written by all row workers, av1/encoder/ethread.c:2083-2108). */
