@@ -1835,8 +1835,9 @@ __device__ __noinline__ void convolve12(const KParams &P, const T *src, int ss, 
 
 // The same three variants for 16-bit containers with two samples per register.  The 12 taps of
 // MULTITAP_SHARP2 at a fractional position fit a signed byte (-26 .. 127; 128 only occurs at position 0,
-// which is the copy path), the samples (<= 4095) and the 2-D intermediate (< 2^15, convolve.c:96,
-// 149-174) fit a signed halfword, so one IDP.2A does two taps:
+// which is the copy path), the samples (<= 4095) fit a signed halfword, and the 2-D intermediate is narrowed
+// to one as the reference's int16_t im_block is (convolve.c:96; at 10 and 12 bit full-range content takes it
+// past 32767 and it wraps, here as there), so one IDP.2A does two taps:
 //   horizontal stage: a lane produces two adjacent outputs of a row from eight aligned words (the byte
 //     parity of the row start is uniform over the warp: one funnel shift per word pair), 12 IDP.2A;
 //   the intermediate is stored TRANSPOSED (im[col][row], column pitch h + 12), so the vertical stage reads

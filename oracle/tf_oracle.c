@@ -20,6 +20,11 @@
 static int clampi(int v, int lo, int hi) { return v < lo ? lo : (v > hi ? hi : v); }
 static int align_pow2(int v, int n) { return (v + (1 << n) - 1) & ~((1 << n) - 1); }
 
+/* Event counters (tf_oracle.h): observe only. */
+static tfo_stats g_stats;
+void tfo_reset_stats(void) { memset(&g_stats, 0, sizeof(g_stats)); }
+void tfo_get_stats(tfo_stats *out) { *out = g_stats; }
+
 typedef struct { int row, col; } mv_t; /* MV / FULLPEL_MV, av1/common/mv.h:37-47 */
 
 /* ------------------------------------------------------------------------- */
@@ -158,7 +163,7 @@ void tfo_get_output(tfo_ctx *c, int plane, uint16_t *dst, int w, int h) {
 /* ------------------------------------------------------------------------- */
 /* Noise estimate: temporal_filter.c:1150-1194                                */
 /* ------------------------------------------------------------------------- */
-static double estimate_noise(const uint16_t *src, int stride, int width, int height, int bd) {
+static double estimate_noise(const uint16_t *src, int stride, int width, int height, int bd, int edge_thresh) {
   int64_t accum = 0;
   int count = 0;
   for (int i = 1; i < height - 1; ++i) {
@@ -170,7 +175,7 @@ static double estimate_noise(const uint16_t *src, int stride, int width, int hei
       const int Gx = (a - c) + (g - k) + 2 * (d - f);
       const int Gy = (a - g) + (c - k) + 2 * (b - h);
       const int Ga = RPOT(abs(Gx) + abs(Gy), bd - 8);
-      if (Ga < 50) {
+      if (Ga < edge_thresh) {
         const int v = 4 * e - 2 * (b + h + d + f) + (a + c + g + k);
         accum += RPOT(abs(v), bd - 8);
         ++count;
@@ -179,11 +184,13 @@ static double estimate_noise(const uint16_t *src, int stride, int width, int hei
   }
   return (count < 16) ? -1.0 : (double)accum / (6 * count) * 1.25331413732;
 }
-double tfo_estimate_noise(tfo_ctx *c, int idx, int plane) {
+/* edge_thresh: NOISE_ESTIMATION_EDGE_THRESHOLD (50, temporal_filter.h:79) unless the caller passes another */
+double tfo_estimate_noise_thresh(tfo_ctx *c, int idx, int plane, int edge_thresh) {
   const frame_t *f = &c->frames[idx];
   const int k = plane > 0;
-  return estimate_noise(f->buf[plane], f->stride[k], f->crop_w[k], f->crop_h[k], c->p.bit_depth);
+  return estimate_noise(f->buf[plane], f->stride[k], f->crop_w[k], f->crop_h[k], c->p.bit_depth, edge_thresh);
 }
+double tfo_estimate_noise(tfo_ctx *c, int idx, int plane) { return tfo_estimate_noise_thresh(c, idx, plane, 50); }
 
 /* ------------------------------------------------------------------------- */
 /* SAD / variance primitives                                                  */
@@ -195,8 +202,16 @@ unsigned tfo_sad(const uint16_t *a, int as, const uint16_t *b, int bs, int w, in
                  int bd, int use_hbd) {
   unsigned s = 0;
   const int step = skip ? 2 : 1;
-  for (int y = 0; y < h; y += step)
-    for (int x = 0; x < w; x++) s += abs((int)a[y * as + x] - (int)b[y * bs + x]);
+  const int maxd = (1 << (use_hbd ? bd : 8)) - 1;
+  for (int y = 0; y < h; y += step) {
+    int peak = 0;
+    for (int x = 0; x < w; x++) {
+      const int d = abs((int)a[y * as + x] - (int)b[y * bs + x]);
+      s += d;
+      peak += d == maxd;
+      if ((x & 15) == 15) { g_stats.sad_peak_groups += peak == 16; peak = 0; }
+    }
+  }
   if (skip) s *= 2;
   if (use_hbd) s >>= (bd == 10 ? 2 : (bd == 12 ? 4 : 0));
   return s;
@@ -270,6 +285,12 @@ static const int16_t k12[16][12] = {
 };
 
 static uint16_t clip_px(int v, int bd) { const int m = (1 << bd) - 1; return (uint16_t)(v < 0 ? 0 : (v > m ? m : v)); }
+/* clip_px of the predictor, counted */
+static uint16_t clip_pred(int v, int bd) {
+  g_stats.pred_clip_lo += v < 0;
+  g_stats.pred_clip_hi += v > (1 << bd) - 1;
+  return clip_px(v, bd);
+}
 
 void tfo_convolve12(const uint16_t *src, int ss, uint16_t *dst, int ds, int w, int h,
                     int subpel_x, int subpel_y, int bd, int use_hbd) {
@@ -289,7 +310,7 @@ void tfo_convolve12(const uint16_t *src, int ss, uint16_t *dst, int ds, int w, i
         int32_t res = 0;
         for (int k = 0; k < 12; k++) res += f[k] * src[y * ss + x - fo + k];
         res = RPOT(res, r0);
-        dst[y * ds + x] = clip_px(RPOT(res, bits), pbd);
+        dst[y * ds + x] = clip_pred(RPOT(res, bits), pbd);
       }
   } else if (!subpel_x && subpel_y) { /* convolve.c:128-147 / :596-614 */
     const int16_t *f = k12[subpel_y];
@@ -297,7 +318,7 @@ void tfo_convolve12(const uint16_t *src, int ss, uint16_t *dst, int ds, int w, i
       for (int x = 0; x < w; x++) {
         int32_t res = 0;
         for (int k = 0; k < 12; k++) res += f[k] * src[(y - fo + k) * ss + x];
-        dst[y * ds + x] = clip_px(RPOT(res, 7), pbd);
+        dst[y * ds + x] = clip_pred(RPOT(res, 7), pbd);
       }
   } else { /* convolve.c:76-126 / :616-668 */
     int16_t im[(32 + 11) * 32];
@@ -309,6 +330,7 @@ void tfo_convolve12(const uint16_t *src, int ss, uint16_t *dst, int ds, int w, i
       for (int x = 0; x < w; x++) {
         int32_t sum = 1 << (pbd + 7 - 1);
         for (int k = 0; k < 12; k++) sum += fx[k] * sh[y * ss + x - fo + k];
+        g_stats.conv_im_overflow += RPOT(sum, r0) < INT16_MIN || RPOT(sum, r0) > INT16_MAX;
         im[y * w + x] = (int16_t)RPOT(sum, r0);
       }
     const int ob = pbd + 14 - r0;
@@ -318,7 +340,7 @@ void tfo_convolve12(const uint16_t *src, int ss, uint16_t *dst, int ds, int w, i
         for (int k = 0; k < 12; k++) sum += fy[k] * im[(y + k) * w + x];
         int32_t res = RPOT(sum, r1) - ((1 << (ob - r1)) + (1 << (ob - r1 - 1)));
         if (!use_hbd) res = (int16_t)res; /* convolve.c:120 keeps it in an int16_t */
-        dst[y * ds + x] = clip_px(RPOT(res, bits), pbd);
+        dst[y * ds + x] = clip_pred(RPOT(res, bits), pbd);
       }
   }
 }
@@ -564,6 +586,7 @@ static unsigned diamond_search(const search_t *s, mv_t start, int search_step, i
       const int r = best_mv->row + site[idx].row, c = best_mv->col + site[idx].col;
       if (!all_in && !in_range(&s->lim, r, c)) continue;
       unsigned thissad = s_sad(s, r, c, skip);
+      g_stats.diamond_ties += thissad + sad_cost(s, r, c) == bestsad;
       if (thissad < bestsad) {
         thissad += sad_cost(s, r, c);
         if (thissad < bestsad) { bestsad = thissad; best_site = idx; }
@@ -608,6 +631,7 @@ static int full_pixel_diamond(const search_t *s, mv_t start, int step_param, int
 
 /* update_mvs_and_sad mcomp.c:839-858 */
 static void upd(const search_t *s, unsigned this_sad, int r, int c, unsigned *best_sad, mv_t *best) {
+  g_stats.mesh_ties += this_sad + sad_cost(s, r, c) == *best_sad;
   if (this_sad >= *best_sad) return;
   const unsigned sad = this_sad + sad_cost(s, r, c);
   if (sad < *best_sad) { *best_sad = sad; best->row = r; best->col = c; }
@@ -646,6 +670,7 @@ static int full_pixel_exhaustive(const search_t *s, mv_t start, int skip, mv_t *
   int interval = p->mesh[0][1], range = p->mesh[0][0];
   *best_mv = start;
   if (range < 7 || range > 256 || interval < 1 || interval > range) return INT_MAX;
+  g_stats.mesh_searches++;
   const int baseline_interval_divisor = range / interval;
   range = MAXI(range, (5 * MAXI(abs(best_mv->row), abs(best_mv->col))) / 4);
   range = MINI(range, 256);
@@ -768,6 +793,7 @@ static unsigned check_better(subpel_t *sp, int r8, int c8, int accurate, int *is
   if (!in_range(&sp->lim, r8, c8)) return INT_MAX;
   unsigned sse;
   const unsigned cost = accurate ? upsampled_err(sp->s, r8, c8, &sse) : bilinear_err(sp->s, r8, c8, &sse);
+  g_stats.subpel_ties += cost == sp->besterr;
   if (cost < sp->besterr) {
     sp->besterr = cost;
     sp->best.row = r8; sp->best.col = c8;
@@ -916,6 +942,14 @@ void tfo_full_pixel_search(tfo_ctx *c, int src_idx, int ref_idx, int bsize, int 
   out[1] = best.col;
 }
 
+/* counters only: a full-pel MV on a search limit, and whether the +-1023 clamp set that limit */
+static void count_on_limit(const limits_t *l, mv_t mv) {
+  const int rl = mv.row == l->row_min || mv.row == l->row_max;
+  const int cl = mv.col == l->col_min || mv.col == l->col_max;
+  g_stats.mv_on_limit += rl || cl;
+  g_stats.mv_on_clamp += (mv.row == -1023 || mv.row == 1023 || mv.col == -1023 || mv.col == 1023) && (rl || cl);
+}
+
 /* tf_motion_search temporal_filter.c:87-253 */
 static void motion_search(const tfo_ctx *c, const sites_t *sites, const frame_t *cur, const frame_t *ref,
                           int mb_row, int mb_col, mv_t *ref_mv, mv_t *sub_mvs, int *sub_mses) {
@@ -934,6 +968,7 @@ static void motion_search(const tfo_ctx *c, const sites_t *sites, const frame_t 
   s.w = s.h = 32;
   mv_t best_full;
   full_pixel_search(&s, start, step_param, skip, &best_full);
+  count_on_limit(&s.lim, best_full);
   int block_mse;
   mv_t block_mv;
   if (p->force_integer_mv == 1) {
@@ -956,6 +991,7 @@ static void motion_search(const tfo_ctx *c, const sites_t *sites, const frame_t 
         s.ref = ref->buf[0] + y_offset + i * st + j;
         s.w = s.h = 16;
         full_pixel_search(&s, start, step_param, skip, &best_full);
+        count_on_limit(&s.lim, best_full);
         err = subpel_search(&s, best_full, &best);
         sub_mses[idx] = (int)((err + 128) / 256);
         sub_mvs[idx] = best;
@@ -971,7 +1007,8 @@ static void motion_search(const tfo_ctx *c, const sites_t *sites, const frame_t 
     for (int i = 0; i < 4; i++) { sub_mvs[i] = block_mv; sub_mses[i] = block_mse; }
   }
   const int thresh = (min_frame_size >= 720) ? 12 : 3;
-  if (block_mse > (thresh << (p->bit_depth - 8))) { ref_mv->row = 0; ref_mv->col = 0; }
+  g_stats.block_mse_at_thresh += block_mse == (thresh << (p->bit_depth - 8));
+  if (block_mse > (thresh << (p->bit_depth - 8))) { ref_mv->row = 0; ref_mv->col = 0; g_stats.ref_mv_resets++; }
 }
 
 /* av1_tf_do_filtering_row temporal_filter.c:788-939 for rows [row_begin,row_end) */

@@ -42,6 +42,8 @@ void tfo_destroy(tfo_ctx *c);
 /* planes: crop-sized, tightly packed, u8 (use_hbd=0) or u16 (use_hbd=1) */
 void tfo_set_frame(tfo_ctx *c, int idx, const void *y, const void *u, const void *v);
 double tfo_estimate_noise(tfo_ctx *c, int idx, int plane);
+/* av1_estimate_noise_from_single_plane with an explicit edge_thresh (tfo_estimate_noise passes 50) */
+double tfo_estimate_noise_thresh(tfo_ctx *c, int idx, int plane, int edge_thresh);
 /* Runs block rows [row_begin,row_end). Recorders may be NULL:
  *  mvs  [blocks][frames][4][2] int16 (row,col); mses [blocks][frames][4] int32;
  *  pred [blocks][frames][num_pels] u16; accum/count [blocks][num_pels]. */
@@ -81,6 +83,26 @@ unsigned tfo_subpel_variance(const uint16_t *ref, int rs, int xoff, int yoff,
 void tfo_convolve12(const uint16_t *src, int ss, uint16_t *dst, int ds, int w, int h,
                     int subpel_x, int subpel_y, int bd, int use_hbd);
 int tfo_od_divu(unsigned x, unsigned d);
+
+/* Event counters: they only observe, never change a result.  They show that a test input reaches the
+ * regime it targets (exact ties, int16 wrap of the 2-D intermediate, clamped predictor samples, ...).
+ * One process-wide set; tfo_reset_stats() zeroes it. */
+typedef struct {
+  int64_t mesh_searches;      /* full_pixel_exhaustive calls that run the mesh (range/interval valid) */
+  int64_t diamond_ties;       /* diamond candidates whose sad + cost equals the incumbent (strict < keeps it) */
+  int64_t mesh_ties;          /* mesh candidates whose sad + cost equals the incumbent */
+  int64_t subpel_ties;        /* sub-pel candidates whose error equals the incumbent */
+  int64_t conv_im_overflow;   /* 2-D convolve intermediates outside int16 before the cast */
+  int64_t pred_clip_lo;       /* predictor samples clamped to 0 by clip_px */
+  int64_t pred_clip_hi;       /* predictor samples clamped to (1 << bd) - 1 by clip_px */
+  int64_t mv_on_limit;        /* full-pel MVs (32x32 and 16x16) on a row or column search limit */
+  int64_t mv_on_clamp;        /* of those, on a limit set by the +-1023 clamp */
+  int64_t ref_mv_resets;      /* block_mse > thresh: ref_mv reset to zero */
+  int64_t block_mse_at_thresh; /* block_mse == thresh exactly (the reset's boundary) */
+  int64_t sad_peak_groups;    /* 16-sample aligned row groups of a SAD whose every |difference| is (1 << bd) - 1 */
+} tfo_stats;
+void tfo_reset_stats(void);
+void tfo_get_stats(tfo_stats *out);
 
 #ifdef __cplusplus
 }

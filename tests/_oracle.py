@@ -28,6 +28,15 @@ class OParams(C.Structure):
     ]
 
 
+STAT_FIELDS = ("mesh_searches", "diamond_ties", "mesh_ties", "subpel_ties", "conv_im_overflow", "pred_clip_lo",
+               "pred_clip_hi", "mv_on_limit", "mv_on_clamp", "ref_mv_resets", "block_mse_at_thresh",
+               "sad_peak_groups")
+
+
+class OStats(C.Structure):
+    _fields_ = [(k, C.c_int64) for k in STAT_FIELDS]
+
+
 _lib = None
 
 
@@ -47,6 +56,8 @@ def lib():
         l.tfo_set_frame.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
         l.tfo_estimate_noise.restype = C.c_double
         l.tfo_estimate_noise.argtypes = [C.c_void_p, C.c_int, C.c_int]
+        l.tfo_estimate_noise_thresh.restype = C.c_double
+        l.tfo_estimate_noise_thresh.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int]
         l.tfo_run.argtypes = [C.c_void_p, C.c_int, C.c_int] + [C.c_void_p] * 6
         l.tfo_get_output.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int]
         l.tfo_get_plane_with_border.restype = C.c_int
@@ -65,12 +76,28 @@ def lib():
                                           + [C.c_int] * 4 + [C.POINTER(C.c_uint)])
         l.tfo_convolve12.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int] + [C.c_int] * 6
         l.tfo_od_divu.argtypes = [C.c_uint, C.c_uint]
+        l.tfo_reset_stats.argtypes = []
+        l.tfo_reset_stats.restype = None
+        l.tfo_get_stats.argtypes = [C.POINTER(OStats)]
+        l.tfo_get_stats.restype = None
         _lib = l
     return _lib
 
 
 def _ptr(a):
     return None if a is None else a.ctypes.data_as(C.c_void_p)
+
+
+def reset_stats():
+    """Zero the oracle's event counters (process-wide)."""
+    lib().tfo_reset_stats()
+
+
+def get_stats():
+    """The oracle's event counters since the last reset_stats(), as a dict (see tfo_stats in tf_oracle.h)."""
+    st = OStats()
+    lib().tfo_get_stats(C.byref(st))
+    return {k: int(getattr(st, k)) for k in STAT_FIELDS}
 
 
 def make_params(p):
@@ -103,9 +130,9 @@ class OracleFilter:
             vs = None if v is None else np.ascontiguousarray(v.astype(dt))
             lib().tfo_set_frame(self.h, i, _ptr(ys), _ptr(us), _ptr(vs))
 
-    def estimate_noise(self, idx=None):
+    def estimate_noise(self, idx=None, edge_thresh=50):
         idx = self.p["filter_frame_idx"] if idx is None else idx
-        return [lib().tfo_estimate_noise(self.h, idx, pl) for pl in range(self.num_planes)]
+        return [lib().tfo_estimate_noise_thresh(self.h, idx, pl, edge_thresh) for pl in range(self.num_planes)]
 
     def run(self, record=True, rows=None):
         nb = self.mb_rows * self.mb_cols
