@@ -35,7 +35,7 @@ EXPORTS = [
     "tf_gpu_cache_frame_async", "tf_gpu_debug_read_plane", "tf_gpu_device_border", "tf_gpu_fullpel_search_batch",
     "tf_gpu_output_ipc_export", "tf_gpu_output_ipc_import", "tf_gpu_cache_frame_device",
     "tf_gpu_filter_batch_async", "tf_gpu_filter_batch_result", "tf_gpu_download_batch_output",
-    "tf_gpu_batch_output_device_plane",
+    "tf_gpu_batch_output_device_plane", "tf_gpu_motion_search_batch",
 ]
 
 
@@ -80,6 +80,27 @@ class SearchResult(C.Structure):
     _fields_ = [("row", C.c_int16), ("col", C.c_int16), ("var", C.c_int32)]
 
 
+class MotionItem(C.Structure):
+    """tf_gpu_motion_item: one block of the source searched against references[ref]."""
+    _fields_ = [("x", C.c_int), ("y", C.c_int), ("start_row", C.c_int16), ("start_col", C.c_int16),
+                ("ref", C.c_int32)]
+
+
+class MotionResult(C.Structure):
+    """tf_gpu_motion_result: the full-pel result and the final 1/8-pel MV with its error."""
+    _fields_ = [("fullpel_row", C.c_int16), ("fullpel_col", C.c_int16), ("fullpel_var", C.c_int32),
+                ("row", C.c_int16), ("col", C.c_int16), ("err", C.c_uint32)]
+
+
+# numpy views of the two structs above, so that large batches are packed and unpacked without a Python loop
+_MOTION_ITEM_DTYPE = np.dtype([("x", "<i4"), ("y", "<i4"), ("start_row", "<i2"), ("start_col", "<i2"),
+                               ("ref", "<i4")])
+_MOTION_RESULT_DTYPE = np.dtype([("fullpel_row", "<i2"), ("fullpel_col", "<i2"), ("fullpel_var", "<i4"),
+                                 ("row", "<i2"), ("col", "<i2"), ("err", "<u4")])
+assert _MOTION_ITEM_DTYPE.itemsize == C.sizeof(MotionItem) == 16
+assert _MOTION_RESULT_DTYPE.itemsize == C.sizeof(MotionResult) == 16
+
+
 class Dump(C.Structure):
     _fields_ = [("subblock_mvs", C.c_void_p), ("subblock_mses", C.c_void_p), ("pred", C.c_void_p),
                 ("accum", C.c_void_p), ("count", C.c_void_p)]
@@ -118,6 +139,8 @@ def load_library():
     lib.tf_gpu_output_ipc_import.argtypes = [vp, i, C.c_char_p, C.c_size_t, C.c_size_t]
     lib.tf_gpu_fullpel_search_batch.argtypes = [vp, C.POINTER(Params), C.POINTER(Frame), C.POINTER(Frame), i,
                                                 C.POINTER(SearchItem), i, C.POINTER(SearchResult)]
+    lib.tf_gpu_motion_search_batch.argtypes = [vp, C.POINTER(Params), u64, C.POINTER(u64), i, i,
+                                               C.POINTER(MotionItem), i, C.POINTER(MotionResult)]
     lib.tf_gpu_filter_resident.argtypes = [vp, C.POINTER(Params), C.POINTER(u64), C.POINTER(C.c_int64),
                                            C.POINTER(C.c_float)]
     lib.tf_gpu_download_output.argtypes = [vp, C.POINTER(Frame), i, i]
@@ -325,6 +348,39 @@ def batch_args(params_list, frame_ids_list):
     return n, params, ptrs, ids
 
 
+def motion_search_args(ref_ids, block_size, items):
+    """Arguments of tf_gpu_motion_search_batch: (uint64_t ref_ids[num_refs], num_refs, items, n), items packed as
+    tf_gpu_motion_item[n] in a numpy array.  items: integer array-like of shape (n, 5) = x, y, start_row, start_col,
+    ref (an empty sequence is n = 0).  Raises ValueError, before anything reaches the library, for items of another
+    shape or a non-integer dtype, x / y outside int32, starts outside int16, a ref outside [0, num_refs), 0 or more
+    than TF_GPU_MAX_FRAMES - 1 references, and a block size other than 16 or 32.  The block positions are checked by
+    the library, which knows the frame size."""
+    if block_size not in (16, 32):
+        raise ValueError(f"block_size must be 16 or 32, got {block_size}")
+    ids = [int(r) for r in ref_ids]
+    if not 1 <= len(ids) <= TF_GPU_MAX_FRAMES - 1:
+        raise ValueError(f"1 to {TF_GPU_MAX_FRAMES - 1} reference frames, got {len(ids)}")
+    a = np.asarray(items)
+    if a.ndim == 1 and a.size == 0:
+        a = a.reshape(0, 5).astype(np.int64)
+    if a.ndim != 2 or a.shape[1] != 5:
+        raise ValueError(f"items must have shape (n, 5) (x, y, start_row, start_col, ref), got {a.shape}")
+    if not np.issubdtype(a.dtype, np.integer):
+        raise ValueError(f"items must be integers, got dtype {a.dtype}")
+    a = a.astype(np.int64)
+    i16, i32 = np.iinfo(np.int16), np.iinfo(np.int32)
+    if ((a[:, 0:2] < i32.min) | (a[:, 0:2] > i32.max)).any():
+        raise ValueError("item positions must fit in int32")
+    if ((a[:, 2:4] < i16.min) | (a[:, 2:4] > i16.max)).any():
+        raise ValueError("start MVs must fit in int16")
+    if ((a[:, 4] < 0) | (a[:, 4] >= len(ids))).any():
+        raise ValueError(f"item ref out of [0, {len(ids)})")
+    packed = np.zeros(len(a), _MOTION_ITEM_DTYPE)
+    for k, name in enumerate(_MOTION_ITEM_DTYPE.names):
+        packed[name] = a[:, k]
+    return (C.c_uint64 * len(ids))(*ids), len(ids), packed, len(a)
+
+
 class TemporalFilterGpu:
     """One tf_gpu_ctx (CUDA device + stream + frame cache)."""
 
@@ -529,6 +585,19 @@ class TemporalFilterGpu:
         cs, cr = src.c_frame(), ref.c_frame()
         self._check(self.lib.tf_gpu_fullpel_search_batch(self.h, C.byref(cp), C.byref(cs), C.byref(cr), block_size, arr, n, res))
         return np.array([(r.row, r.col, r.var) for r in res[:n]], np.int64).reshape(n, 3)
+
+    def motion_search_batch(self, params, src_id, ref_ids, block_size, items):
+        """tf_motion_search()'s search of many blocks of the resident frame src_id against the resident frames
+        ref_ids (uploaded or ingested from tensors) in one call: see tf_gpu_motion_search_batch in tf_gpu.h and
+        motion_search_args for items.  Returns an int64 array (n, 6): fullpel_row, fullpel_col, fullpel_var, row,
+        col (1/8 pel), err."""
+        cp = make_params(params) if isinstance(params, dict) else params
+        ids, num_refs, packed, n = motion_search_args(ref_ids, block_size, items)
+        res = np.zeros(max(n, 1), _MOTION_RESULT_DTYPE)
+        self._check(self.lib.tf_gpu_motion_search_batch(
+            self.h, C.byref(cp), int(src_id), ids, num_refs, block_size,
+            C.cast(packed.ctypes.data, C.POINTER(MotionItem)), n, C.cast(res.ctypes.data, C.POINTER(MotionResult))))
+        return np.stack([res[k][:n].astype(np.int64) for k in _MOTION_RESULT_DTYPE.names], axis=1).reshape(n, 6)
 
     def device_border(self):
         return self.lib.tf_gpu_device_border()

@@ -86,7 +86,7 @@ struct tf_gpu_ctx {
   bool done_valid[2] = { false, false };
   cudaEvent_t ev_f32[TF_GPU_MAX_FRAMES] = {};
   cudaEvent_t ev_s16 = nullptr;
-  cudaEvent_t ev0 = nullptr, ev1 = nullptr;   // microbenchmark timing
+  cudaEvent_t ev0 = nullptr, ev1 = nullptr;   // microbenchmark and motion-search kernel timing
   CallEvents res_ev;                          // resident path
   const CallEvents *last_ev = nullptr;        // events of the last completed filter call
   bool split_valid = false;
@@ -127,9 +127,9 @@ struct tf_gpu_ctx {
   int batch_n = 0;                        // windows of the last batch enqueued (0: none, or it failed)
   int batch_planes[TF_GPU_MAX_BATCH] = {}; // planes each window writes (its num_planes; bout[w] may hold more)
   CallEvents batch_ev;
-  // dump buffers (device), grown on demand
-  void *d_dump[12] = {};
-  size_t d_dump_sz[12] = {};
+  // dump buffers (device), grown on demand; 10, 11: full-pel search items / results, 12, 13: motion search
+  void *d_dump[14] = {};
+  size_t d_dump_sz[14] = {};
   char err[512] = { 0 };
 };
 
@@ -1125,7 +1125,7 @@ void tf_gpu_destroy(tf_gpu_ctx *ctx) {
       if (b.base[p]) cudaFree(b.base[p]);
   if (ctx->d_bdiff) cudaFree(ctx->d_bdiff);
   if (ctx->h_bdiff) cudaFreeHost(ctx->h_bdiff);
-  for (int i = 0; i < 12; i++)
+  for (int i = 0; i < (int)(sizeof(ctx->d_dump) / sizeof(ctx->d_dump[0])); i++)
     if (ctx->d_dump[i]) cudaFree(ctx->d_dump[i]);
   for (int p = 0; p < 3; p++)
     if (ctx->peer_base[p]) cudaIpcCloseMemHandle(ctx->peer_base[p]);
@@ -1588,6 +1588,28 @@ int tf_gpu_output_ipc_import(tf_gpu_ctx *ctx, int plane, const unsigned char *ha
   return TF_GPU_OK;
 }
 
+namespace {
+
+// The params of a batched search: the caller's search fields, and window fields that validate_params accepts --
+// frame 0 the source, frames 1 .. num_frames - 1 the references, luma only.
+tf_gpu_params search_params(const tf_gpu_params &in, int num_frames) {
+  tf_gpu_params p = in;
+  p.num_frames = num_frames;
+  p.filter_frame_idx = 0;
+  p.num_planes = 1;
+  return p;
+}
+
+// A batched search item's block starts inside the mi grid (it may stick out of it like the last 32x32 row of a
+// 1080p frame); the SAD engine reads source rows with 16-byte loads.
+int check_item_position(tf_gpu_ctx *ctx, const tf_gpu_params &p, int i, int x, int y) {
+  if (x < 0 || y < 0 || (x & 15) || (y & 3) || x >= p.mi_cols * 4 || y >= p.mi_rows * 4)
+    return fail(ctx, TF_GPU_ERR_INVALID, "item %d: block position (%d, %d) not supported", i, x, y);
+  return TF_GPU_OK;
+}
+
+}  // namespace
+
 int tf_gpu_fullpel_search_batch(tf_gpu_ctx *ctx, const tf_gpu_params *params, const tf_gpu_frame *src,
                                 const tf_gpu_frame *ref, int block_size, const tf_gpu_search_item *items, int n,
                                 tf_gpu_search_result *results) {
@@ -1598,10 +1620,7 @@ int tf_gpu_fullpel_search_batch(tf_gpu_ctx *ctx, const tf_gpu_params *params, co
   if (n == 0) return TF_GPU_OK;
   static_assert(sizeof(tf_gpu_search_item) == sizeof(SearchItem) && sizeof(tf_gpu_search_result) == sizeof(SearchResult),
                 "ABI structs and device structs must agree");
-  tf_gpu_params p = *params;  // only the search fields are read; make the window fields valid
-  p.num_frames = 2;
-  p.filter_frame_idx = 0;
-  p.num_planes = 1;
+  tf_gpu_params p = search_params(*params, 2);  // only the search fields are read
   if (p.subpel_iters_per_step < 1) p.subpel_iters_per_step = 1;
   int rc = validate_params(ctx, &p);
   if (rc) return rc;
@@ -1618,11 +1637,8 @@ int tf_gpu_fullpel_search_batch(tf_gpu_ctx *ctx, const tf_gpu_params *params, co
   rc = validate_geometry(ctx, &p, g);
   if (rc) return rc;
   for (int i = 0; i < n; i++) {
-    const tf_gpu_search_item &it = items[i];
-    // the block starts inside the mi grid (it may stick out of it like the last 32x32 row of a 1080p frame);
-    // the SAD engine reads source rows with 16-byte loads
-    if (it.x < 0 || it.y < 0 || (it.x & 15) || (it.y & 3) || it.x >= p.mi_cols * 4 || it.y >= p.mi_rows * 4)
-      return fail(ctx, TF_GPU_ERR_INVALID, "item %d: block position (%d, %d) not supported", i, it.x, it.y);
+    rc = check_item_position(ctx, p, i, items[i].x, items[i].y);
+    if (rc) return rc;
   }
   KParams K;
   fill_kparams(ctx, &p, g, K);
@@ -1649,6 +1665,79 @@ int tf_gpu_fullpel_search_batch(tf_gpu_ctx *ctx, const tf_gpu_params *params, co
   ctx->last_launches++;
   CU(cudaMemcpyAsync(results, d_res, (size_t)n * sizeof(SearchResult), cudaMemcpyDeviceToHost, ctx->stream));
   CU(cudaStreamSynchronize(ctx->stream));
+  return TF_GPU_OK;
+}
+
+int tf_gpu_motion_search_batch(tf_gpu_ctx *ctx, const tf_gpu_params *params, uint64_t src_id, const uint64_t *ref_ids,
+                               int num_refs, int block_size, const tf_gpu_motion_item *items, int n,
+                               tf_gpu_motion_result *results) {
+  static_assert(sizeof(tf_gpu_motion_item) == sizeof(MotionItem) && sizeof(tf_gpu_motion_result) == sizeof(MotionResult),
+                "ABI structs and device structs must agree");
+  if (!ctx) return TF_GPU_ERR_INVALID;
+  // every check comes before anything is enqueued or pinned: a rejected call leaves the context as it was
+  if (!params || !ref_ids || !items || !results) return fail(ctx, TF_GPU_ERR_INVALID, "NULL argument");
+  if (block_size != 16 && block_size != 32) return fail(ctx, TF_GPU_ERR_INVALID, "block_size must be 16 or 32");
+  if (n < 0) return fail(ctx, TF_GPU_ERR_INVALID, "negative item count");
+  if (num_refs < 1 || num_refs > TF_GPU_MAX_FRAMES - 1)
+    return fail(ctx, TF_GPU_ERR_INVALID, "num_refs %d out of [1,%d]", num_refs, TF_GPU_MAX_FRAMES - 1);
+  if (n == 0) return TF_GPU_OK;
+  const tf_gpu_params p = search_params(*params, 1 + num_refs);
+  int rc = validate_params(ctx, &p);
+  if (rc) return rc;
+  DevFrame *devf[TF_GPU_MAX_FRAMES];
+  for (int f = 0; f <= num_refs; f++) {
+    const uint64_t id = f ? ref_ids[f - 1] : src_id;
+    devf[f] = find_cached(ctx, id, nullptr);
+    if (!devf[f]) return fail(ctx, TF_GPU_ERR_INVALID, "frame id %llu is not resident", (unsigned long long)id);
+    if (!(devf[f]->g == devf[0]->g)) return fail(ctx, TF_GPU_ERR_INVALID, "the source and references must share one geometry");
+  }
+  const Geometry &g = devf[0]->g;
+  rc = validate_geometry(ctx, &p, g);
+  if (rc) return rc;
+  for (int i = 0; i < n; i++) {
+    rc = check_item_position(ctx, p, i, items[i].x, items[i].y);
+    if (rc) return rc;
+    if (items[i].ref < 0 || items[i].ref >= num_refs)
+      return fail(ctx, TF_GPU_ERR_INVALID, "item %d: ref %d out of [0,%d)", i, (int)items[i].ref, num_refs);
+  }
+  CU(cudaSetDevice(ctx->device));
+  CallScope scope(ctx);
+  ctx->last_launches = 0;
+  for (int f = 0; f <= num_refs; f++) {
+    DevFrame *d = devf[f];
+    if (d->pinned_epoch != ctx->epoch) CU(cudaStreamWaitEvent(ctx->stream, d->ready, 0));
+    d->last_use = ++ctx->use_counter;
+    d->pinned_epoch = ctx->epoch;
+  }
+  KParams K;
+  fill_kparams(ctx, &p, g, K);
+  for (int f = 0; f <= num_refs; f++) {
+    K.frm[f][0] = devf[f]->p00[0];
+    K.tmap[f] = devf[f]->d_tmap;  // TF_FAR_TMA builds: each reference's own descriptors
+  }
+  rc = ensure_dump(ctx, 12, (size_t)n * sizeof(MotionItem));
+  if (rc) return rc;
+  rc = ensure_dump(ctx, 13, (size_t)n * sizeof(MotionResult));
+  if (rc) return rc;
+  MotionItem *d_items = (MotionItem *)ctx->d_dump[12];
+  MotionResult *d_res = (MotionResult *)ctx->d_dump[13];
+  CU(cudaMemcpyAsync(d_items, items, (size_t)n * sizeof(MotionItem), cudaMemcpyHostToDevice, ctx->stream));
+  CU(cudaEventRecord(ctx->ev0, ctx->stream));
+  if (g.is_hbd) {
+    if (block_size == 32) tf_motion_batch_kernel<uint16_t, 32><<<n, 32, SearchSmem<uint16_t, 32>::TOTAL, ctx->stream>>>(K, d_items, d_res, n);
+    else tf_motion_batch_kernel<uint16_t, 16><<<n, 32, SearchSmem<uint16_t, 16>::TOTAL, ctx->stream>>>(K, d_items, d_res, n);
+  } else {
+    if (block_size == 32) tf_motion_batch_kernel<uint8_t, 32><<<n, 32, SearchSmem<uint8_t, 32>::TOTAL, ctx->stream>>>(K, d_items, d_res, n);
+    else tf_motion_batch_kernel<uint8_t, 16><<<n, 32, SearchSmem<uint8_t, 16>::TOTAL, ctx->stream>>>(K, d_items, d_res, n);
+  }
+  CU(cudaGetLastError());
+  ctx->last_launches++;
+  CU(cudaEventRecord(ctx->ev1, ctx->stream));
+  CU(cudaMemcpyAsync(results, d_res, (size_t)n * sizeof(MotionResult), cudaMemcpyDeviceToHost, ctx->stream));
+  CU(cudaStreamSynchronize(ctx->stream));
+  float ms = 0.f;
+  CU(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
+  ctx->last_kernel_ms = ms;
   return TF_GPU_OK;
 }
 

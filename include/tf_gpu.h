@@ -272,6 +272,36 @@ typedef struct {
 int tf_gpu_fullpel_search_batch(tf_gpu_ctx *ctx, const tf_gpu_params *params, const tf_gpu_frame *src,
                                 const tf_gpu_frame *ref, int block_size, const tf_gpu_search_item *items, int n,
                                 tf_gpu_search_result *results);
+/* The whole per-block motion search over resident frames, against up to TF_GPU_MAX_FRAMES - 1 references in one
+ * launch.  Every item gets what tf_motion_search() (temporal_filter.c:145-188) does to one block of frame src_id
+ * searched in frame ref_ids[item.ref], with the MV limits of the item's own size and position (the rule of
+ * tf_gpu_fullpel_search_batch): av1_full_pixel_search() from the item's start MV, then find_fractional_mv_step
+ * (mcomp.c:2844-3133: MV_COST_NONE, forced_stop = EIGHTH_PEL, no cost list, limits from
+ * av1_set_subpel_mv_search_range around a zero MV); under force_integer_mv == 1 there is no sub-pel stage:
+ * row, col = 8 x the full-pel MV and err = the variance at it (:162-172).  TPL (tpl_model.c:285) and first pass
+ * (firstpass.c:261-300) run this search per 16x16 / 32x32 block against each of their reference frames.
+ * Of `params` the fields tf_gpu_fullpel_search_batch reads are read, plus force_integer_mv, allow_hp,
+ * subpel_method and subpel_iters_per_step.  src_id and every ref_ids[r] must be resident (tf_gpu_cache_frame*,
+ * tf_gpu_cache_frame_device) with one geometry; a reference may repeat or equal the source.  The stream waits
+ * for each frame's upload or ingest.  TF_GPU_ERR_INVALID, with nothing enqueued and the context unchanged, for
+ * a NULL pointer, block_size other than 16 or 32, n < 0, num_refs outside [1, TF_GPU_MAX_FRAMES - 1], an id
+ * that is not resident, frames of different geometry, an item whose position fails the rule above or whose
+ * ref is outside [0, num_refs).  n == 0 returns TF_GPU_OK.  Synchronous; tf_gpu_last_stats reports one launch
+ * and the search kernel's device time. */
+typedef struct {
+  int x, y;                     /* luma position of the block's top-left sample */
+  int16_t start_row, start_col; /* full-pel start MV */
+  int32_t ref;                  /* index into ref_ids */
+} tf_gpu_motion_item;
+typedef struct {
+  int16_t fullpel_row, fullpel_col; /* av1_full_pixel_search() best MV */
+  int32_t fullpel_var;              /* its return value (variance + MV cost), as tf_gpu_search_result.var */
+  int16_t row, col;                 /* final MV, 1/8 pel */
+  uint32_t err;                     /* sub-pel besterr; under force_integer_mv the variance at the full-pel MV */
+} tf_gpu_motion_result;
+int tf_gpu_motion_search_batch(tf_gpu_ctx *ctx, const tf_gpu_params *params, uint64_t src_id,
+                               const uint64_t *ref_ids, int num_refs, int block_size,
+                               const tf_gpu_motion_item *items, int n, tf_gpu_motion_result *results);
 
 /* Pinned host memory helpers so lookahead buffers can be DMA'd directly. */
 int tf_gpu_host_register(tf_gpu_ctx *ctx, void *ptr, size_t bytes);
