@@ -35,7 +35,7 @@ EXPORTS = [
     "tf_gpu_cache_frame_async", "tf_gpu_debug_read_plane", "tf_gpu_device_border", "tf_gpu_fullpel_search_batch",
     "tf_gpu_output_ipc_export", "tf_gpu_output_ipc_import", "tf_gpu_cache_frame_device",
     "tf_gpu_filter_batch_async", "tf_gpu_filter_batch_result", "tf_gpu_download_batch_output",
-    "tf_gpu_batch_output_device_plane", "tf_gpu_motion_search_batch",
+    "tf_gpu_batch_output_device_plane", "tf_gpu_motion_search_batch", "tf_gpu_motion_search_device",
 ]
 
 
@@ -99,6 +99,7 @@ _MOTION_RESULT_DTYPE = np.dtype([("fullpel_row", "<i2"), ("fullpel_col", "<i2"),
                                  ("row", "<i2"), ("col", "<i2"), ("err", "<u4")])
 assert _MOTION_ITEM_DTYPE.itemsize == C.sizeof(MotionItem) == 16
 assert _MOTION_RESULT_DTYPE.itemsize == C.sizeof(MotionResult) == 16
+TF_GPU_MOTION_REJECTED = -1  # fullpel_var of an item tf_gpu_motion_search_device rejected (tf_gpu.h)
 
 
 class Dump(C.Structure):
@@ -141,6 +142,7 @@ def load_library():
                                                 C.POINTER(SearchItem), i, C.POINTER(SearchResult)]
     lib.tf_gpu_motion_search_batch.argtypes = [vp, C.POINTER(Params), u64, C.POINTER(u64), i, i,
                                                C.POINTER(MotionItem), i, C.POINTER(MotionResult)]
+    lib.tf_gpu_motion_search_device.argtypes = [vp, C.POINTER(Params), u64, C.POINTER(u64), i, i, vp, i, vp, vp]
     lib.tf_gpu_filter_resident.argtypes = [vp, C.POINTER(Params), C.POINTER(u64), C.POINTER(C.c_int64),
                                            C.POINTER(C.c_float)]
     lib.tf_gpu_download_output.argtypes = [vp, C.POINTER(Frame), i, i]
@@ -381,6 +383,55 @@ def motion_search_args(ref_ids, block_size, items):
     return (C.c_uint64 * len(ids))(*ids), len(ids), packed, len(a)
 
 
+def motion_search_device_args(ref_ids, block_size, items, device):
+    """Arguments of tf_gpu_motion_search_device that can be checked without reading the items (which would
+    synchronise): (uint64_t ref_ids[num_refs], num_refs, n).  items: an integer CUDA tensor of shape (n, 5) = x, y,
+    start_row, start_col, ref on `device`, the context's torch.device.  Raises ValueError, before anything reaches
+    the library, for items that are not such a tensor, 0 or more than TF_GPU_MAX_FRAMES - 1 references, and a block
+    size other than 16 or 32.  Positions and refs are checked per item by the kernel (tf_gpu.h)."""
+    import torch
+    if block_size not in (16, 32):
+        raise ValueError(f"block_size must be 16 or 32, got {block_size}")
+    ids = [int(r) for r in ref_ids]
+    if not 1 <= len(ids) <= TF_GPU_MAX_FRAMES - 1:
+        raise ValueError(f"1 to {TF_GPU_MAX_FRAMES - 1} reference frames, got {len(ids)}")
+    if not isinstance(items, torch.Tensor):
+        raise ValueError(f"items must be a torch tensor, got {type(items).__name__}")
+    if items.dim() != 2 or items.shape[1] != 5:
+        raise ValueError(f"items must have shape (n, 5) (x, y, start_row, start_col, ref), got {tuple(items.shape)}")
+    if items.dtype.is_floating_point or items.dtype.is_complex or items.dtype == torch.bool:
+        raise ValueError(f"items must be integers, got dtype {items.dtype}")
+    if not items.is_cuda:
+        raise ValueError(f"items must be a CUDA tensor, got one on {items.device}")
+    if items.device != torch.device(device):
+        raise ValueError(f"items are on {items.device}, the context on {torch.device(device)}")
+    return (C.c_uint64 * len(ids))(*ids), len(ids), items.shape[0]
+
+
+def pack_motion_items(items):
+    """(n, 5) integer tensor (x, y, start_row, start_col, ref) -> (n, 4) int32 tensor whose rows are
+    tf_gpu_motion_item, by torch ops on the tensor's device (and current stream).  Values are converted as the C
+    struct holds them: x, y and ref to int32, the starts to int16 (each modulo its type's range)."""
+    import torch
+    out = torch.empty((items.shape[0], 4), dtype=torch.int32, device=items.device)
+    out[:, 0] = items[:, 0]
+    out[:, 1] = items[:, 1]
+    out[:, 3] = items[:, 4]
+    half = out.view(torch.int16)  # (n, 8): start_row, start_col are halves 4 and 5 (bytes 8..11)
+    half[:, 4] = items[:, 2]
+    half[:, 5] = items[:, 3]
+    return out
+
+
+def unpack_motion_results(res):
+    """(n, 4) int32 tensor of tf_gpu_motion_result rows -> int64 tensor (n, 6) = fullpel_row, fullpel_col,
+    fullpel_var, row, col, err (err unsigned), by torch ops on the tensor's device (and current stream)."""
+    import torch
+    half = res.view(torch.int16)
+    cols = (half[:, 0], half[:, 1], res[:, 1], half[:, 4], half[:, 5], res[:, 3].to(torch.int64) & 0xFFFFFFFF)
+    return torch.stack([c.to(torch.int64) for c in cols], dim=1)
+
+
 class TemporalFilterGpu:
     """One tf_gpu_ctx (CUDA device + stream + frame cache)."""
 
@@ -598,6 +649,29 @@ class TemporalFilterGpu:
             self.h, C.byref(cp), int(src_id), ids, num_refs, block_size,
             C.cast(packed.ctypes.data, C.POINTER(MotionItem)), n, C.cast(res.ctypes.data, C.POINTER(MotionResult))))
         return np.stack([res[k][:n].astype(np.int64) for k in _MOTION_RESULT_DTYPE.names], axis=1).reshape(n, 6)
+
+    def motion_search_tensors(self, params, src_id, ref_ids, block_size, items):
+        """motion_search_batch() with items and results on the GPU (tf_gpu_motion_search_device): items is an integer
+        CUDA tensor (n, 5) on the context's device (see motion_search_device_args); returns a new int64 CUDA tensor
+        (n, 6) with the columns of motion_search_batch.  Packing, search and unpacking run in order on the current
+        torch stream of that device, after what is already enqueued there, and the call does not synchronise: read
+        the result on that stream (or after synchronising it).  The starts are taken as int16, as the C struct holds
+        them, without a range check (which would need a synchronise); the full-pel search clamps its start into the
+        block's MV limits, so any start is safe.  An item whose position or ref the kernel rejects gets
+        fullpel_var = TF_GPU_MOTION_REJECTED, MVs 0 and err = 2**32 - 1.  The input buffers need no record_stream:
+        the library makes the stream wait for the search before the call returns."""
+        import torch
+        cp = make_params(params) if isinstance(params, dict) else params
+        dev = self._torch_device(torch)
+        ids, num_refs, n = motion_search_device_args(ref_ids, block_size, items, dev)
+        with torch.cuda.device(dev):
+            packed = pack_motion_items(items) if n else torch.zeros((1, 4), dtype=torch.int32, device=dev)
+            res = torch.empty((max(n, 1), 4), dtype=torch.int32, device=dev)
+            s = torch.cuda.current_stream(dev)
+            self._check(self.lib.tf_gpu_motion_search_device(self.h, C.byref(cp), int(src_id), ids, num_refs,
+                                                             block_size, packed.data_ptr(), n, res.data_ptr(),
+                                                             s.cuda_stream))
+            return unpack_motion_results(res[:n])
 
     def device_border(self):
         return self.lib.tf_gpu_device_border()

@@ -94,6 +94,8 @@ struct tf_gpu_ctx {
   cudaEvent_t ev_async_upload = nullptr;      // last tf_gpu_cache_frame_async upload
   bool async_upload_pending = false;
   cudaEvent_t ev_ingest_src = nullptr;        // producer's stream at a tf_gpu_cache_frame_device call
+  cudaEvent_t ev_search_src = nullptr;        // caller's stream at a tf_gpu_motion_search_device call
+  cudaEvent_t ev_search_done = nullptr;       // that call's search on the main stream
   cudaEvent_t user_ev[4] = { nullptr, nullptr, nullptr, nullptr };
   std::vector<DevFrame> cache;
   DevFrame out;
@@ -228,6 +230,43 @@ AddressRangeFn address_range_fn() {
       fn = (AddressRangeFn)p;
   }
   return fn;
+}
+// `ptr` is device (or managed) memory of the context's device, `align`-byte aligned, and the `bytes` from it lie
+// inside the allocation it belongs to.  Allocators that map memory in chunks (the virtual-memory API behind torch's
+// expandable segments, stream-ordered pools) may report one chunk per call: the extent may go on into chunks mapped
+// right after it, each device memory of this device, so the walk follows the ranges as long as they are contiguous.
+// `what` names the pointer in the error message.
+int check_device_extent(tf_gpu_ctx *ctx, const void *ptr, size_t bytes, size_t align, const char *what) {
+  const AddressRangeFn range = address_range_fn();
+  if (!range) return fail(ctx, TF_GPU_ERR_CUDA, "cuMemGetAddressRange is not available in this driver");
+  if ((uintptr_t)ptr % align) return fail(ctx, TF_GPU_ERR_INVALID, "%s is not %zu-byte aligned", what, align);
+  cudaPointerAttributes at;
+  if (cudaPointerGetAttributes(&at, ptr) != cudaSuccess) {
+    cudaGetLastError();
+    return fail(ctx, TF_GPU_ERR_INVALID, "%s is not a CUDA pointer", what);
+  }
+  if ((at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged) || at.device != ctx->device)
+    return fail(ctx, TF_GPU_ERR_INVALID, "%s is not device memory of device %d", what, ctx->device);
+  CUdeviceptr base = 0;
+  size_t size = 0;
+  const CUdeviceptr dp = (CUdeviceptr)(uintptr_t)ptr;
+  if (range(&base, &size, dp) != CUDA_SUCCESS || dp < base || dp - base > size)
+    return fail(ctx, TF_GPU_ERR_INVALID, "%s: no device allocation at this address", what);
+  CUdeviceptr end = base + size;
+  while (end - dp < bytes) {
+    CUdeviceptr nb = 0;
+    size_t ns = 0;
+    cudaPointerAttributes na;
+    if (range(&nb, &ns, end) != CUDA_SUCCESS || nb != end || ns == 0 ||
+        cudaPointerGetAttributes(&na, (const void *)(uintptr_t)end) != cudaSuccess ||
+        (na.type != cudaMemoryTypeDevice && na.type != cudaMemoryTypeManaged) || na.device != ctx->device) {
+      cudaGetLastError();
+      return fail(ctx, TF_GPU_ERR_INVALID, "%s: its extent (%zu bytes) runs past its allocation (%zu bytes)", what, bytes,
+                  (size_t)(end - dp));
+    }
+    end = nb + ns;
+  }
+  return TF_GPU_OK;
 }
 int make_tensor_maps(tf_gpu_ctx *ctx, DevFrame *d) {
   EncodeTiledFn enc = encode_tiled_fn();
@@ -1074,6 +1113,8 @@ int tf_gpu_create(tf_gpu_ctx **out, const tf_gpu_device_cfg *cfg) {
   if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&ctx->noise_stream, cudaStreamNonBlocking);
   if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ctx->ev_async_upload, cudaEventDisableTiming);
   if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ctx->ev_ingest_src, cudaEventDisableTiming);
+  if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ctx->ev_search_src, cudaEventDisableTiming);
+  if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ctx->ev_search_done, cudaEventDisableTiming);
   for (int i = 0; i < 4 && e == cudaSuccess; i++) e = cudaEventCreate(&ctx->user_ev[i]);
   for (int i = 0; i < 8 && e == cudaSuccess; i++) e = cudaEventCreateWithFlags(&ctx->tickets[i].ev, cudaEventDisableTiming);
   if (e == cudaSuccess) e = cudaMalloc(&ctx->d_diff, 18 * sizeof(unsigned long long));
@@ -1153,6 +1194,8 @@ void tf_gpu_destroy(tf_gpu_ctx *ctx) {
   }
   if (ctx->ev_async_upload) cudaEventDestroy(ctx->ev_async_upload);
   if (ctx->ev_ingest_src) cudaEventDestroy(ctx->ev_ingest_src);
+  if (ctx->ev_search_src) cudaEventDestroy(ctx->ev_search_src);
+  if (ctx->ev_search_done) cudaEventDestroy(ctx->ev_search_done);
   if (ctx->ev0) cudaEventDestroy(ctx->ev0);
   if (ctx->ev1) cudaEventDestroy(ctx->ev1);
   for (int i = 0; i < TF_GPU_MAX_FRAMES; i++)
@@ -1207,52 +1250,22 @@ int tf_gpu_cache_frame_device(tf_gpu_ctx *ctx, const tf_gpu_frame *frame, void *
   Geometry g;
   if (!make_geometry(frame, num_planes, &g)) return fail(ctx, TF_GPU_ERR_INVALID, "bad frame geometry");
   CU(cudaSetDevice(ctx->device));
-  const AddressRangeFn range = address_range_fn();
-  if (!range) return fail(ctx, TF_GPU_ERR_CUDA, "cuMemGetAddressRange is not available in this driver");
   // Everything the ingest kernels will read is checked here, before anything is enqueued: a plane is device (or
   // managed) memory of this context's device, and its crop area, rows `stride` samples apart, lies inside the
   // allocation the pointer belongs to (or in allocations mapped contiguously after it).
   const size_t es = g.is_hbd ? 2 : 1;
   for (int p = 0; p < num_planes; p++) {
     const int k = p > 0;
-    const void *ptr = frame->plane[p];
-    if (!ptr) return fail(ctx, TF_GPU_ERR_INVALID, "frame plane %d is NULL", p);
+    if (!frame->plane[p]) return fail(ctx, TF_GPU_ERR_INVALID, "frame plane %d is NULL", p);
     if (g.crop_w[k] <= 0 || g.crop_h[k] <= 0 || g.aligned_w[k] < g.crop_w[k] || g.aligned_h[k] < g.crop_h[k])
       return fail(ctx, TF_GPU_ERR_INVALID, "plane %d: bad crop / aligned size", p);
     if (frame->stride[k] < g.crop_w[k])
       return fail(ctx, TF_GPU_ERR_INVALID, "plane %d: stride %d is smaller than the crop width %d", p, frame->stride[k], g.crop_w[k]);
-    if ((uintptr_t)ptr % es) return fail(ctx, TF_GPU_ERR_INVALID, "plane %d is not aligned to its %zu-byte samples", p, es);
-    cudaPointerAttributes at;
-    if (cudaPointerGetAttributes(&at, ptr) != cudaSuccess) {
-      cudaGetLastError();
-      return fail(ctx, TF_GPU_ERR_INVALID, "plane %d is not a CUDA pointer", p);
-    }
-    if ((at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged) || at.device != ctx->device)
-      return fail(ctx, TF_GPU_ERR_INVALID, "plane %d is not device memory of device %d", p, ctx->device);
-    CUdeviceptr base = 0;
-    size_t size = 0;
-    const CUdeviceptr dp = (CUdeviceptr)(uintptr_t)ptr;
-    if (range(&base, &size, dp) != CUDA_SUCCESS || dp < base || dp - base > size)
-      return fail(ctx, TF_GPU_ERR_INVALID, "plane %d: no device allocation at this address", p);
-    const size_t need = ((size_t)(g.crop_h[k] - 1) * frame->stride[k] + g.crop_w[k]) * es;
-    // Allocators that map memory in chunks (the virtual-memory API behind torch's expandable segments, stream-ordered
-    // pools) may report one chunk per call: the extent may go on into chunks mapped right after it, each device
-    // memory of this device, so the walk follows the ranges as long as they are contiguous.
-    CUdeviceptr end = base + size;
-    while (end - dp < need) {
-      CUdeviceptr nb = 0;
-      size_t ns = 0;
-      cudaPointerAttributes na;
-      if (range(&nb, &ns, end) != CUDA_SUCCESS || nb != end || ns == 0 ||
-          cudaPointerGetAttributes(&na, (const void *)(uintptr_t)end) != cudaSuccess ||
-          (na.type != cudaMemoryTypeDevice && na.type != cudaMemoryTypeManaged) || na.device != ctx->device) {
-        cudaGetLastError();
-        return fail(ctx, TF_GPU_ERR_INVALID,
-                    "plane %d: its crop area (%zu bytes from pixel (0,0)) runs past its allocation (%zu bytes)", p,
-                    need, (size_t)(end - dp));
-      }
-      end = nb + ns;
-    }
+    char what[16];
+    snprintf(what, sizeof(what), "plane %d", p);
+    const int rc = check_device_extent(ctx, frame->plane[p], ((size_t)(g.crop_h[k] - 1) * frame->stride[k] + g.crop_w[k]) * es,
+                                       es, what);
+    if (rc) return rc;
   }
   CallScope scope(ctx);
   FrameSource src;
@@ -1600,11 +1613,70 @@ tf_gpu_params search_params(const tf_gpu_params &in, int num_frames) {
   return p;
 }
 
-// A batched search item's block starts inside the mi grid (it may stick out of it like the last 32x32 row of a
-// 1080p frame); the SAD engine reads source rows with 16-byte loads.
+// A batched search item's position against the rule tf_motion_batch_kernel applies to items in device memory.
 int check_item_position(tf_gpu_ctx *ctx, const tf_gpu_params &p, int i, int x, int y) {
-  if (x < 0 || y < 0 || (x & 15) || (y & 3) || x >= p.mi_cols * 4 || y >= p.mi_rows * 4)
+  if (!item_position_ok(x, y, p.mi_rows, p.mi_cols))
     return fail(ctx, TF_GPU_ERR_INVALID, "item %d: block position (%d, %d) not supported", i, x, y);
+  return TF_GPU_OK;
+}
+
+// The checks both motion-search entry points make before anything is enqueued or pinned, short of the items (the
+// synchronous call reads them on the host, the device call leaves them to the kernel) and of where items / results
+// live.  n == 0 passes without the frame checks: the caller returns TF_GPU_OK.  Otherwise *p holds the search
+// params, devf[0] the source slot and devf[1 .. num_refs] the reference slots.
+int check_motion_search(tf_gpu_ctx *ctx, const tf_gpu_params *params, uint64_t src_id, const uint64_t *ref_ids,
+                        int num_refs, int block_size, const void *items, int n, const void *results, tf_gpu_params *p,
+                        DevFrame **devf) {
+  if (!params || !ref_ids || !items || !results) return fail(ctx, TF_GPU_ERR_INVALID, "NULL argument");
+  if (block_size != 16 && block_size != 32) return fail(ctx, TF_GPU_ERR_INVALID, "block_size must be 16 or 32");
+  if (n < 0) return fail(ctx, TF_GPU_ERR_INVALID, "negative item count");
+  if (num_refs < 1 || num_refs > TF_GPU_MAX_FRAMES - 1)
+    return fail(ctx, TF_GPU_ERR_INVALID, "num_refs %d out of [1,%d]", num_refs, TF_GPU_MAX_FRAMES - 1);
+  if (n == 0) return TF_GPU_OK;
+  *p = search_params(*params, 1 + num_refs);
+  int rc = validate_params(ctx, p);
+  if (rc) return rc;
+  for (int f = 0; f <= num_refs; f++) {
+    const uint64_t id = f ? ref_ids[f - 1] : src_id;
+    devf[f] = find_cached(ctx, id, nullptr);
+    if (!devf[f]) return fail(ctx, TF_GPU_ERR_INVALID, "frame id %llu is not resident", (unsigned long long)id);
+    if (!(devf[f]->g == devf[0]->g)) return fail(ctx, TF_GPU_ERR_INVALID, "the source and references must share one geometry");
+  }
+  return validate_geometry(ctx, p, devf[0]->g);
+}
+
+// The search itself, on the main stream, for both entry points: pins the slots for the current epoch (so that
+// done_ev covers the kernel for a later eviction), waits for each slot's upload or ingest, and makes one launch over
+// items / results in device memory; `timed`: ctx->ev0 / ev1 around the launch.
+int enqueue_motion_search(tf_gpu_ctx *ctx, const tf_gpu_params &p, DevFrame *const *devf, int num_refs, int block_size,
+                          const MotionItem *d_items, MotionResult *d_res, int n, bool timed) {
+  for (int f = 0; f <= num_refs; f++) {
+    DevFrame *d = devf[f];
+    if (d->pinned_epoch != ctx->epoch) CU(cudaStreamWaitEvent(ctx->stream, d->ready, 0));
+    d->last_use = ++ctx->use_counter;
+    d->pinned_epoch = ctx->epoch;
+  }
+  const Geometry &g = devf[0]->g;
+  KParams K;
+  fill_kparams(ctx, &p, g, K);
+  // frames past the references are the source's: an item's ref is checked in the kernel, and even a wrong check
+  // could then not reach a null or stale frame pointer
+  for (int f = 0; f < MAXF; f++) {
+    const DevFrame *d = devf[f <= num_refs ? f : 0];
+    K.frm[f][0] = d->p00[0];
+    K.tmap[f] = d->d_tmap;  // TF_FAR_TMA builds: each reference's own descriptors
+  }
+  if (timed) CU(cudaEventRecord(ctx->ev0, ctx->stream));
+  if (g.is_hbd) {
+    if (block_size == 32) tf_motion_batch_kernel<uint16_t, 32><<<n, 32, SearchSmem<uint16_t, 32>::TOTAL, ctx->stream>>>(K, d_items, d_res, n);
+    else tf_motion_batch_kernel<uint16_t, 16><<<n, 32, SearchSmem<uint16_t, 16>::TOTAL, ctx->stream>>>(K, d_items, d_res, n);
+  } else {
+    if (block_size == 32) tf_motion_batch_kernel<uint8_t, 32><<<n, 32, SearchSmem<uint8_t, 32>::TOTAL, ctx->stream>>>(K, d_items, d_res, n);
+    else tf_motion_batch_kernel<uint8_t, 16><<<n, 32, SearchSmem<uint8_t, 16>::TOTAL, ctx->stream>>>(K, d_items, d_res, n);
+  }
+  CU(cudaGetLastError());
+  ctx->last_launches++;
+  if (timed) CU(cudaEventRecord(ctx->ev1, ctx->stream));
   return TF_GPU_OK;
 }
 
@@ -1675,25 +1747,10 @@ int tf_gpu_motion_search_batch(tf_gpu_ctx *ctx, const tf_gpu_params *params, uin
                 "ABI structs and device structs must agree");
   if (!ctx) return TF_GPU_ERR_INVALID;
   // every check comes before anything is enqueued or pinned: a rejected call leaves the context as it was
-  if (!params || !ref_ids || !items || !results) return fail(ctx, TF_GPU_ERR_INVALID, "NULL argument");
-  if (block_size != 16 && block_size != 32) return fail(ctx, TF_GPU_ERR_INVALID, "block_size must be 16 or 32");
-  if (n < 0) return fail(ctx, TF_GPU_ERR_INVALID, "negative item count");
-  if (num_refs < 1 || num_refs > TF_GPU_MAX_FRAMES - 1)
-    return fail(ctx, TF_GPU_ERR_INVALID, "num_refs %d out of [1,%d]", num_refs, TF_GPU_MAX_FRAMES - 1);
-  if (n == 0) return TF_GPU_OK;
-  const tf_gpu_params p = search_params(*params, 1 + num_refs);
-  int rc = validate_params(ctx, &p);
-  if (rc) return rc;
+  tf_gpu_params p;
   DevFrame *devf[TF_GPU_MAX_FRAMES];
-  for (int f = 0; f <= num_refs; f++) {
-    const uint64_t id = f ? ref_ids[f - 1] : src_id;
-    devf[f] = find_cached(ctx, id, nullptr);
-    if (!devf[f]) return fail(ctx, TF_GPU_ERR_INVALID, "frame id %llu is not resident", (unsigned long long)id);
-    if (!(devf[f]->g == devf[0]->g)) return fail(ctx, TF_GPU_ERR_INVALID, "the source and references must share one geometry");
-  }
-  const Geometry &g = devf[0]->g;
-  rc = validate_geometry(ctx, &p, g);
-  if (rc) return rc;
+  int rc = check_motion_search(ctx, params, src_id, ref_ids, num_refs, block_size, items, n, results, &p, devf);
+  if (rc || n == 0) return rc;
   for (int i = 0; i < n; i++) {
     rc = check_item_position(ctx, p, i, items[i].x, items[i].y);
     if (rc) return rc;
@@ -1703,18 +1760,6 @@ int tf_gpu_motion_search_batch(tf_gpu_ctx *ctx, const tf_gpu_params *params, uin
   CU(cudaSetDevice(ctx->device));
   CallScope scope(ctx);
   ctx->last_launches = 0;
-  for (int f = 0; f <= num_refs; f++) {
-    DevFrame *d = devf[f];
-    if (d->pinned_epoch != ctx->epoch) CU(cudaStreamWaitEvent(ctx->stream, d->ready, 0));
-    d->last_use = ++ctx->use_counter;
-    d->pinned_epoch = ctx->epoch;
-  }
-  KParams K;
-  fill_kparams(ctx, &p, g, K);
-  for (int f = 0; f <= num_refs; f++) {
-    K.frm[f][0] = devf[f]->p00[0];
-    K.tmap[f] = devf[f]->d_tmap;  // TF_FAR_TMA builds: each reference's own descriptors
-  }
   rc = ensure_dump(ctx, 12, (size_t)n * sizeof(MotionItem));
   if (rc) return rc;
   rc = ensure_dump(ctx, 13, (size_t)n * sizeof(MotionResult));
@@ -1722,22 +1767,46 @@ int tf_gpu_motion_search_batch(tf_gpu_ctx *ctx, const tf_gpu_params *params, uin
   MotionItem *d_items = (MotionItem *)ctx->d_dump[12];
   MotionResult *d_res = (MotionResult *)ctx->d_dump[13];
   CU(cudaMemcpyAsync(d_items, items, (size_t)n * sizeof(MotionItem), cudaMemcpyHostToDevice, ctx->stream));
-  CU(cudaEventRecord(ctx->ev0, ctx->stream));
-  if (g.is_hbd) {
-    if (block_size == 32) tf_motion_batch_kernel<uint16_t, 32><<<n, 32, SearchSmem<uint16_t, 32>::TOTAL, ctx->stream>>>(K, d_items, d_res, n);
-    else tf_motion_batch_kernel<uint16_t, 16><<<n, 32, SearchSmem<uint16_t, 16>::TOTAL, ctx->stream>>>(K, d_items, d_res, n);
-  } else {
-    if (block_size == 32) tf_motion_batch_kernel<uint8_t, 32><<<n, 32, SearchSmem<uint8_t, 32>::TOTAL, ctx->stream>>>(K, d_items, d_res, n);
-    else tf_motion_batch_kernel<uint8_t, 16><<<n, 32, SearchSmem<uint8_t, 16>::TOTAL, ctx->stream>>>(K, d_items, d_res, n);
-  }
-  CU(cudaGetLastError());
-  ctx->last_launches++;
-  CU(cudaEventRecord(ctx->ev1, ctx->stream));
+  rc = enqueue_motion_search(ctx, p, devf, num_refs, block_size, d_items, d_res, n, true);
+  if (rc) return rc;
   CU(cudaMemcpyAsync(results, d_res, (size_t)n * sizeof(MotionResult), cudaMemcpyDeviceToHost, ctx->stream));
   CU(cudaStreamSynchronize(ctx->stream));
   float ms = 0.f;
   CU(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
   ctx->last_kernel_ms = ms;
+  return TF_GPU_OK;
+}
+
+int tf_gpu_motion_search_device(tf_gpu_ctx *ctx, const tf_gpu_params *params, uint64_t src_id, const uint64_t *ref_ids,
+                                int num_refs, int block_size, const tf_gpu_motion_item *items, int n,
+                                tf_gpu_motion_result *results, void *stream) {
+  static_assert(TF_GPU_MOTION_REJECTED == MOTION_REJECTED, "header and kernel must agree on the rejection sentinel");
+  if (!ctx) return TF_GPU_ERR_INVALID;
+  // every check comes before anything is enqueued or pinned: a rejected call leaves the context as it was
+  tf_gpu_params p;
+  DevFrame *devf[TF_GPU_MAX_FRAMES];
+  int rc = check_motion_search(ctx, params, src_id, ref_ids, num_refs, block_size, items, n, results, &p, devf);
+  if (rc || n == 0) return rc;
+  CU(cudaSetDevice(ctx->device));
+  const size_t bytes = (size_t)n * sizeof(MotionItem);
+  rc = check_device_extent(ctx, items, bytes, 4, "items");
+  if (rc) return rc;
+  rc = check_device_extent(ctx, results, bytes, 4, "results");
+  if (rc) return rc;
+  const uintptr_t a = (uintptr_t)items, b = (uintptr_t)results;
+  if (a < b + bytes && b < a + bytes) return fail(ctx, TF_GPU_ERR_INVALID, "items and results overlap");
+  CallScope scope(ctx);
+  ctx->last_launches = 0;
+  ctx->last_kernel_ms = 0.f;  // not timed: the call does not wait for the kernel
+  // on the main stream between the caller's stream and back, so that done_ev covers the search (see get_frame)
+  const cudaStream_t s = (cudaStream_t)stream;
+  CU(cudaEventRecord(ctx->ev_search_src, s));
+  CU(cudaStreamWaitEvent(ctx->stream, ctx->ev_search_src, 0));
+  rc = enqueue_motion_search(ctx, p, devf, num_refs, block_size, (const MotionItem *)items, (MotionResult *)results, n,
+                             false);
+  if (rc) return rc;
+  CU(cudaEventRecord(ctx->ev_search_done, ctx->stream));
+  CU(cudaStreamWaitEvent(s, ctx->ev_search_done, 0));
   return TF_GPU_OK;
 }
 

@@ -1719,6 +1719,13 @@ __global__ void __launch_bounds__(32, S16_WARPS) tf_search16_kernel(const __grid
   search16_task<T>(P, blockIdx.x);
 }
 
+// Position rule of a batched search item (tf_gpu.h): the block starts inside the mi grid (it may stick out of it
+// like the last 32x32 row of a 1080p frame); x is a multiple of 16 because the SAD engine reads source rows with
+// 16-byte loads.  The host checks it for the synchronous calls, tf_motion_batch_kernel for device-memory items.
+__host__ __device__ __forceinline__ bool item_position_ok(int x, int y, int mi_rows, int mi_cols) {
+  return x >= 0 && y >= 0 && !(x & 15) && !(y & 3) && x < mi_cols * 4 && y < mi_rows * 4;
+}
+
 // Batched full-pixel search (tf_gpu_fullpel_search_batch): one warp per item, the engine of the two
 // kernels above on an arbitrary block of an arbitrary frame pair.
 struct SearchItem {
@@ -1780,6 +1787,9 @@ __global__ void __launch_bounds__(32, W == 32 ? S32_WARPS_LO : 24)
 // routines read it from there, as in search16_task) and find_fractional_mv_step refines the MV to 1/8 pel in the
 // shared memory of the search (MV_COST_NONE, forced_stop = EIGHTH_PEL, no cost list); under force_integer_mv the
 // result is the variance at the full-pel MV instead (:162-172).
+// Every item is checked before any frame is read (items in device memory are never seen by the host): an item whose
+// position fails item_position_ok or whose ref is outside [0, P.num_frames - 1) gets fullpel_var =
+// MOTION_REJECTED, MVs 0 and err = UINT32_MAX.
 struct MotionItem {
   int x, y;
   int16_t start_row, start_col;
@@ -1791,6 +1801,7 @@ struct MotionResult {
   int16_t row, col;
   uint32_t err;
 };
+constexpr int MOTION_REJECTED = -1;  // TF_GPU_MOTION_REJECTED; a searched item's fullpel_var is never negative
 template <typename T, int W>
 __global__ void __launch_bounds__(32, W == 32 ? S32_WARPS_LO : 24)
     tf_motion_batch_kernel(const __grid_constant__ KParams P, const MotionItem *items, MotionResult *results, int n) {
@@ -1798,6 +1809,16 @@ __global__ void __launch_bounds__(32, W == 32 ? S32_WARPS_LO : 24)
   const int lane = lane_id();
   if ((int)blockIdx.x >= n) return;
   const MotionItem it = items[blockIdx.x];
+  if (!item_position_ok(it.x, it.y, P.mi_rows, P.mi_cols) || it.ref < 0 || it.ref >= P.num_frames - 1) {
+    if (lane == 0) {
+      MotionResult r;
+      r.fullpel_row = r.fullpel_col = r.row = r.col = 0;
+      r.fullpel_var = MOTION_REJECTED;
+      r.err = 0xffffffffu;
+      results[blockIdx.x] = r;
+    }
+    return;
+  }
   const int f = 1 + it.ref;
   Search<T> S;
   const MV2 start = { (int)it.start_row, (int)it.start_col };

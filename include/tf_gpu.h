@@ -286,8 +286,9 @@ int tf_gpu_fullpel_search_batch(tf_gpu_ctx *ctx, const tf_gpu_params *params, co
  * for each frame's upload or ingest.  TF_GPU_ERR_INVALID, with nothing enqueued and the context unchanged, for
  * a NULL pointer, block_size other than 16 or 32, n < 0, num_refs outside [1, TF_GPU_MAX_FRAMES - 1], an id
  * that is not resident, frames of different geometry, an item whose position fails the rule above or whose
- * ref is outside [0, num_refs).  n == 0 returns TF_GPU_OK.  Synchronous; tf_gpu_last_stats reports one launch
- * and the search kernel's device time. */
+ * ref is outside [0, num_refs) (the whole call is rejected; tf_gpu_motion_search_device below rejects such an
+ * item alone).  n == 0 returns TF_GPU_OK.  Synchronous; tf_gpu_last_stats reports one launch and the search
+ * kernel's device time. */
 typedef struct {
   int x, y;                     /* luma position of the block's top-left sample */
   int16_t start_row, start_col; /* full-pel start MV */
@@ -302,6 +303,28 @@ typedef struct {
 int tf_gpu_motion_search_batch(tf_gpu_ctx *ctx, const tf_gpu_params *params, uint64_t src_id,
                                const uint64_t *ref_ids, int num_refs, int block_size,
                                const tf_gpu_motion_item *items, int n, tf_gpu_motion_result *results);
+/* The same search with items and results in DEVICE (or managed) memory of the context's device, ordered on the
+ * caller's `stream` (a cudaStream_t; NULL = the legacy default stream): for a caller whose blocks and start MVs are
+ * already on the GPU (a torch pipeline; a two-stage search whose 32x32 MVs start the 16x16 blocks), with no round
+ * trip through the host between stages.  Params, ids, block size, the fields read and the results are those of
+ * tf_gpu_motion_search_batch, bit for bit.  The search starts after the work already enqueued on `stream`, and
+ * before returning the call makes `stream` wait for it, so the caller may produce the items and consume or free
+ * both buffers in its own stream order.  The search runs on the context's stream, so it also queues behind a filter
+ * call already submitted on this context.  Never blocks the host (no synchronise, no host copy, no allocation).
+ * TF_GPU_ERR_INVALID, with nothing enqueued and the context unchanged, for what tf_gpu_motion_search_batch rejects
+ * before reading its items (NULL pointers, block_size, n < 0, num_refs, residency, geometry), for items or results
+ * that are not device or managed memory of the context's device, not 4-byte aligned, or whose n * 16 bytes run past
+ * their allocation (checked as tf_gpu_cache_frame_device checks a plane), and for items and results that overlap.
+ * n == 0 returns TF_GPU_OK with nothing enqueued.  The host cannot read the items, so the kernel checks each one
+ * against the position rule and 0 <= ref < num_refs; where tf_gpu_motion_search_batch rejects the whole call, here
+ * only the item is rejected: its result is fullpel_var = TF_GPU_MOTION_REJECTED, MVs 0 and err = UINT32_MAX, and the
+ * other items are searched as usual.  tf_gpu_last_stats reports one launch and a kernel time of 0: the call does not
+ * wait for the kernel, so it does not time it. */
+#define TF_GPU_MOTION_REJECTED (-1) /* fullpel_var of a rejected item; a searched item's is never negative */
+int tf_gpu_motion_search_device(tf_gpu_ctx *ctx, const tf_gpu_params *params, uint64_t src_id,
+                                const uint64_t *ref_ids /* host */, int num_refs, int block_size,
+                                const tf_gpu_motion_item *items /* device */, int n,
+                                tf_gpu_motion_result *results /* device */, void *stream);
 
 /* Pinned host memory helpers so lookahead buffers can be DMA'd directly. */
 int tf_gpu_host_register(tf_gpu_ctx *ctx, void *ptr, size_t bytes);
