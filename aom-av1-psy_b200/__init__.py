@@ -304,8 +304,24 @@ def tensor_frame(frame_id, y, u=None, v=None):
     return f, y.device
 
 
+def _coded_value(p, key, lo):
+    """Optional integer key of make_params' dict, >= lo; absent or None: None."""
+    v = p.get(key)
+    if v is None:
+        return None
+    if isinstance(v, bool) or not isinstance(v, (int, np.integer)):
+        raise ValueError(f"{key} must be an integer, got {v!r}")
+    if not lo <= int(v) <= np.iinfo(np.int32).max:
+        raise ValueError(f"{key} must be in [{lo}, 2**31), got {v}")
+    return int(v)
+
+
 def make_params(p):
-    """dict (tests/_params.tf_params) -> tf_gpu_params."""
+    """dict (tests/_params.tf_params) -> tf_gpu_params.  Optional keys carry the encoder's coded geometry where it
+    differs from the frames' crop size (superres, resize): mi_rows / mi_cols (cm->mi_params; default the frame's own
+    grid, align8(size) / 4) and cm_width / cm_height (cm->width / height; default 0, the crop size).  Raises
+    ValueError for a value of these keys that is not an integer, a grid below 1 or a coded size below 0; the library
+    checks the grid against the frames."""
     c = Params()
     c.num_frames, c.filter_frame_idx = p["num_frames"], p["filter_frame_idx"]
     c.num_planes = 1 if p["monochrome"] else 3
@@ -313,7 +329,10 @@ def make_params(p):
     for i in range(3):
         c.noise_levels[i] = float(p["noise_levels"][i])
     c.q_factor, c.filter_strength = p["q_factor"], p["filter_strength"]
-    c.mi_rows, c.mi_cols = _align(p["height"], 8) // 4, _align(p["width"], 8) // 4
+    mi_rows, mi_cols = _coded_value(p, "mi_rows", 1), _coded_value(p, "mi_cols", 1)
+    cm_w, cm_h = _coded_value(p, "cm_width", 0), _coded_value(p, "cm_height", 0)
+    c.mi_rows = _align(p["height"], 8) // 4 if mi_rows is None else mi_rows
+    c.mi_cols = _align(p["width"], 8) // 4 if mi_cols is None else mi_cols
     c.border_in_pixels = p["border"]
     c.force_integer_mv, c.allow_hp = p["force_integer_mv"], p["allow_hp"]
     c.subpel_method, c.subpel_iters_per_step = p["subpel_method"], p["subpel_iters_per_step"]
@@ -323,7 +342,7 @@ def make_params(p):
     c.use_downsampled_sad, c.compute_frame_diff = p["use_downsampled_sad"], p["compute_frame_diff"]
     c.out_row_begin, c.out_row_end = p.get("out_row_begin", 0), p.get("out_row_end", 0)
     c.extend_output_borders = p.get("extend_output_borders", 0)
-    c.cm_width, c.cm_height = p.get("cm_width", 0), p.get("cm_height", 0)
+    c.cm_width, c.cm_height = cm_w or 0, cm_h or 0
     return c
 
 

@@ -459,9 +459,10 @@ int validate_params(tf_gpu_ctx *ctx, const tf_gpu_params *p) {
 // exceeds the frames would make the search read outside the allocation.
 int validate_geometry(tf_gpu_ctx *ctx, const tf_gpu_params *p, const Geometry &g) {
   if (p->mi_rows <= 0 || p->mi_cols <= 0) return fail(ctx, TF_GPU_ERR_INVALID, "mi_rows / mi_cols must be positive");
-  if (p->mi_rows * 4 > g.aligned_h[0] || p->mi_cols * 4 > g.aligned_w[0])
-    return fail(ctx, TF_GPU_ERR_INVALID, "mi grid %dx%d exceeds the frame's aligned size %dx%d", p->mi_cols * 4, p->mi_rows * 4,
-                g.aligned_w[0], g.aligned_h[0]);
+  // compared in mi units: the aligned sizes are multiples of 8, and mi_rows * 4 could overflow
+  if (p->mi_rows > g.aligned_h[0] / 4 || p->mi_cols > g.aligned_w[0] / 4)
+    return fail(ctx, TF_GPU_ERR_INVALID, "mi grid %dx%d (mi units) exceeds the frame's aligned size %dx%d", p->mi_cols,
+                p->mi_rows, g.aligned_w[0], g.aligned_h[0]);
   if (g.is_hbd == 0 && p->bit_depth != 8) return fail(ctx, TF_GPU_ERR_INVALID, "8-bit container needs bit_depth 8");
   if (g.num_planes < p->num_planes) return fail(ctx, TF_GPU_ERR_INVALID, "frames lack chroma planes");
   return TF_GPU_OK;

@@ -322,6 +322,17 @@ TFREF_API void *tfref_create(const tfref_cfg *cfg) {
   return t;
 }
 
+/* cm->mi_params and cm->width / cm->height where the coded size differs from the crop size (superres / resize);
+ * 0 keeps the value tfref_create derived from the crop size.  Call before tfref_run.  A setter rather than tfref_cfg
+ * fields, so that the layout of tfref_cfg stays what existing callers were built against. */
+TFREF_API void tfref_set_coded(void *h, int mi_rows, int mi_cols, int cm_width, int cm_height) {
+  AV1_COMMON *cm = &((tfref_ctx *)h)->cpi->common;
+  if (mi_rows > 0) cm->mi_params.mi_rows = mi_rows;
+  if (mi_cols > 0) cm->mi_params.mi_cols = mi_cols;
+  if (cm_width > 0) cm->width = cm_width;
+  if (cm_height > 0) cm->height = cm_height;
+}
+
 TFREF_API void tfref_set_frame(void *h, int idx, const void *y, const void *u,
                                const void *v) {
   tfref_ctx *t = (tfref_ctx *)h;

@@ -22,8 +22,10 @@ static int align_pow2(int v, int n) { return (v + (1 << n) - 1) & ~((1 << n) - 1
 
 /* Event counters (tf_oracle.h): observe only. */
 static tfo_stats g_stats;
-void tfo_reset_stats(void) { memset(&g_stats, 0, sizeof(g_stats)); }
+static tfo_limit_stats g_lstats;
+void tfo_reset_stats(void) { memset(&g_stats, 0, sizeof(g_stats)); memset(&g_lstats, 0, sizeof(g_lstats)); }
 void tfo_get_stats(tfo_stats *out) { *out = g_stats; }
+void tfo_get_limit_stats(tfo_limit_stats *out) { *out = g_lstats; }
 
 typedef struct { int row, col; } mv_t; /* MV / FULLPEL_MV, av1/common/mv.h:37-47 */
 
@@ -44,6 +46,7 @@ typedef struct {
 struct tfo_ctx {
   tfo_params p;
   int num_planes, num_pels, mb_rows, mb_cols, mi_rows, mi_cols;
+  int min_cm_size; /* AOMMIN(cm->width, cm->height), temporal_filter.c:99-100 */
   frame_t *frames;
   frame_t out;
 };
@@ -53,7 +56,11 @@ static void frame_alloc(frame_t *f, const tfo_params *p) {
   /* yv12config.c:229-245: aligned_width=(w+7)&~7, y_stride=align32(aw+2*border),
    * uv dims = aligned >> ss, uv_stride = y_stride >> ss_x, uv border = border >> ss */
   const int aw = align_pow2(p->width, 3), ah = align_pow2(p->height, 3);
-  const int border = p->border;
+  /* The frames' own border is border_in_pixels, but at least 64 (AOM_ENC_ALLINTRA_BORDER, the smallest the encoder
+   * configures).  Below 64 the MV limits still keep the luma reads inside border_in_pixels, but a chroma predictor
+   * at the limit reads (limit >> ss) + 5 samples out, past a (border >> ss) chroma border; the library's frames
+   * have a wide replicated border, so the oracle gives those reads replicated samples too. */
+  const int border = MAXI(p->border, 64);
   f->aw[0] = aw; f->ah[0] = ah;
   f->aw[1] = aw >> p->ss_x; f->ah[1] = ah >> p->ss_y;
   f->crop_w[0] = p->width; f->crop_h[0] = p->height;
@@ -73,14 +80,15 @@ static void frame_alloc(frame_t *f, const tfo_params *p) {
 }
 static void frame_free(frame_t *f) { for (int i = 0; i < 3; i++) free(f->alloc[i]); }
 
-/* extend.c:20-65 (copy_and_extend_plane) with the extents of :113-131 */
+/* extend.c:20-65 (copy_and_extend_plane) with the extents of :113-131 (dst->border: the frame's own border) */
 static void plane_fill(frame_t *f, int pl, const void *src, int use_hbd, const tfo_params *p) {
   const int c = pl > 0;
   const int w = f->crop_w[c], h = f->crop_h[c], st = f->stride[c];
-  const int er_y = MAXI(f->aw[0] + p->border, align_pow2(f->aw[0], 6)) - f->crop_w[0];
-  const int eb_y = MAXI(f->ah[0] + p->border, align_pow2(f->ah[0], 6)) - f->crop_h[0];
-  const int et = c ? p->border >> p->ss_y : p->border;
-  const int el = c ? p->border >> p->ss_x : p->border;
+  const int border = f->bw[0];
+  const int er_y = MAXI(f->aw[0] + border, align_pow2(f->aw[0], 6)) - f->crop_w[0];
+  const int eb_y = MAXI(f->ah[0] + border, align_pow2(f->ah[0], 6)) - f->crop_h[0];
+  const int et = c ? border >> p->ss_y : border;
+  const int el = c ? border >> p->ss_x : border;
   const int er = c ? er_y >> p->ss_x : er_y;
   const int eb = c ? eb_y >> p->ss_y : eb_y;
   uint16_t *dst = f->buf[pl];
@@ -104,12 +112,20 @@ tfo_ctx *tfo_create(const tfo_params *p) {
   c->num_pels = 1024 + (p->monochrome ? 0 : 2 * (1024 >> (p->ss_x + p->ss_y)));
   c->mb_rows = (p->height + 31) / 32; /* temporal_filter.c:1236-1237 */
   c->mb_cols = (p->width + 31) / 32;
-  c->mi_rows = align_pow2(p->height, 3) >> 2;
-  c->mi_cols = align_pow2(p->width, 3) >> 2;
+  tfo_set_coded(c, 0, 0, 0, 0);
   c->frames = (frame_t *)calloc(p->num_frames, sizeof(frame_t));
   for (int i = 0; i < p->num_frames; i++) frame_alloc(&c->frames[i], p);
   frame_alloc(&c->out, p);
   return c;
+}
+void tfo_set_coded(tfo_ctx *c, int mi_rows, int mi_cols, int cm_width, int cm_height) {
+  const tfo_params *p = &c->p;
+  /* cm->mi_params (alloccommon.c enc_set_mb_mi: 4-px units of the 8-aligned coded size) unless given */
+  c->mi_rows = mi_rows > 0 ? mi_rows : align_pow2(p->height, 3) >> 2;
+  c->mi_cols = mi_cols > 0 ? mi_cols : align_pow2(p->width, 3) >> 2;
+  /* cm->width / cm->height: the coded size, equal to the crop size unless given */
+  const int cm_w = cm_width > 0 ? cm_width : p->width, cm_h = cm_height > 0 ? cm_height : p->height;
+  c->min_cm_size = MINI(cm_w, cm_h);
 }
 void tfo_destroy(tfo_ctx *c) {
   if (!c) return;
@@ -561,12 +577,19 @@ static int in_range(const limits_t *l, int r, int c) {
   return c >= l->col_min && c <= l->col_max && r >= l->row_min && r <= l->row_max;
 }
 
+/* clamp_fullmv, as diamond_search_sad and exhaustive_mesh_search call it on their start MV: clamp() tests the low
+ * bound first (v < lo ? lo : v > hi ? hi : v), so the high bound wins when the limits invert.  Counted. */
+static mv_t clamp_start(const limits_t *l, mv_t mv) {
+  const mv_t c = { clampi(mv.row, l->row_min, l->row_max), clampi(mv.col, l->col_min, l->col_max) };
+  g_lstats.start_clamped += c.row != mv.row || c.col != mv.col;
+  return c;
+}
+
 /* diamond_search_sad mcomp.c:1299-1416 */
 static unsigned diamond_search(const search_t *s, mv_t start, int search_step, int skip, int *num00,
                                mv_t *best_mv) {
   const sites_t *cfg = s->sites;
-  start.col = clampi(start.col, s->lim.col_min, s->lim.col_max);
-  start.row = clampi(start.row, s->lim.row_min, s->lim.row_max);
+  start = clamp_start(&s->lim, start);
   const int tot_steps = 15 - search_step;
   *num00 = 0;
   *best_mv = start;
@@ -640,8 +663,7 @@ static void upd(const search_t *s, unsigned this_sad, int r, int c, unsigned *be
 /* exhaustive_mesh_search mcomp.c:1474-1543 */
 static int mesh_search(const search_t *s, mv_t start, int range, int step, int skip, mv_t *best_mv) {
   const int col_step = (step > 1) ? step : 4;
-  start.col = clampi(start.col, s->lim.col_min, s->lim.col_max);
-  start.row = clampi(start.row, s->lim.row_min, s->lim.row_max);
+  start = clamp_start(&s->lim, start);
   *best_mv = start;
   unsigned best_sad = s_sad(s, start.row, start.col, skip) + sad_cost(s, start.row, start.col);
   const int start_row = MAXI(-range, s->lim.row_min - start.row);
@@ -892,30 +914,41 @@ static unsigned subpel_search(const search_t *s, mv_t start_full, mv_t *best) {
 static void set_limits(const tfo_ctx *c, int mi_row, int mi_col, int mi_size, limits_t *l) {
   const int border = c->p.border;
   const int mih = mi_size, miw = mi_size;
-  l->row_min = MAXI(-(mi_row * 4 + border - 8), -(((mi_row + mih) * 4) + 8));
-  l->row_max = MINI((c->mi_rows - mi_row - mih) * 4 + border - 8, (c->mi_rows - mi_row) * 4 + 8);
-  l->col_min = MAXI(-(mi_col * 4 + border - 8), -(((mi_col + miw) * 4) + 8));
-  l->col_max = MINI((c->mi_cols - mi_col - miw) * 4 + border - 8, (c->mi_cols - mi_col) * 4 + 8);
+  /* cm->mi_params: c->mi_rows / c->mi_cols (the coded grid) */
+  const int b_row_min = -(mi_row * 4 + border - 8), b_row_max = (c->mi_rows - mi_row - mih) * 4 + border - 8;
+  const int b_col_min = -(mi_col * 4 + border - 8), b_col_max = (c->mi_cols - mi_col - miw) * 4 + border - 8;
+  const int e_row_min = -(((mi_row + mih) * 4) + 8), e_row_max = (c->mi_rows - mi_row) * 4 + 8;
+  const int e_col_min = -(((mi_col + miw) * 4) + 8), e_col_max = (c->mi_cols - mi_col) * 4 + 8;
+  l->row_min = MAXI(b_row_min, e_row_min);
+  l->row_max = MINI(b_row_max, e_row_max);
+  l->col_min = MAXI(b_col_min, e_col_min);
+  l->col_max = MINI(b_col_max, e_col_max);
   /* ref_mv = 0: [-1023, 1023] intersect (MV_LOW/8+1.. never binds) */
   l->col_min = MAXI(l->col_min, -1023); l->col_max = MINI(l->col_max, 1023);
   l->row_min = MAXI(l->row_min, -1023); l->row_max = MINI(l->row_max, 1023);
+  /* counters only */
+  g_lstats.lim_inverted += l->row_min > l->row_max || l->col_min > l->col_max;
+  g_lstats.lim_border_bound += (b_row_min > e_row_min && b_row_min > -1023) || (b_row_max < e_row_max && b_row_max < 1023) ||
+                              (b_col_min > e_col_min && b_col_min > -1023) || (b_col_max < e_col_max && b_col_max < 1023);
 }
 
 /* tf_motion_search temporal_filter.c:94-130: the search state of one frame pair; returns step_param */
 static int search_setup(const tfo_ctx *c, const sites_t *sites, int stride, search_t *s, int *skip) {
   const tfo_params *p = &c->p;
-  const int min_frame_size = MINI(p->width, p->height);
+  /* :99-100 min_frame_size = AOMMIN(cm->width, cm->height): the coded size */
+  const int min_frame_size = c->min_cm_size;
   memset(s, 0, sizeof(*s));
   s->p = p;
   s->stride = stride;
   s->sites = sites;
   s->min_frame_size = min_frame_size;
+  /* :119-122 MV_COST_L1_{HDRES,MIDRES,LOWRES} by min_frame_size, mcomp.c:237-244 */
   if (min_frame_size >= 720) { s->sad_lambda = 8; s->sse_lambda = 1; }
   else if (min_frame_size >= 480) { s->sad_lambda = 15; s->sse_lambda = 0; }
   else { s->sad_lambda = 32; s->sse_lambda = 2; }
   /* use_downsampled_sad && block_size_high >= 16: true for both sizes */
   *skip = p->use_downsampled_sad ? 1 : 0;
-  /* av1_init_search_range mcomp.c:217-226 */
+  /* av1_init_search_range mcomp.c:217-226 of the larger crop dimension of the frame to filter (not cm->width) */
   int size = MAXI(16, MAXI(p->width, p->height));
   int step_param = 0;
   while ((size << step_param) < 1023) step_param++;
@@ -956,7 +989,7 @@ static void motion_search(const tfo_ctx *c, const sites_t *sites, const frame_t 
   const tfo_params *p = &c->p;
   const int st = cur->stride[0];
   const int y_offset = mb_row * 32 * st + mb_col * 32;
-  const int min_frame_size = MINI(p->width, p->height);
+  const int min_frame_size = c->min_cm_size; /* :99-100, AOMMIN(cm->width, cm->height) */
   search_t s;
   int skip;
   const int step_param = search_setup(c, sites, st, &s, &skip);
@@ -1006,7 +1039,7 @@ static void motion_search(const tfo_ctx *c, const sites_t *sites, const frame_t 
       (((int64_t)block_mse * 14 < sum * 4) && mx - mn < 24)) {
     for (int i = 0; i < 4; i++) { sub_mvs[i] = block_mv; sub_mses[i] = block_mse; }
   }
-  const int thresh = (min_frame_size >= 720) ? 12 : 3;
+  const int thresh = (min_frame_size >= 720) ? 12 : 3; /* :249-250 */
   g_stats.block_mse_at_thresh += block_mse == (thresh << (p->bit_depth - 8));
   if (block_mse > (thresh << (p->bit_depth - 8))) { ref_mv->row = 0; ref_mv->col = 0; g_stats.ref_mv_resets++; }
 }

@@ -38,6 +38,12 @@ typedef struct {
 typedef struct tfo_ctx tfo_ctx;
 
 tfo_ctx *tfo_create(const tfo_params *p);
+/* cm->mi_params.mi_rows / mi_cols (4-px units; the MV limits, mcomp.h:216-240) and cm->width / cm->height (the coded
+ * size: MV cost class and ref_mv reset threshold, temporal_filter.c:99-100,119-122,249-250), which differ from the
+ * crop size under superres / resize.  0 = derived from the crop size (what tfo_create sets): align8(crop) / 4, and
+ * the crop size itself.  Call before any search.  A setter rather than tfo_params fields, so that the layout of
+ * tfo_params stays what existing callers were built against. */
+void tfo_set_coded(tfo_ctx *c, int mi_rows, int mi_cols, int cm_width, int cm_height);
 void tfo_destroy(tfo_ctx *c);
 /* planes: crop-sized, tightly packed, u8 (use_hbd=0) or u16 (use_hbd=1) */
 void tfo_set_frame(tfo_ctx *c, int idx, const void *y, const void *u, const void *v);
@@ -101,8 +107,16 @@ typedef struct {
   int64_t block_mse_at_thresh; /* block_mse == thresh exactly (the reset's boundary) */
   int64_t sad_peak_groups;    /* 16-sample aligned row groups of a SAD whose every |difference| is (1 << bd) - 1 */
 } tfo_stats;
+/* Counters of the MV limits, in a struct of their own (tfo_stats keeps its layout); tfo_reset_stats zeroes them too. */
+typedef struct {
+  int64_t lim_inverted;       /* MV limits with an empty row or column interval (min > max) */
+  int64_t start_clamped;      /* search starts moved by the clamp into the limits (diamond and mesh) */
+  int64_t lim_border_bound;   /* MV limits with a bound set by the border_in_pixels term (strictly tighter than
+                                 the +-8 term and inside the +-1023 clamp) */
+} tfo_limit_stats;
 void tfo_reset_stats(void);
 void tfo_get_stats(tfo_stats *out);
+void tfo_get_limit_stats(tfo_limit_stats *out);
 
 #ifdef __cplusplus
 }

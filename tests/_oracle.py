@@ -28,13 +28,59 @@ class OParams(C.Structure):
     ]
 
 
-STAT_FIELDS = ("mesh_searches", "diamond_ties", "mesh_ties", "subpel_ties", "conv_im_overflow", "pred_clip_lo",
-               "pred_clip_hi", "mv_on_limit", "mv_on_clamp", "ref_mv_resets", "block_mse_at_thresh",
-               "sad_peak_groups")
+BASE_STAT_FIELDS = ("mesh_searches", "diamond_ties", "mesh_ties", "subpel_ties", "conv_im_overflow", "pred_clip_lo",
+                    "pred_clip_hi", "mv_on_limit", "mv_on_clamp", "ref_mv_resets", "block_mse_at_thresh",
+                    "sad_peak_groups")
+LIMIT_STAT_FIELDS = ("lim_inverted", "start_clamped", "lim_border_bound")
+STAT_FIELDS = BASE_STAT_FIELDS + LIMIT_STAT_FIELDS
+
+# optional keys of the params dict: the coded grid and size the encoder passes (0 or absent: the crop size's),
+# handed to tfo_set_coded in this order
+CODED_KEYS = ("mi_rows", "mi_cols", "cm_width", "cm_height")
 
 
-class OStats(C.Structure):
-    _fields_ = [(k, C.c_int64) for k in STAT_FIELDS]
+class OStats(C.Structure):  # tfo_stats
+    _fields_ = [(k, C.c_int64) for k in BASE_STAT_FIELDS]
+
+
+class OLimitStats(C.Structure):  # tfo_limit_stats
+    _fields_ = [(k, C.c_int64) for k in LIMIT_STAT_FIELDS]
+
+
+def coded_values(p):
+    """The tfo_set_coded arguments of a params dict: mi_rows, mi_cols, cm_width, cm_height (0 where absent)."""
+    return tuple(int(p.get(k) or 0) for k in CODED_KEYS)
+
+
+def bind_common(l):
+    """argtypes of the entry points the filter oracle and the motion oracle library share."""
+    l.tfo_create.restype = C.c_void_p
+    l.tfo_create.argtypes = [C.POINTER(OParams)]
+    l.tfo_set_coded.argtypes = [C.c_void_p] + [C.c_int] * 4
+    l.tfo_set_coded.restype = None
+    l.tfo_destroy.argtypes = [C.c_void_p]
+    l.tfo_set_frame.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
+    l.tfo_reset_stats.argtypes = []
+    l.tfo_reset_stats.restype = None
+    l.tfo_get_stats.argtypes = [C.POINTER(OStats)]
+    l.tfo_get_stats.restype = None
+    l.tfo_get_limit_stats.argtypes = [C.POINTER(OLimitStats)]
+    l.tfo_get_limit_stats.restype = None
+
+
+def create(l, p):
+    """tfo_create + tfo_set_coded for a params dict; returns (handle, OParams kept alive)."""
+    cp = make_params(p)
+    h = l.tfo_create(C.byref(cp))
+    l.tfo_set_coded(h, *coded_values(p))
+    return h, cp
+
+
+def read_stats(l):
+    st, ls = OStats(), OLimitStats()
+    l.tfo_get_stats(C.byref(st))
+    l.tfo_get_limit_stats(C.byref(ls))
+    return {**{k: int(getattr(st, k)) for k in BASE_STAT_FIELDS}, **{k: int(getattr(ls, k)) for k in LIMIT_STAT_FIELDS}}
 
 
 _lib = None
@@ -50,10 +96,7 @@ def lib():
     if _lib is None:
         build()
         l = C.CDLL(LIB)
-        l.tfo_create.restype = C.c_void_p
-        l.tfo_create.argtypes = [C.POINTER(OParams)]
-        l.tfo_destroy.argtypes = [C.c_void_p]
-        l.tfo_set_frame.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
+        bind_common(l)
         l.tfo_estimate_noise.restype = C.c_double
         l.tfo_estimate_noise.argtypes = [C.c_void_p, C.c_int, C.c_int]
         l.tfo_estimate_noise_thresh.restype = C.c_double
@@ -76,10 +119,6 @@ def lib():
                                           + [C.c_int] * 4 + [C.POINTER(C.c_uint)])
         l.tfo_convolve12.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int] + [C.c_int] * 6
         l.tfo_od_divu.argtypes = [C.c_uint, C.c_uint]
-        l.tfo_reset_stats.argtypes = []
-        l.tfo_reset_stats.restype = None
-        l.tfo_get_stats.argtypes = [C.POINTER(OStats)]
-        l.tfo_get_stats.restype = None
         _lib = l
     return _lib
 
@@ -94,10 +133,9 @@ def reset_stats():
 
 
 def get_stats():
-    """The oracle's event counters since the last reset_stats(), as a dict (see tfo_stats in tf_oracle.h)."""
-    st = OStats()
-    lib().tfo_get_stats(C.byref(st))
-    return {k: int(getattr(st, k)) for k in STAT_FIELDS}
+    """The oracle's event counters since the last reset_stats(), as a dict (tfo_stats and tfo_limit_stats in
+    tf_oracle.h)."""
+    return read_stats(lib())
 
 
 def make_params(p):
@@ -117,8 +155,7 @@ def make_params(p):
 class OracleFilter:
     def __init__(self, p, frames):
         self.p = dict(p)
-        self.cp = make_params(p)
-        self.h = lib().tfo_create(C.byref(self.cp))
+        self.h, self.cp = create(lib(), p)
         self.num_planes = 1 if p["monochrome"] else 3
         self.mb_rows = (p["height"] + 31) // 32
         self.mb_cols = (p["width"] + 31) // 32

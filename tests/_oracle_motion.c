@@ -42,3 +42,14 @@ void tfo_motion_search(tfo_ctx *c, int src_idx, int ref_idx, int bsize, int x, i
   out[4] = best.col;
   out[5] = (int)err;
 }
+
+/* The full-pel MV limits set_limits gives a bsize x bsize block at luma (x, y): out = row_min, row_max, col_min,
+ * col_max. */
+void tfo_mv_limits(tfo_ctx *c, int bsize, int x, int y, int *out) {
+  limits_t l;
+  set_limits(c, y >> 2, x >> 2, bsize >> 2, &l);
+  out[0] = l.row_min;
+  out[1] = l.row_max;
+  out[2] = l.col_min;
+  out[3] = l.col_max;
+}

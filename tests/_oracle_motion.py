@@ -37,15 +37,9 @@ def lib():
     global _lib
     if _lib is None:
         l = C.CDLL(build())
-        l.tfo_create.restype = C.c_void_p
-        l.tfo_create.argtypes = [C.POINTER(_oracle.OParams)]
-        l.tfo_destroy.argtypes = [C.c_void_p]
-        l.tfo_set_frame.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
+        _oracle.bind_common(l)
         l.tfo_motion_search.argtypes = [C.c_void_p] + [C.c_int] * 7 + [C.POINTER(C.c_int)]
-        l.tfo_reset_stats.argtypes = []
-        l.tfo_reset_stats.restype = None
-        l.tfo_get_stats.argtypes = [C.POINTER(_oracle.OStats)]
-        l.tfo_get_stats.restype = None
+        l.tfo_mv_limits.argtypes = [C.c_void_p] + [C.c_int] * 3 + [C.POINTER(C.c_int)]
         _lib = l
     return _lib
 
@@ -56,17 +50,14 @@ def reset_stats():
 
 
 def get_stats():
-    st = _oracle.OStats()
-    lib().tfo_get_stats(C.byref(st))
-    return {k: int(getattr(st, k)) for k in _oracle.STAT_FIELDS}
+    return _oracle.read_stats(lib())
 
 
 class MotionOracle:
     """Frames as for _oracle.OracleFilter (params dict of tests/_params.tf_params, list of (y, u, v))."""
 
     def __init__(self, p, frames):
-        self.cp = _oracle.make_params(p)
-        self.h = lib().tfo_create(C.byref(self.cp))
+        self.h, self.cp = _oracle.create(lib(), p)
         dt = np.uint16 if p["use_hbd"] else np.uint8
         for i, planes in enumerate(frames):  # tfo_set_frame copies the samples
             arrs = [None if a is None else np.ascontiguousarray(a.astype(dt)) for a in planes]
@@ -77,6 +68,12 @@ class MotionOracle:
         out = (C.c_int * 6)()
         lib().tfo_motion_search(self.h, src_idx, ref_idx, bsize, x, y, start_row, start_col, out)
         return tuple(int(v) for v in out[:5]) + (out[5] & 0xffffffff,)
+
+    def mv_limits(self, bsize, x, y):
+        """The full-pel MV limits of a bsize block at (x, y): (row_min, row_max, col_min, col_max)."""
+        out = (C.c_int * 4)()
+        lib().tfo_mv_limits(self.h, bsize, x, y, out)
+        return tuple(out)
 
     def close(self):
         if self.h:

@@ -158,6 +158,10 @@ class RefFilter:
         self.L = seam_lib() if seam else avx2_lib() if avx2 else lib()
         self.h = self.L.tfref_create(C.byref(self.cfg))
         assert self.h
+        coded = tuple(int(p.get(k) or 0) for k in ("mi_rows", "mi_cols", "cm_width", "cm_height"))
+        if any(coded):  # the coded grid and size, where they differ from the crop size's
+            self.L.tfref_set_coded.argtypes = [C.c_void_p] + [C.c_int] * 4
+            self.L.tfref_set_coded(self.h, *coded)
         self.num_planes = 1 if p["monochrome"] else 3
         self.mb_rows = (p["height"] + 31) // 32
         self.mb_cols = (p["width"] + 31) // 32

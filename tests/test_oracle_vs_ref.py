@@ -63,6 +63,35 @@ def test_oracle_equals_reference(case):
     o.close()
 
 
+# coded size and grid decoupled from the crop size (superres / resize): name, W, H, coded W, coded H, N, bit depth,
+# border, parameter options
+CODED_CASES = [
+    ("half_720_lowres", 1280, 720, 640, 360, 5, 10, 160, dict(speed=4)),
+    ("sr9_wide_mid", 704, 544, 626, 544, 4, 8, 288, dict(speed=2, allow_hp=1)),
+    ("half_width_inverted", 2816, 64, 1408, 64, 3, 8, 288, dict(speed=0)),  # column limits invert for x > 2439
+]
+# (no border below 64 here: the reference's frames are allocated with border_in_pixels, and a chroma predictor at
+# such a border's MV limit reads past them; the oracle's frames have a border of at least 64)
+
+
+@pytest.mark.parametrize("case", CODED_CASES, ids=[c[0] for c in CODED_CASES])
+def test_oracle_equals_reference_on_coded_sizes(case):
+    """cm->width / cm->height and cm->mi_params set apart from the crop size: the cost class, the ref_mv reset
+    threshold and the MV limits (inverted ones included) follow them in both."""
+    name, W, H, cw, ch, N, bd, border, pkw = case
+    frames = _clips.moving_texture(W, H, N, bd, motion=(2, 9))
+    p = _params.tf_params(W, H, N, bit_depth=bd, border=border, **pkw)
+    p.update(cm_width=cw, cm_height=ch, mi_rows=(ch + 7) // 8 * 2, mi_cols=(cw + 7) // 8 * 2)
+    r, o = _ref.RefFilter(p, frames), _oracle.OracleFilter(p, frames)
+    a, b = r.run(), o.run()
+    for k in ("mvs", "mses", "pred", "diff"):
+        assert (a[k] == b[k]).all(), k
+    for x, y in zip(a["out"], b["out"]):
+        assert (x == y).all()
+    r.close()
+    o.close()
+
+
 def test_od_divu_equals_division_exhaustive():
     """OD_DIVU (aom_dsp/odintrin.h:30-42) uses a multiply-shift table for d < 1024; the product
     and the oracle use plain division.  Proven equal for every count in [1000,1023] and every
