@@ -9,7 +9,7 @@
 // frame and FRAME_DIFF.  No CPU fallback: without a CUDA device every entry
 // point returns TF_GPU_ERR_NO_DEVICE.
 #include "tf_kernels.cuh"
-#include <cuda.h>  // CUtensorMap types only; the encoder is fetched through cudaGetDriverEntryPoint (no libcuda link)
+#include <cuda.h>  // CUdeviceptr / CUresult only; cuMemGetAddressRange is fetched through cudaGetDriverEntryPoint (no libcuda link)
 
 #include <math.h>
 #include <stdarg.h>
@@ -45,9 +45,6 @@ struct DevFrame {
   void *base[3] = { nullptr, nullptr, nullptr };  // allocation base
   void *p00[3] = { nullptr, nullptr, nullptr };   // pixel (0,0)
   cudaEvent_t ready = nullptr;                    // upload + border extension finished (copy stream)
-  // TMA descriptors of the luma plane (device memory, 2 x 128 bytes: box of a 16x16 and of a 32x32 skip-row
-  // candidate), see make_tensor_maps(); nullptr when the driver has no tensor-map encoder
-  void *d_tmap = nullptr;
 };
 
 // Timing events of one filter call (main stream): start, after the search32 chain, after the
@@ -110,12 +107,6 @@ struct tf_gpu_ctx {
   unsigned long long *d_ctr = nullptr;    // [4] executed-work counters (instrumentation)
   unsigned long long h_ctr[4] = { 0, 0, 0, 0 };
   bool collect_counters = false;
-  // development switches (environment, read once at create): TF_GPU_CHAIN=fused|frames overrides the choice of
-  // the latency mode in launch_filter(); TF_GPU_S16=single launches the 16x16 searches of
-  // all frames as one grid after the chain instead of one grid per frame; TF_GPU_PRIO=flat gives every stream
-  // the same priority
-  int s16_mode = 0;  // TF_GPU_S16: 1 = single launch after the chain, otherwise one launch per frame
-  int chain_mode = 0;  // TF_GPU_CHAIN: 0 = auto (fused for row-range calls resident in one wave), 1 = fused, 2 = per frame
   unsigned long long *h_noise = nullptr;
   Ticket tickets[8];
   uint64_t next_ticket = 1;
@@ -198,25 +189,6 @@ bool make_geometry(const tf_gpu_frame *f, int num_planes, Geometry *g, int luma_
   return true;
 }
 
-// TMA descriptors for the far candidates of the search kernels: the luma allocation as a 3-D tensor
-// (x, row parity, row / 2) so that a box of (W + pad, 1, W / 2) elements at (X & ~(pad - 1), Y & 1, Y >> 1) holds
-// exactly the W / 2 rows Y, Y + 2, ... of a skip-row SAD candidate (aom_dsp/sad.c:66-70), landing dense in
-// shared memory (pad = 16 bytes of samples: the innermost box coordinate has to be 16-byte aligned).
-typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
-                                  const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn encode_tiled_fn() {
-  static EncodeTiledFn fn = nullptr;
-  static bool tried = false;
-  if (!tried) {
-    tried = true;
-    void *p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-      fn = (EncodeTiledFn)p;
-  }
-  return fn;
-}
 // cuMemGetAddressRange (allocation base and size of a device pointer), for the extent check of device frames
 typedef CUresult (*AddressRangeFn)(CUdeviceptr *, size_t *, CUdeviceptr);
 AddressRangeFn address_range_fn() {
@@ -268,31 +240,7 @@ int check_device_extent(tf_gpu_ctx *ctx, const void *ptr, size_t bytes, size_t a
   }
   return TF_GPU_OK;
 }
-int make_tensor_maps(tf_gpu_ctx *ctx, DevFrame *d) {
-  EncodeTiledFn enc = encode_tiled_fn();
-  if (!enc) return fail(ctx, TF_GPU_ERR_CUDA, "cuTensorMapEncodeTiled is not available in this driver");
-  const Geometry &g = d->g;
-  const size_t es = g.is_hbd ? 2 : 1;
-  alignas(64) CUtensorMap maps[2];
-  for (int k = 0; k < 2; k++) {
-    const cuuint32_t W = k ? 32 : 16;
-    const cuuint64_t dims[3] = { (cuuint64_t)g.pitch[0], 2, (cuuint64_t)(g.rows[0] / 2) };
-    const cuuint64_t strides[2] = { (cuuint64_t)g.pitch[0] * es, (cuuint64_t)g.pitch[0] * es * 2 };
-    // the innermost start coordinate of a box copy must be 16-byte aligned (an unaligned one is an illegal
-    // instruction): the box is 16 bytes wider than the candidate and starts at the aligned column below it
-    const cuuint32_t box[3] = { W + (cuuint32_t)(16 / es), 1, W / 2 };
-    const cuuint32_t estr[3] = { 1, 1, 1 };
-    const CUresult r = enc(&maps[k], g.is_hbd ? CU_TENSOR_MAP_DATA_TYPE_UINT16 : CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, d->base[0], dims,
-                           strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                           CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(ctx, TF_GPU_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d)", (int)r);
-  }
-  if (!d->d_tmap) CU(cudaMalloc(&d->d_tmap, sizeof(maps)));
-  CU(cudaMemcpy(d->d_tmap, maps, sizeof(maps), cudaMemcpyHostToDevice));
-  return TF_GPU_OK;
-}
-
-int alloc_dev_frame(tf_gpu_ctx *ctx, DevFrame *d, const Geometry &g, bool with_maps = false) {
+int alloc_dev_frame(tf_gpu_ctx *ctx, DevFrame *d, const Geometry &g) {
   const size_t es = g.is_hbd ? 2 : 1;
   if (d->base[0] && d->g == g) return TF_GPU_OK;
   for (int p = 0; p < 3; p++) {
@@ -307,7 +255,6 @@ int alloc_dev_frame(tf_gpu_ctx *ctx, DevFrame *d, const Geometry &g, bool with_m
     CU(cudaMalloc(&d->base[p], bytes));
     d->p00[p] = (char *)d->base[p] + ((size_t)g.by[k] * g.pitch[k] + g.bx[k]) * es;
   }
-  if (with_maps && TF_FAR_TMA) return make_tensor_maps(ctx, d);  // descriptors only for the build that uses them
   return TF_GPU_OK;
 }
 
@@ -413,7 +360,7 @@ int get_frame(tf_gpu_ctx *ctx, const tf_gpu_frame *f, int num_planes, DevFrame *
       }
     }
     if (!victim) return fail(ctx, TF_GPU_ERR_MEM, "frame cache too small for this window");
-    int rc = alloc_dev_frame(ctx, victim, g, true);
+    int rc = alloc_dev_frame(ctx, victim, g);
     if (rc) return rc;
     victim->valid = false;
     {
@@ -555,8 +502,6 @@ void fill_kparams(const tf_gpu_ctx *ctx, const tf_gpu_params *p, const Geometry 
     K.pitch[k] = g.pitch[k];
     K.out_pitch[k] = ctx->out.g.pitch[k];
   }
-  K.abx = g.bx[0];
-  K.aby = g.by[0];
   K.border = p->border_in_pixels;
   K.num_frames = p->num_frames;
   K.filter_idx = p->filter_frame_idx;
@@ -611,15 +556,38 @@ void window_kparams(const tf_gpu_ctx *ctx, const tf_gpu_params *p, DevFrame *con
     double thr = min_frame_size * 0.1;  // TF_SEARCH_DISTANCE_THRESHOLD, :603-604
     K.dist_thr = thr > 1 ? thr : 1;
   }
-  for (int f = 0; f < p->num_frames; f++) {
+  for (int f = 0; f < p->num_frames; f++)
     for (int pl = 0; pl < p->num_planes; pl++) K.frm[f][pl] = frames[f]->p00[pl];
-    K.tmap[f] = frames[f]->d_tmap;
-  }
   for (int k = 0; k < 2; k++) K.out_pitch[k] = out.g.pitch[k];
   for (int pl = 0; pl < p->num_planes; pl++) K.out[pl] = out.p00[pl];
   K.num_pels = 1024 + (p->num_planes > 1 ? 2 * (1024 >> (g.ss_x + g.ss_y)) : 0);
   K.row_begin = 0;
   K.row_end = K.mb_rows;
+}
+
+// Warps per SM of the denser register build of the 32x32 search (16-bit samples: 128 registers / 16 warps per SM,
+// 1080p 10-bit 296 -> 310 frames/s; 8-bit: 96 / 20).
+int s32_warps_hi(int is_hbd) { return is_hbd ? S32_WARPS_HI_HBD : S32_WARPS_HI; }
+
+template <typename T, int MINB>
+auto search32_kernel(const KParams &) { return tf_search32_kernel<T, MINB>; }
+template <typename T, int MINB>
+auto search32_kernel(const KParamsBatch &) { return tf_search32_batch_kernel<T, MINB>; }
+
+// One launch of the 32x32 search on the main stream (KParamsBatch: the batched kernel).  The denser register build
+// only where it saves a second wave: a grid that is resident at once with the 168-register build runs faster per
+// block with it (no spills).
+template <typename KP>
+void launch_search32(const tf_gpu_ctx *ctx, int is_hbd, dim3 grid, const KP &K) {
+  const long long blocks = (long long)grid.x * grid.y;
+  const bool dense = blocks <= (long long)ctx->num_sms * s32_warps_hi(is_hbd) && blocks > (long long)ctx->num_sms * S32_WARPS_LO;
+  if (is_hbd) {
+    const auto kernel = dense ? search32_kernel<uint16_t, S32_WARPS_HI_HBD>(K) : search32_kernel<uint16_t, S32_WARPS_LO>(K);
+    kernel<<<grid, 32, SearchSmem<uint16_t, 32>::TOTAL, ctx->stream>>>(K);
+  } else {
+    const auto kernel = dense ? search32_kernel<uint8_t, S32_WARPS_HI>(K) : search32_kernel<uint8_t, S32_WARPS_LO>(K);
+    kernel<<<grid, 32, SearchSmem<uint8_t, 32>::TOTAL, ctx->stream>>>(K);
+  }
 }
 
 // Build kernel parameters and launch the block kernel over rows [rb, re).
@@ -689,23 +657,14 @@ int launch_filter(tf_gpu_ctx *ctx, const tf_gpu_params *p, DevFrame *const *fram
   // (ref_mv); one search32 launch walks all frames of its block instead (time = the slowest block's total, not
   // the sum of the per-frame maxima), followed by one search16 launch over all frames.
   const bool row_range = (K.row_end - K.row_begin) < K.mb_rows;
-  const int hi_warps = g.is_hbd ? S32_WARPS_HI_HBD : S32_WARPS_HI;
-  const bool fused_chain = nref > 0 && grid <= ctx->num_sms * hi_warps &&
-                           (ctx->chain_mode == 1 || (ctx->chain_mode == 0 && row_range));
+  const bool fused_chain = nref > 0 && row_range && grid <= ctx->num_sms * s32_warps_hi(g.is_hbd);
   if (fused_chain) {
     for (int f = 0; f < p->num_frames; f++)
       if (f != p->filter_frame_idx) CU(cudaStreamWaitEvent(ctx->stream, frames[f]->ready, 0));
     KParams Kf = K;
     Kf.frame_begin = 0;
     Kf.frame_end = p->num_frames;
-    const bool dense = grid > ctx->num_sms * S32_WARPS_LO;  // resident at once only with the denser build
-    if (g.is_hbd) {
-      if (dense) tf_search32_kernel<uint16_t, S32_WARPS_HI_HBD><<<grid, 32, SearchSmem<uint16_t, 32>::TOTAL_BASE, ctx->stream>>>(Kf);
-      else tf_search32_kernel<uint16_t, S32_WARPS_LO><<<grid, 32, SearchSmem<uint16_t, 32>::TOTAL, ctx->stream>>>(Kf);
-    } else {
-      if (dense) tf_search32_kernel<uint8_t, S32_WARPS_HI><<<grid, 32, SearchSmem<uint8_t, 32>::TOTAL_BASE, ctx->stream>>>(Kf);
-      else tf_search32_kernel<uint8_t, S32_WARPS_LO><<<grid, 32, SearchSmem<uint8_t, 32>::TOTAL, ctx->stream>>>(Kf);
-    }
+    launch_search32(ctx, g.is_hbd, grid, Kf);
     nlaunch++;
     if (timed) cudaEventRecord(te->evk[0], ctx->stream);
     if (!p->force_integer_mv) {
@@ -715,11 +674,9 @@ int launch_filter(tf_gpu_ctx *ctx, const tf_gpu_params *p, DevFrame *const *fram
     }
     if (timed) cudaEventRecord(te->evk[1], ctx->stream);
   } else if (nref > 0) {
-    // (one search16 launch over all frames after the chain instead: 4K 10-bit with three windows in flight
-    // 62.6 -> 63.6 frames/s, 1080p 329 -> 321, and a single window loses the overlap with its own chain: not the
-    // default)
-    const bool s16_single = ctx->s16_mode == 1;
-    bool any16 = false;
+    // (Measured and rejected: one search16 launch over all frames after the chain instead: 4K 10-bit with three
+    // windows in flight 62.6 -> 63.6 frames/s, 1080p 329 -> 321, and a single window loses the overlap with its own
+    // chain.)
     for (int f = 0; f < p->num_frames; f++) {
       if (f == p->filter_frame_idx) continue;
       KParams Kf = K;
@@ -727,20 +684,9 @@ int launch_filter(tf_gpu_ctx *ctx, const tf_gpu_params *p, DevFrame *const *fram
       Kf.frame_end = f + 1;
       if (f > 0 && f - 1 == p->filter_frame_idx) Kf.frame_begin = f - 1;  // negate ref_mv at the centre frame
       CU(cudaStreamWaitEvent(ctx->stream, frames[f]->ready, 0));  // uploads of later frames overlap this search
-      // the 96-register build only where it saves a second wave: a grid that is resident at once with the
-      // 168-register build runs faster per block with it (no spills)
-      // (16-bit samples: 128 registers / 16 warps per SM, 1080p 10-bit 296 -> 310 frames/s; 8-bit: 96 / 20)
-      const int hi = g.is_hbd ? S32_WARPS_HI_HBD : S32_WARPS_HI;
-      const bool one_wave = grid <= ctx->num_sms * hi && grid > ctx->num_sms * S32_WARPS_LO;
-      if (g.is_hbd) {
-        if (one_wave) tf_search32_kernel<uint16_t, S32_WARPS_HI_HBD><<<grid, 32, SearchSmem<uint16_t, 32>::TOTAL_BASE, ctx->stream>>>(Kf);
-        else tf_search32_kernel<uint16_t, S32_WARPS_LO><<<grid, 32, SearchSmem<uint16_t, 32>::TOTAL, ctx->stream>>>(Kf);
-      } else {
-        if (one_wave) tf_search32_kernel<uint8_t, S32_WARPS_HI><<<grid, 32, SearchSmem<uint8_t, 32>::TOTAL_BASE, ctx->stream>>>(Kf);
-        else tf_search32_kernel<uint8_t, S32_WARPS_LO><<<grid, 32, SearchSmem<uint8_t, 32>::TOTAL, ctx->stream>>>(Kf);
-      }
+      launch_search32(ctx, g.is_hbd, grid, Kf);
       nlaunch++;
-      if (!p->force_integer_mv && !s16_single) {
+      if (!p->force_integer_mv) {
         CU(cudaEventRecord(ctx->ev_f32[f], ctx->stream));
         CU(cudaStreamWaitEvent(ctx->stream2, ctx->ev_f32[f], 0));
         Kf.frame_begin = f;
@@ -751,19 +697,10 @@ int launch_filter(tf_gpu_ctx *ctx, const tf_gpu_params *p, DevFrame *const *fram
         if (g.is_hbd) tf_search16_kernel<uint16_t><<<grid * 4, 32, SearchSmem<uint16_t, 16>::TOTAL, ctx->stream2>>>(K16);
         else tf_search16_kernel<uint8_t><<<grid * 4, 32, SearchSmem<uint8_t, 16>::TOTAL, ctx->stream2>>>(K16);
         nlaunch++;
-        any16 = true;
       }
     }
     if (timed) cudaEventRecord(te->evk[0], ctx->stream);
-    if (!p->force_integer_mv && s16_single) {
-      KParams K16 = K;
-      K16.frame_begin = 0;
-      K16.frame_end = p->num_frames;
-      if (g.is_hbd) tf_search16_kernel<uint16_t><<<grid * 4 * nref, 32, SearchSmem<uint16_t, 16>::TOTAL, ctx->stream>>>(K16);
-      else tf_search16_kernel<uint8_t><<<grid * 4 * nref, 32, SearchSmem<uint8_t, 16>::TOTAL, ctx->stream>>>(K16);
-      nlaunch++;
-    }
-    if (any16) {
+    if (!p->force_integer_mv) {
       CU(cudaEventRecord(ctx->ev_s16, ctx->stream2));
       CU(cudaStreamWaitEvent(ctx->stream, ctx->ev_s16, 0));
     }
@@ -830,19 +767,7 @@ int launch_filter_batch(tf_gpu_ctx *ctx, int n, const tf_gpu_params *params,
   CU(cudaEventRecord(te->ev0, ctx->stream));
   int nlaunch = 0;
   if (n32) {
-    // the register build as launch_filter picks it for its per-frame grids, from the grid of the whole batch: the
-    // denser one only where it makes the grid resident in one wave
-    const long long total = (long long)nblk * n32;
-    const int hi = g.is_hbd ? S32_WARPS_HI_HBD : S32_WARPS_HI;
-    const bool one_wave = total <= (long long)ctx->num_sms * hi && total > (long long)ctx->num_sms * S32_WARPS_LO;
-    const dim3 grid(nblk, n32);
-    if (g.is_hbd) {
-      if (one_wave) tf_search32_batch_kernel<uint16_t, S32_WARPS_HI_HBD><<<grid, 32, SearchSmem<uint16_t, 32>::TOTAL_BASE, ctx->stream>>>(s32);
-      else tf_search32_batch_kernel<uint16_t, S32_WARPS_LO><<<grid, 32, SearchSmem<uint16_t, 32>::TOTAL, ctx->stream>>>(s32);
-    } else {
-      if (one_wave) tf_search32_batch_kernel<uint8_t, S32_WARPS_HI><<<grid, 32, SearchSmem<uint8_t, 32>::TOTAL_BASE, ctx->stream>>>(s32);
-      else tf_search32_batch_kernel<uint8_t, S32_WARPS_LO><<<grid, 32, SearchSmem<uint8_t, 32>::TOTAL, ctx->stream>>>(s32);
-    }
+    launch_search32(ctx, g.is_hbd, dim3(nblk, n32), s32);  // the register build from the grid of the whole batch
     nlaunch++;
   }
   CU(cudaEventRecord(te->evk[0], ctx->stream));
@@ -1071,23 +996,6 @@ int tf_gpu_create(tf_gpu_ctx **out, const tf_gpu_device_cfg *cfg) {
   // independent 16x16 searches that fill the machine underneath it
   int prio_lo = 0, prio_hi = 0;
   if (e == cudaSuccess) e = cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi);
-  {
-    const char *m = getenv("TF_GPU_S16");
-    ctx->s16_mode = m && strcmp(m, "single") == 0 ? 1 : (m && strcmp(m, "frames") == 0 ? 2 : 0);
-    const char *cm = getenv("TF_GPU_CHAIN");
-    ctx->chain_mode = cm && strcmp(cm, "fused") == 0 ? 1 : (cm && strcmp(cm, "frames") == 0 ? 2 : 0);
-    const char *pr = getenv("TF_GPU_PRIO");
-    if (pr && strcmp(pr, "flat") == 0) prio_hi = prio_lo;
-    // TF_GPU_CARVEOUT=<percent>: preferred shared-memory carveout of the search kernels (development switch)
-    const char *cv = getenv("TF_GPU_CARVEOUT");
-    if (cv && e == cudaSuccess) {
-      const int pct = atoi(cv);
-      cudaFuncSetAttribute(tf_search16_kernel<uint16_t>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
-      cudaFuncSetAttribute(tf_search16_kernel<uint8_t>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
-      cudaFuncSetAttribute(tf_search32_kernel<uint16_t, S32_WARPS_LO>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
-      cudaFuncSetAttribute(tf_search32_kernel<uint8_t, S32_WARPS_LO>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
-    }
-  }
   if (e == cudaSuccess) e = cudaStreamCreateWithPriority(&ctx->stream, cudaStreamNonBlocking, prio_hi);
   if (e == cudaSuccess) e = cudaStreamCreateWithPriority(&ctx->stream2, cudaStreamNonBlocking, prio_lo);
   if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking);
@@ -1151,7 +1059,6 @@ void tf_gpu_destroy(tf_gpu_ctx *ctx) {
   for (auto &d : ctx->cache) {
     for (int p = 0; p < 3; p++)
       if (d.base[p]) cudaFree(d.base[p]);
-    if (d.d_tmap) cudaFree(d.d_tmap);
     if (d.ready) cudaEventDestroy(d.ready);
   }
   for (int i = 0; i < 2; i++)
@@ -1662,11 +1569,7 @@ int enqueue_motion_search(tf_gpu_ctx *ctx, const tf_gpu_params &p, DevFrame *con
   fill_kparams(ctx, &p, g, K);
   // frames past the references are the source's: an item's ref is checked in the kernel, and even a wrong check
   // could then not reach a null or stale frame pointer
-  for (int f = 0; f < MAXF; f++) {
-    const DevFrame *d = devf[f <= num_refs ? f : 0];
-    K.frm[f][0] = d->p00[0];
-    K.tmap[f] = d->d_tmap;  // TF_FAR_TMA builds: each reference's own descriptors
-  }
+  for (int f = 0; f < MAXF; f++) K.frm[f][0] = devf[f <= num_refs ? f : 0]->p00[0];
   if (timed) CU(cudaEventRecord(ctx->ev0, ctx->stream));
   if (g.is_hbd) {
     if (block_size == 32) tf_motion_batch_kernel<uint16_t, 32><<<n, 32, SearchSmem<uint16_t, 32>::TOTAL, ctx->stream>>>(K, d_items, d_res, n);
@@ -1715,7 +1618,6 @@ int tf_gpu_fullpel_search_batch(tf_gpu_ctx *ctx, const tf_gpu_params *params, co
   }
   KParams K;
   fill_kparams(ctx, &p, g, K);
-  K.tmap[1] = dr->d_tmap;  // the reference frame's TMA descriptors (the kernel searches frame pair (0, 1))
   rc = ensure_dump(ctx, 10, (size_t)n * sizeof(SearchItem));
   if (rc) return rc;
   rc = ensure_dump(ctx, 11, (size_t)n * sizeof(SearchResult));

@@ -31,18 +31,6 @@ constexpr unsigned FULL = 0xffffffffu;
 #ifndef TF_PU16
 #define TF_PU16 2
 #endif
-// TF_SAD_IDP: high-bitdepth SAD as sum(a) + sum(b) - 2 sum(min(a, b)) with the sums on the FMA pipe (IDP.2A): the
-// ALU pipe (VIMNMX, shifts, logic: 54% busy in the 16x16 search) is the busier one, the FMA pipe idles at 16%.
-// 4K 10-bit 62.5 -> 63.4 frames/s.
-#ifndef TF_SAD_IDP
-#define TF_SAD_IDP 1
-#endif
-// TF_FILT_WUNROLL: unroll factor of the weight loop of the filter kernel (0 = full, the co-located luma sums
-// of the chroma planes precomputed in registers).  Not unrolled: the filter kernel shrinks from 64 to 40 KB of
-// code (its instruction-cache request rate was 89% of peak) and loses its spills: 2.85 -> 2.65 ms at 4K 10-bit.
-#ifndef TF_FILT_WUNROLL
-#define TF_FILT_WUNROLL 1
-#endif
 // Inlining policy: every search routine is inlined into its kernel.  A routine that is not inlined re-materialises
 // the global-memory descriptor for each of its loads (LDC + 2 x R2UR per LDG: 10% of the executed instructions of
 // both search kernels in the round-1 build) and passes its context through the stack; the out-of-line routines
@@ -83,8 +71,6 @@ struct KParams {
   // planes (pointers to pixel (0,0)); pitch in samples
   const void *frm[MAXF][3];
   int pitch[2];
-  const void *tmap[MAXF];  // per frame: TMA descriptors of the luma plane (16x16 box, then 32x32 box), device memory
-  int abx, aby;             // position of pixel (0, 0) inside the luma allocation the descriptors describe
   void *out[3];
   int out_pitch[2];
   unsigned long long *diff;  // [2]
@@ -164,11 +150,6 @@ struct Search {
   // from global memory through L1.
   unsigned char *win;  // nullptr = no window
   unsigned srcs;       // shared address of the source-block tile (SrcTile layout), 0 = not staged
-  // TMA staging of far candidates (diamond_search): the block's origin in allocation coordinates, the reference
-  // frame's descriptor for this block size, the staging buffer and its mbarrier (shared addresses)
-  int ax, ay;
-  const void *tmap;
-  unsigned farbuf, mbar;
   int wr, wc, wR;
   int wpitch;  // bytes; wpitch/4 is odd
   int wshift;  // bytes the window origin was aligned down by
@@ -177,10 +158,6 @@ struct Search {
   unsigned long long *ctr;
 };
 
-#ifndef TF_VAR_VIA_SUBPEL
-#define TF_VAR_VIA_SUBPEL 1
-#endif
-constexpr bool VAR_VIA_SUBPEL_ROUTINE = TF_VAR_VIA_SUBPEL != 0;
 constexpr int WIN_BYTES = 9472;  // window capacity per warp, 32x32 search
 constexpr int WIN16_BYTES = 4608;  // 16x16 search (R = 12): lets >= 24 warps share an SM
 
@@ -215,31 +192,10 @@ struct SrcTile {
   static constexpr int BYTES = W * PITCH;
 };
 // Dynamic shared memory of a search kernel: the window, then the source tile.
-// TF_FAR_TMA: far candidates of a diamond stage staged through TMA (cp.async.bulk.tensor, UTMALDG) instead of
-// per-lane global loads.  Built, parity-green (the whole GPU suite passes with it) and measured on one box against
-// the default: 4K 10-bit 54.8 vs 62.6 frames/s, 1080p 10-bit 318 vs 330, 1080p 8-bit 476 vs 499 -- the copies of a
-// stage are issued by one lane (as many issue slots as the loads they replace), their round trip is longer than
-// an L2 load's and nothing of the warp overlaps it, and because the innermost box coordinate must be 16-byte
-// aligned (an unaligned start is an illegal instruction: scripts/tma_probe.cu) the candidates do not land aligned,
-// so the funnel shifts stay.  Off by default; -DTF_FAR_TMA=1 builds it.
-#ifndef TF_FAR_TMA
-#define TF_FAR_TMA 0
-#endif
 template <typename T, int W>
 struct SearchSmem {
   static constexpr int WIN = (WinCfg<T, W>::ROWS * WinCfg<T, W>::PITCH + 15) / 16 * 16;
-  static constexpr int TOTAL_BASE = WIN + SrcTile<T, W>::BYTES;  // kernels without the TMA staging buffer
-  // far candidates of a diamond stage land here through TMA: the W/2 even rows of a candidate (skip-row SAD), each
-  // row from the 16-byte aligned column at or below the candidate's; eight sites of a stage at a time for the
-  // 16x16 search, four for the 32x32 search
-  static constexpr int FAR_PAD = 16 / (int)sizeof(T);                  // samples: the box starts at the 16-byte aligned column
-  static constexpr int FAR_ROWB = (W + FAR_PAD) * (int)sizeof(T);       // bytes per staged row
-  static constexpr int FAR_CAND = FAR_ROWB * (W / 2);                   // a multiple of 128 for every (T, W)
-  static constexpr int FAR_SLOTS = W == 16 ? 8 : 4;
-  static_assert(FAR_CAND % 128 == 0, "TMA destinations are 128-byte aligned");
-  static constexpr int FAR = (TOTAL_BASE + 127) / 128 * 128;
-  static constexpr int MBAR = FAR + FAR_SLOTS * FAR_CAND;  // 8-byte mbarrier, then its phase word
-  static constexpr int TOTAL = TF_FAR_TMA ? MBAR + 16 : TOTAL_BASE;
+  static constexpr int TOTAL = WIN + SrcTile<T, W>::BYTES;
   static_assert((W + 7) * W * (int)sizeof(T) <= WIN, "8-tap scratch of SUBPEL_TREE lives in the window buffer");
 };
 template <typename T, int W>
@@ -388,50 +344,6 @@ __device__ __forceinline__ uint32_t lds_u16(unsigned addr) {
   asm("ld.shared.u16 %0, [%1];" : "=r"(v) : "r"(addr));
   return v;
 }
-// mbarrier + TMA (cp.async.bulk.tensor) wrappers for the far-candidate staging; shared addresses are 32-bit.
-__device__ __forceinline__ void sts_u32(unsigned addr, uint32_t v) { asm volatile("st.shared.u32 [%0], %1;" ::"r"(addr), "r"(v) : "memory"); }
-__device__ __forceinline__ void mbar_init(unsigned bar, unsigned count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-  asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(unsigned bar, unsigned bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(unsigned bar, unsigned parity) {
-  // bounded: a copy that never completes (a descriptor / coordinate bug) traps instead of hanging the GPU
-  for (unsigned spin = 0;; spin++) {
-    unsigned done;
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n"
-        "selp.u32 %0, 1, 0, p;\n"
-        "}\n"
-        : "=r"(done)
-        : "r"(bar), "r"(parity)
-        : "memory");
-    if (done) break;
-    if (spin > (1u << 22)) __trap();
-  }
-}
-__device__ __forceinline__ void tma_load_3d(unsigned dst, const void *tmap, int c0, int c1, int c2, unsigned bar) {
-  asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];" ::"r"(dst),
-               "l"(tmap), "r"(c0), "r"(c1), "r"(c2), "r"(bar)
-               : "memory");
-}
-// Staging set-up of a search kernel: one mbarrier per warp-CTA, phase word next to it.
-template <typename T, int W>
-__device__ __forceinline__ void far_stage_init(Search<T> &S, unsigned char *smem_raw, int ax, int ay) {
-  S.ax = ax;
-  S.ay = ay;
-  S.farbuf = (unsigned)__cvta_generic_to_shared(smem_raw + SearchSmem<T, W>::FAR);
-  S.mbar = (unsigned)__cvta_generic_to_shared(smem_raw + SearchSmem<T, W>::MBAR);
-  if (lane_id() == 0) {
-    mbar_init(S.mbar, 1);
-    sts_u32(S.mbar + 8, 0);
-  }
-  __syncwarp();
-}
 template <typename T, int W, bool SKIP>
 __device__ __forceinline__ unsigned sad_partial_win(unsigned win_origin /* shared addr of MV (0,0), row 0 */,
                                                     int wpitch, int r, int c, int row,
@@ -446,9 +358,10 @@ __device__ __forceinline__ unsigned sad_partial_win(unsigned win_origin /* share
   if (sizeof(T) == 1) {
 #pragma unroll
     for (int j = 0; j < L::NW; j++) s = __vsadu4(__funnelshift_r(w[j], w[j + 1], sh), sw[j]) + s;
-  } else if (TF_SAD_IDP) {
+  } else {
     // |a - b| = a + b - 2 min(a, b): the sum of the source row (sa) is known, the candidate's sum and the sum of
     // the minima come from IDP.2A on the FMA pipe -- one VIMNMX on the ALU pipe per word instead of two plus the add
+    // (the ALU pipe is the busier one: 54% in the 16x16 search, the FMA pipe 16%; 4K 10-bit 62.5 -> 63.4 frames/s)
     unsigned accb = 0, accm = 0;
 #pragma unroll
     for (int j = 0; j < L::NW; j++) {
@@ -457,14 +370,6 @@ __device__ __forceinline__ unsigned sad_partial_win(unsigned win_origin /* share
       accm = __dp2a_lo(__vminu2(x, sw[j]), 0x0101u, accm);
     }
     s = sa + accb - 2 * accm;
-  } else {
-    unsigned acc = 0;
-#pragma unroll
-    for (int j = 0; j < L::NW; j++) {
-      const unsigned x = __funnelshift_r(w[j], w[j + 1], sh);
-      acc += __vmaxu2(x, sw[j]) - __vminu2(x, sw[j]);
-    }
-    s = (acc & 0xffffu) + (acc >> 16);
   }
   return s;
 }
@@ -567,8 +472,7 @@ __device__ __forceinline__ unsigned far_partial_off(const unsigned char *lane_ba
     w0[it] = __ldg(wp + it * step_words);
     w1[it] = __ldg(wp + it * step_words + 1);
   }
-  unsigned s = 0;
-  if (sizeof(T) != 1 && TF_SAD_IDP) {
+  if (sizeof(T) != 1) {  // a + b - 2 min(a, b), as in sad_partial_win
     unsigned accb = 0, accm = 0;
 #pragma unroll
     for (int it = 0; it < F::IT; it++) {
@@ -578,38 +482,9 @@ __device__ __forceinline__ unsigned far_partial_off(const unsigned char *lane_ba
     }
     return sa + accb - 2 * accm;
   }
-#pragma unroll
-  for (int it = 0; it < F::IT; it++) {
-    const unsigned x = __funnelshift_r(w0[it], w1[it], sh);
-    if (sizeof(T) == 1) s = __vsadu4(x, sf[it]) + s;
-    else s += __vmaxu2(x, sf[it]) - __vminu2(x, sf[it]);
-  }
-  if (sizeof(T) != 1) s = (s & 0xffffu) + (s >> 16);
-  return s;
-}
-
-// SAD of a staged candidate against the source block in the far (row-major) lane layout; dxb = byte offset of
-// the candidate's first sample inside a staged row (0 .. 15).
-template <typename T, int W, bool SKIP>
-__device__ __forceinline__ unsigned far_partial_smem(unsigned cand, int dxb, int lane, const uint32_t (&sf)[FarL<T, W, SKIP>::IT]) {
-  using F = FarL<T, W, SKIP>;
-  constexpr int ROWB = SearchSmem<T, W>::FAR_ROWB;
-  const unsigned a = cand + (unsigned)((lane / F::NW) * ROWB + (lane % F::NW) * 4 + (dxb & ~3));
-  const unsigned sh = (unsigned)(dxb & 3) * 8;
-  uint32_t w0[F::IT], w1[F::IT];
-#pragma unroll
-  for (int it = 0; it < F::IT; it++) {
-    w0[it] = lds_u32(a + (unsigned)(it * F::RPI * ROWB));
-    w1[it] = lds_u32(a + (unsigned)(it * F::RPI * ROWB + 4));
-  }
   unsigned s = 0;
 #pragma unroll
-  for (int it = 0; it < F::IT; it++) {
-    const unsigned x = __funnelshift_r(w0[it], w1[it], sh);
-    if (sizeof(T) == 1) s = __vsadu4(x, sf[it]) + s;
-    else s += __vmaxu2(x, sf[it]) - __vminu2(x, sf[it]);
-  }
-  if (sizeof(T) != 1) s = (s & 0xffffu) + (s >> 16);
+  for (int it = 0; it < F::IT; it++) s = __vsadu4(__funnelshift_r(w0[it], w1[it], sh), sf[it]) + s;
   return s;
 }
 
@@ -658,16 +533,9 @@ __device__ __forceinline__ unsigned bilinear_err(const Search<T> &S_in, int r8, 
 // shared-memory window whenever the MV lies inside it instead of from global memory.
 template <typename T, int W>
 __device__ __forceinline__ int var_cost(const Search<T> &S, int r, int c) {
-  if constexpr (VAR_VIA_SUBPEL_ROUTINE) {
-    // vf(src, ref): the difference is src - ref, and the high-bitdepth rounding of the sum
-    // (ROUND_POWER_OF_TWO of a signed value) is not symmetric under negation -> mode 3
-    return (int)bilinear_err<T, W>(S, r * 8, c * 8, 3) + sse_cost(S, r * 8, c * 8);
-  } else {
-    unsigned sse;
-    const int v = (int)variance<T, W>(S.src, S.stride, S.ref + r * S.stride + c, S.stride, S.hbd_shift, &sse);
-    if (S.ctr && lane_id() == 0) atomicAdd(&S.ctr[2], (unsigned long long)(W * W));
-    return v + sse_cost(S, r * 8, c * 8);
-  }
+  // vf(src, ref): the difference is src - ref, and the high-bitdepth rounding of the sum
+  // (ROUND_POWER_OF_TWO of a signed value) is not symmetric under negation -> mode 3
+  return (int)bilinear_err<T, W>(S, r * 8, c * 8, 3) + sse_cost(S, r * 8, c * 8);
 }
 
 // ---------------------------------------------------------------------------
@@ -682,7 +550,7 @@ __device__ __forceinline__ int var_cost(const Search<T> &S, int r, int c) {
 // over keys (total << 4 | site index): bit-exact, and without any sequential
 // per-candidate code.
 // ---------------------------------------------------------------------------
-template <typename T, int W, bool SKIP, bool TMAF>
+template <typename T, int W, bool SKIP>
 __device__ __forceinline__ unsigned diamond_search(const Search<T> &S_in, MV2 start, int search_step, int *num00,
                                                 MV2 *best_out) {
   using L = SadL<T, W, SKIP>;
@@ -695,8 +563,8 @@ __device__ __forceinline__ unsigned diamond_search(const Search<T> &S_in, MV2 st
   sad_load_src<T, W, SKIP>(S.src, S.stride, sw);
   uint32_t sf[FarL<T, W, SKIP>::IT];
   far_load_src<T, W, SKIP>(S.src, S.stride, lane, sf);
-  unsigned sa_near = 0, sa_far = 0;  // sums of this lane's source samples in the two layouts (TF_SAD_IDP)
-  if (sizeof(T) != 1 && TF_SAD_IDP) {
+  unsigned sa_near = 0, sa_far = 0;  // sums of this lane's source samples in the two layouts (16-bit SAD)
+  if (sizeof(T) != 1) {
 #pragma unroll
     for (int j = 0; j < L::NW; j++) sa_near = __dp2a_lo(sw[j], 0x0101u, sa_near);
 #pragma unroll
@@ -778,63 +646,6 @@ __device__ __forceinline__ unsigned diamond_search(const Search<T> &S_in, MV2 st
       // incumbent of a predicted start, few candidates die early, and the second dependent load round trip
       // lengthens the chain: 45.9 vs 51.0 frames/s.)
       ncand += __popc(okmask);
-      if constexpr (SKIP && TMAF) {
-        // TMA staging: one lane issues a box copy per live site (the descriptor views the plane as (x, row
-        // parity, row / 2), so a box of one parity is the candidate's even rows; it starts at the 16-byte aligned
-        // column at or below the candidate's, the only start the copy engine accepts); the copies of a batch are
-        // all in flight before anything is evaluated, bypass the L1 load path the per-lane global loads of this
-        // stage saturate, and complete on the warp's mbarrier.
-        using SM = SearchSmem<T, W>;
-        const int cx = S.ax + sc, cy = S.ay + sr;  // the candidate's first sample in allocation coordinates
-        unsigned phase = lds_u32(S.mbar + 8);
-#pragma unroll 1
-        for (unsigned m = okmask; m != 0;) {
-          unsigned batch = 0;
-          int nb = 0;
-#pragma unroll 1
-          for (; m != 0 && nb < SM::FAR_SLOTS; nb++) {
-            batch |= m & (0u - m);
-            m &= m - 1;
-          }
-          if (lane == 0) mbar_expect_tx(S.mbar, (unsigned)(nb * SM::FAR_CAND));
-          {
-            unsigned dst = S.farbuf;
-#pragma unroll 1
-            for (unsigned b = batch; b != 0; b &= b - 1, dst += SM::FAR_CAND) {
-              const int i = __ffs(b) - 1;
-              const int x = __shfl_sync(FULL, cx, i), y = __shfl_sync(FULL, cy, i);
-              if (lane == 0) tma_load_3d(dst, S.tmap, x & ~(SM::FAR_PAD - 1), y & 1, y >> 1, S.mbar);
-            }
-          }
-          mbar_wait(S.mbar, phase);
-          phase ^= 1u;
-          unsigned cand = S.farbuf;
-#pragma unroll 1
-          for (unsigned b = batch; b != 0;) {
-            int si[4];
-            unsigned part[4];
-#pragma unroll
-            for (int u = 0; u < 4; u++) {
-              si[u] = b ? __ffs(b) - 1 : -1;
-              b &= b - 1;
-            }
-#pragma unroll
-            for (int u = 0; u < 4; u++) {
-              const int dxb = (__shfl_sync(FULL, cx, si[u] & 31) & (SM::FAR_PAD - 1)) * (int)sizeof(T);
-              part[u] = si[u] >= 0 ? far_partial_smem<T, W, SKIP>(cand + (unsigned)(u * SM::FAR_CAND), dxb, lane, sf) : 0u;
-            }
-            cand += 4 * SM::FAR_CAND;
-            const unsigned tot4 = reduce4_u32(part, lane);
-            const int ms = (lane & 16) ? ((lane & 8) ? si[3] : si[2]) : ((lane & 8) ? si[1] : si[0]);
-            const unsigned my_cost = __shfl_sync(FULL, scost, ms & 31);
-            const unsigned tot = sad_post<SKIP>(tot4, S.hbd_shift) + my_cost;
-            mykey = min(mykey, ms >= 0 ? ((tot << 4) | (unsigned)(ms + 1)) : 0xffffffffu);
-          }
-          __syncwarp();  // every lane has read the batch before the next one overwrites the buffer
-        }
-        if (lane == 0) sts_u32(S.mbar + 8, phase);
-        __syncwarp();
-      } else
 #pragma unroll 1
       for (int i0 = 0; i0 < nsites; i0 += 4) {
         if (((okmask >> i0) & 15u) == 0) continue;
@@ -881,7 +692,7 @@ __device__ __forceinline__ unsigned diamond_search(const Search<T> &S_in, MV2 st
 }
 
 // full_pixel_diamond (mcomp.c:1421-1470), cost_list == NULL
-template <typename T, int W, bool SKIP, bool TMAF>
+template <typename T, int W, bool SKIP>
 __device__ int full_pixel_diamond(const Search<T> &S, MV2 start, int step_param, MV2 *best_mv) {
   int n = 0, num00 = 0;
   int bestsme = 0;
@@ -900,7 +711,7 @@ __device__ int full_pixel_diamond(const Search<T> &S, MV2 start, int step_param,
     }
     MV2 tmp;
     int nn;
-    int thissme = (int)diamond_search<T, W, SKIP, TMAF>(S, start, step_param + (first ? 0 : n), &nn, &tmp);
+    int thissme = (int)diamond_search<T, W, SKIP>(S, start, step_param + (first ? 0 : n), &nn, &tmp);
     if (thissme < INT_MAX_) {
       // var_cost is a pure function of the MV: passes that end on an MV already scored reuse the value
       if (!first && tmp.row == best_mv->row && tmp.col == best_mv->col) thissme = bestsme;
@@ -1035,11 +846,11 @@ __device__ int full_pixel_exhaustive(Search<T> &S, const KParams &P, MV2 start, 
 // av1_full_pixel_search (mcomp.c:1693-1832), NSTEP, run_mesh_search = 1.
 // Returns 1 when the skip-row result must be discarded and the search redone
 // with full SAD (mcomp.c:1777-1810).
-template <typename T, int W, bool SKIP, bool TMAF>
+template <typename T, int W, bool SKIP>
 __device__ __forceinline__ int full_pixel_search_pass(Search<T> &S, const KParams &P, MV2 start, MV2 *best_mv,
                                                    unsigned char *winbuf) {
   int run_mesh = 1;
-  int var = full_pixel_diamond<T, W, SKIP, TMAF>(S, start, P.step_param, best_mv);
+  int var = full_pixel_diamond<T, W, SKIP>(S, start, P.step_param, best_mv);
   int prune = 0, thr = 4;
   if (P.prune_level == 2) prune = 1;
   if (P.prune_level == 1) {
@@ -1079,7 +890,7 @@ __device__ __forceinline__ int full_pixel_search_pass(Search<T> &S, const KParam
   return 0;
 }
 
-template <typename T, int W, bool TMAF>
+template <typename T, int W>
 __device__ void full_pixel_search(Search<T> &S, const KParams &P, MV2 start, MV2 *best_mv, unsigned char *winbuf) {
   const int wr = iclamp(start.row, S.lim.row_min, S.lim.row_max);
   const int wc = iclamp(start.col, S.lim.col_min, S.lim.col_max);
@@ -1088,13 +899,13 @@ __device__ void full_pixel_search(Search<T> &S, const KParams &P, MV2 start, MV2
   // best_mv, normally inside the window); SUBPEL_TREE reuses the buffer as 8-tap scratch instead.
   const bool keep = P.subpel_method != 0;
   if (P.use_skip) {
-    if (!full_pixel_search_pass<T, W, true, TMAF>(S, P, start, best_mv, winbuf)) {
+    if (!full_pixel_search_pass<T, W, true>(S, P, start, best_mv, winbuf)) {
       if (!keep) S.win = nullptr;
       return;
     }
     if (S.wr != wr || S.wc != wc) window_load<T, W>(S, winbuf, wr, wc);
   }
-  full_pixel_search_pass<T, W, false, false>(S, P, start, best_mv, winbuf);
+  full_pixel_search_pass<T, W, false>(S, P, start, best_mv, winbuf);
   if (!keep) S.win = nullptr;
 }
 
@@ -1570,9 +1381,6 @@ __device__ __forceinline__ void search_init(Search<T> &S, const KParams &P, int 
   S.is_hbd = P.is_hbd;
   S.win = nullptr;
   S.srcs = 0;
-  S.ax = S.ay = 0;
-  S.tmap = nullptr;
-  S.farbuf = S.mbar = 0;
   S.wr = S.wc = S.wR = S.wpitch = S.wshift = 0;
   S.ctr = P.ctr;
   // av1_set_mv_{row,col}_limits (mcomp.h:216-240) + av1_set_mv_search_range (mcomp.c:196-215)
@@ -1621,8 +1429,6 @@ __device__ __forceinline__ void search32_block(const KParams &P, const unsigned 
   search_init(S, P, mb_row, mb_col);
   S.src = cur + y_offset;
   src_tile_load<T, 32>(S, smem_raw + SearchSmem<T, 32>::WIN);  // once per block: the same source for every frame
-  constexpr bool TMAF = TF_FAR_TMA && MINB == S32_WARPS_LO;  // the denser builds have no shared memory to spare
-  if constexpr (TMAF) far_stage_init<T, 32>(S, smem_raw, P.abx + mb_col * 32, P.aby + mb_row * 32);
   // ref_mv chain (temporal_filter.c:855-871): carried in global memory across launches
   MV2 ref_mv = { 0, 0 };
   if (P.frame_begin > 0) {
@@ -1636,10 +1442,9 @@ __device__ __forceinline__ void search32_block(const KParams &P, const unsigned 
       continue;
     }
     S.ref = reinterpret_cast<const T *>(P.frm[frame][0]) + y_offset;
-    S.tmap = reinterpret_cast<const unsigned char *>(P.tmap[frame]) + 128;  // the 32x32 box descriptor
     const MV2 start = { rawpel(ref_mv.row), rawpel(ref_mv.col) };
     MV2 best_full;
-    full_pixel_search<T, 32, TMAF>(S, P, start, &best_full, smem_raw);
+    full_pixel_search<T, 32>(S, P, start, &best_full, smem_raw);
     int block_mse;
     MV2 block_mv;
     if (P.force_integer_mv == 1) {
@@ -1700,13 +1505,10 @@ __device__ __forceinline__ void search16_task(const KParams &P, const int task) 
   S.src = reinterpret_cast<const T *>(P.frm[P.filter_idx][0]) + off;
   S.ref = reinterpret_cast<const T *>(P.frm[frame][0]) + off;
   src_tile_load<T, 16>(S, smem_raw + SearchSmem<T, 16>::WIN);
-  if constexpr (TF_FAR_TMA != 0)
-    far_stage_init<T, 16>(S, smem_raw, P.abx + mb_col * 32 + (sub & 1) * 16, P.aby + mb_row * 32 + (sub >> 1) * 16);
-  S.tmap = P.tmap[frame];  // the 16x16 box descriptor
   const size_t bf = (size_t)blk * P.num_frames + frame;
   const MV2 start = { rawpel((int)P.s_blk_mv[bf * 2 + 0]), rawpel((int)P.s_blk_mv[bf * 2 + 1]) };
   MV2 best_full, best;
-  full_pixel_search<T, 16, TF_FAR_TMA != 0>(S, P, start, &best_full, smem_raw);
+  full_pixel_search<T, 16>(S, P, start, &best_full, smem_raw);
   const unsigned err = subpel_search<T, 16>(S, P, best_full, &best, reinterpret_cast<T *>(smem_raw));
   if (lane == 0) {
     P.s_sub_mv[(bf * 4 + sub) * 2 + 0] = (int16_t)best.row;
@@ -1738,12 +1540,11 @@ struct SearchResult {
 };
 // The per-item part of the batched searches: MV limits for a W x W block at mi position (y / 4, x / 4),
 // av1_set_mv_{row,col}_limits (mcomp.h:216-240), then av1_set_mv_search_range (mcomp.c:196-215) around a zero
-// reference MV; then av1_full_pixel_search from `start` with `ref` as the reference (tmap: its TMA descriptors).
+// reference MV; then av1_full_pixel_search from `start` with `ref` as the reference.
 // Leaves S set up for the item (source, reference, limits, search window) for what follows.
 template <typename T, int W>
 __device__ __forceinline__ void item_full_pixel_search(Search<T> &S, const KParams &P, const T *src, const T *ref,
-                                                       const void *tmap, int x, int y, MV2 start, MV2 *best,
-                                                       unsigned char *smem_raw) {
+                                                       int x, int y, MV2 start, MV2 *best, unsigned char *smem_raw) {
   search_init(S, P, 0, 0);
   const int border = P.border, mi_row = y >> 2, mi_col = x >> 2, mih = W / 4;
   S.lim.row_min = imax(-(mi_row * 4 + border - 8), -(((mi_row + mih) * 4) + 8));
@@ -1757,9 +1558,7 @@ __device__ __forceinline__ void item_full_pixel_search(Search<T> &S, const KPara
   const int off = y * P.pitch[0] + x;
   S.src = src + off;
   S.ref = ref + off;
-  if constexpr (TF_FAR_TMA != 0) far_stage_init<T, W>(S, smem_raw, P.abx + x, P.aby + y);
-  S.tmap = reinterpret_cast<const unsigned char *>(tmap) + (W == 32 ? 128 : 0);
-  full_pixel_search<T, W, TF_FAR_TMA != 0>(S, P, start, best, smem_raw);
+  full_pixel_search<T, W>(S, P, start, best, smem_raw);
 }
 template <typename T, int W>
 __global__ void __launch_bounds__(32, W == 32 ? S32_WARPS_LO : 24)
@@ -1772,7 +1571,7 @@ __global__ void __launch_bounds__(32, W == 32 ? S32_WARPS_LO : 24)
   Search<T> S;
   const MV2 start = { (int)it.start_row, (int)it.start_col };
   MV2 best;
-  item_full_pixel_search<T, W>(S, P, src, ref, P.tmap[1], it.x, it.y, start, &best, smem_raw);
+  item_full_pixel_search<T, W>(S, P, src, ref, it.x, it.y, start, &best, smem_raw);
   const int var = var_cost<T, W>(S, best.row, best.col);
   if (lane == 0) {
     results[blockIdx.x].row = (int16_t)best.row;
@@ -1824,7 +1623,7 @@ __global__ void __launch_bounds__(32, W == 32 ? S32_WARPS_LO : 24)
   const MV2 start = { (int)it.start_row, (int)it.start_col };
   MV2 best_full;
   item_full_pixel_search<T, W>(S, P, reinterpret_cast<const T *>(P.frm[0][0]), reinterpret_cast<const T *>(P.frm[f][0]),
-                               P.tmap[f], it.x, it.y, start, &best_full, smem_raw);
+                               it.x, it.y, start, &best_full, smem_raw);
   const int var = var_cost<T, W>(S, best_full.row, best_full.col);
   src_tile_load<T, W>(S, smem_raw + SearchSmem<T, W>::WIN);
   MV2 mv;
@@ -1928,9 +1727,6 @@ __device__ __noinline__ void convolve12(const KParams &P, const T *src, int ss, 
 //     shared-memory words, 12 IDP.2A;
 //   vertical-only positions copy the rows transposed and use the same vertical stage.
 // Rounding and offsets are those of convolve12 above, term for term.
-#ifndef TF_CONVOLVE_PACKED
-#define TF_CONVOLVE_PACKED 1
-#endif
 __device__ __forceinline__ unsigned pack_taps(const int16_t *f, int k) {
   return ((unsigned)f[k] & 0xffu) | (((unsigned)f[k + 1] & 0xffu) << 8);
 }
@@ -2057,7 +1853,7 @@ __device__ void build_predictor(const KParams &P, const T *const ref[3], int mb_
     pos_x = iclamp(pos_x, left, (P.aligned_w[k] + 4) << 10);
     const T *src = ref[plane] + (pos_y >> 10) * P.pitch[k] + (pos_x >> 10);
     const int sxp = (pos_x & 1023) >> 6, syp = (pos_y & 1023) >> 6;
-    if constexpr (TF_CONVOLVE_PACKED && sizeof(T) == 2) {
+    if constexpr (sizeof(T) == 2) {
       if (sxp | syp) convolve12_packed(P, src, P.pitch[k], &pred[plane_offset + i * plane_w + j], plane_w, w, h, sxp, syp, im);
       else convolve12<T>(P, src, P.pitch[k], &pred[plane_offset + i * plane_w + j], plane_w, w, h, 0, 0, im);
     } else {
@@ -2077,7 +1873,7 @@ __device__ void build_predictor(const KParams &P, const T *const ref[3], int mb_
 // j = tid % w and rows r0 + k * (NT / w).  The lanes of a row are adjacent lanes of one warp (w = 32:
 // the warp, w = 16: a half warp), so the horizontal 5-sum with edge clamp (:463-493 window, clamped as
 // the reference clamps the coordinates) is four shuffles, the vertical one five conflict-free shared
-// loads of a column, and the co-located luma sums of the chroma planes stay in registers.
+// loads of a column; the chroma planes add the co-located luma squares from lsum.
 //
 // The weight (int)(exp(-scaled_error) * 1000) (:691-693) is computed in fp64 with the reference's
 // operation order.  (An fp32 ex2.approx fast path with an exact fp64 fallback near integer boundaries was
@@ -2094,8 +1890,6 @@ __device__ void apply_filter(const KParams &P, const T *curb, int mb_row, int mb
                              uint32_t *lsum, const double *terms /* shared: d_factor[4], block_error * inv_factor [4] */) {
   constexpr int NT = FILT_THREADS;
   constexpr int MAXPX = 1024 / NT;  // pixels of one plane per thread
-  constexpr int WUNROLL = TF_FILT_WUNROLL > 0 ? TF_FILT_WUNROLL : 1;
-  (void)WUNROLL;
   const int tid = threadIdx.x, lane = tid & 31;
   const double inv_factor = 1.0 / ((5 + 1) * 20);
   const double weight_factor = (double)5 * inv_factor;
@@ -2104,7 +1898,6 @@ __device__ void apply_filter(const KParams &P, const T *curb, int mb_row, int mb
   (void)inv_factor;
   (void)mb_row;
   (void)mb_col;
-  uint32_t lsub[MAXPX];  // chroma: sums of the co-located luma squares of this thread's pixels
   int plane_offset = 0;
   for (int plane = 0; plane < P.num_planes; plane++) {
     const int ssy = plane ? P.ss_y : 0, ssx = plane ? P.ss_x : 0;
@@ -2118,18 +1911,6 @@ __device__ void apply_filter(const KParams &P, const T *curb, int mb_row, int mb
     const int seg = lane & ~(w - 1);
     const int l_m2 = seg + imax(j - 2, 0), l_m1 = seg + imax(j - 1, 0);
     const int l_p1 = seg + imin(j + 1, w - 1), l_p2 = seg + imin(j + 2, w - 1);
-    if (TF_FILT_WUNROLL == 0 && plane == 1) {  // compute_luma_sq_error_sum (:507-522); lsum holds the raw luma squares
-#pragma unroll
-      for (int k = 0; k < MAXPX; k++) {
-        if (k < npass) {
-          const int i = r0 + k * rpp;
-          uint32_t s = 0;
-          for (int ii = 0; ii < (1 << ssy); ii++)
-            for (int jj = 0; jj < (1 << ssx); jj++) s += lsum[((i << ssy) + ii) * 32 + (j << ssx) + jj];
-          lsub[k] = s;
-        }
-      }
-    }
     // compute_square_diff (:463-493) + horizontal 5-sums
 #pragma unroll
     for (int k = 0; k < MAXPX; k++) {
@@ -2149,25 +1930,19 @@ __device__ void apply_filter(const KParams &P, const T *curb, int mb_row, int mb
     // a thread's pixels lie in one column half, i.e. in two sub-blocks: the upper and the lower one
     const double d_factor[2] = { terms[sb_col], terms[2 + sb_col] };
     const double b_term[2] = { terms[4 + sb_col], terms[6 + sb_col] };
-#if TF_FILT_WUNROLL == 0
-#pragma unroll
-#else
-#pragma unroll(WUNROLL)
-#endif
+    // Not unrolled: the filter kernel shrinks from 64 to 40 KB of code (its instruction-cache request rate was 89% of
+    // peak) and loses its spills: 2.85 -> 2.65 ms at 4K 10-bit.
+#pragma unroll 1
     for (int k = 0; k < MAXPX; k++) {
       if (k < npass) {
         const int i = r0 + k * rpp, idx = tid + k * NT;
         // 25 (+4) squares of at most 4095^2: fits 32 bits
         uint32_t sum_square_diff = sq[imax(i - 2, 0) * w + j] + sq[imax(i - 1, 0) * w + j] + sq[idx] +
                                    sq[imin(i + 1, h - 1) * w + j] + sq[imin(i + 2, h - 1) * w + j];
-#if TF_FILT_WUNROLL == 0
-        if (plane) sum_square_diff += lsub[k];
-#else
-        if (plane) {  // compute_luma_sq_error_sum (:507-522) on the fly: the loop is not fully unrolled
+        if (plane) {  // compute_luma_sq_error_sum (:507-522) on the fly
           for (int ii = 0; ii < (1 << ssy); ii++)
             for (int jj = 0; jj < (1 << ssx); jj++) sum_square_diff += lsum[((i << ssy) + ii) * 32 + (j << ssx) + jj];
         }
-#endif
         sum_square_diff >>= hbd_sh;
         const double window_error = __dmul_rn((double)sum_square_diff, inv_num_ref_pixels);
         const int sb = (i >= h / 2);  // rows ascend with k: the first half of the passes is the upper sub-block

@@ -1,5 +1,5 @@
 """Latency of one block-row slab of one 4K 10-bit window on one GPU (what a rank of the slab mode computes),
-for 1/1, 1/2, 1/4, 1/8 of the rows.  TF_GPU_CHAIN=frames|fused selects the chain structure (default: auto)."""
+for 1/1, 1/2, 1/4, 1/8 of the rows, for the library in TF_GPU_LIB (or the in-tree build)."""
 import os, sys, time
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
@@ -28,4 +28,4 @@ for parts in (1, 2, 4, 8):
     for _ in range(K): ctx.filter_resident(pp, ids)
     ctx.event_record(3)
     out[parts] = round(ctx.event_elapsed_ms(2, 3) / K, 3)
-print(os.environ.get("TF_GPU_CHAIN"), out, {k: round(out[1] / v / k, 3) for k, v in out.items()})
+print(os.environ.get("TF_GPU_LIB", "cur"), out, {k: round(out[1] / v / k, 3) for k, v in out.items()})
