@@ -44,7 +44,11 @@ struct DevFrame {
   Geometry g;
   void *base[3] = { nullptr, nullptr, nullptr };  // allocation base
   void *p00[3] = { nullptr, nullptr, nullptr };   // pixel (0,0)
-  cudaEvent_t ready = nullptr;                    // upload + border extension finished (copy stream)
+  // cache slots only: luma row sums R16(i, j) = sum of Y(i, j + t), t < 16, with the luma pitch, for the lower bound
+  // of the 16x16 search (rowsum16_kernel)
+  uint16_t *rs_base = nullptr;
+  uint16_t *rs00 = nullptr;  // at pixel (0,0)
+  cudaEvent_t ready = nullptr;                    // upload + border extension + row sums finished (copy stream)
 };
 
 // Timing events of one filter call (main stream): start, after the search32 chain, after the
@@ -240,13 +244,16 @@ int check_device_extent(tf_gpu_ctx *ctx, const void *ptr, size_t bytes, size_t a
   }
   return TF_GPU_OK;
 }
-int alloc_dev_frame(tf_gpu_ctx *ctx, DevFrame *d, const Geometry &g) {
+// `rowsum`: the slot also gets the luma row-sum plane (frame cache slots; output frames do not).
+int alloc_dev_frame(tf_gpu_ctx *ctx, DevFrame *d, const Geometry &g, bool rowsum = false) {
   const size_t es = g.is_hbd ? 2 : 1;
-  if (d->base[0] && d->g == g) return TF_GPU_OK;
+  if (d->base[0] && d->g == g && (!rowsum || d->rs_base)) return TF_GPU_OK;
   for (int p = 0; p < 3; p++) {
     if (d->base[p]) cudaFree(d->base[p]);
     d->base[p] = d->p00[p] = nullptr;
   }
+  if (d->rs_base) cudaFree(d->rs_base);
+  d->rs_base = d->rs00 = nullptr;
   d->g = g;
   d->valid = false;
   for (int p = 0; p < g.num_planes; p++) {
@@ -255,7 +262,26 @@ int alloc_dev_frame(tf_gpu_ctx *ctx, DevFrame *d, const Geometry &g) {
     CU(cudaMalloc(&d->base[p], bytes));
     d->p00[p] = (char *)d->base[p] + ((size_t)g.by[k] * g.pitch[k] + g.bx[k]) * es;
   }
+  if (rowsum) {
+    CU(cudaMalloc(&d->rs_base, (size_t)g.rows[0] * g.pitch[0] * sizeof(uint16_t)));
+    d->rs00 = d->rs_base + (size_t)g.by[0] * g.pitch[0] + g.bx[0];
+  }
   return TF_GPU_OK;
+}
+
+// Row sums of a freshly filled slot's luma plane, on the copy stream before the slot's `ready` event: every column
+// j of [-bx, aligned_w + bx - 16] and every row of [-by, aligned_h + by), the region a 16x16 candidate inside the
+// MV limits can reach.  Part of filling the luma plane: last_launches keeps counting one launch per plane.
+void launch_rowsum(tf_gpu_ctx *ctx, DevFrame *d) {
+  const Geometry &g = d->g;
+  const int w = g.aligned_w[0] + 2 * g.bx[0] - 15, h = g.aligned_h[0] + 2 * g.by[0];
+  const dim3 grid((w + 16 * ROWSUM_THREADS - 1) / (16 * ROWSUM_THREADS), h);
+  if (g.is_hbd)
+    rowsum16_kernel<uint16_t><<<grid, ROWSUM_THREADS, 0, ctx->copy_stream>>>((const uint16_t *)d->p00[0], g.pitch[0],
+                                                                             d->rs00, g.bx[0], g.by[0], w);
+  else
+    rowsum16_kernel<uint8_t><<<grid, ROWSUM_THREADS, 0, ctx->copy_stream>>>((const uint8_t *)d->p00[0], g.pitch[0],
+                                                                            d->rs00, g.bx[0], g.by[0], w);
 }
 
 // Upload the crop area of a host frame and rebuild the borders on the device.
@@ -281,6 +307,7 @@ int upload_frame(tf_gpu_ctx *ctx, DevFrame *d, const tf_gpu_frame *f) {
                                                                          ext_w, ext_h);
     ctx->last_launches++;
   }
+  launch_rowsum(ctx, d);
   CU(cudaGetLastError());
   CU(cudaEventRecord(d->ready, ctx->copy_stream));
   d->frame_id = f->frame_id;
@@ -310,6 +337,7 @@ int ingest_frame(tf_gpu_ctx *ctx, DevFrame *d, const tf_gpu_frame *f, cudaStream
           g.bx[k], g.by[k], ext_w, ext_h);
     ctx->last_launches++;
   }
+  launch_rowsum(ctx, d);
   CU(cudaGetLastError());
   CU(cudaEventRecord(d->ready, ctx->copy_stream));
   d->frame_id = f->frame_id;
@@ -360,7 +388,7 @@ int get_frame(tf_gpu_ctx *ctx, const tf_gpu_frame *f, int num_planes, DevFrame *
       }
     }
     if (!victim) return fail(ctx, TF_GPU_ERR_MEM, "frame cache too small for this window");
-    int rc = alloc_dev_frame(ctx, victim, g);
+    int rc = alloc_dev_frame(ctx, victim, g, true);
     if (rc) return rc;
     victim->valid = false;
     {
@@ -558,6 +586,7 @@ void window_kparams(const tf_gpu_ctx *ctx, const tf_gpu_params *p, DevFrame *con
   }
   for (int f = 0; f < p->num_frames; f++)
     for (int pl = 0; pl < p->num_planes; pl++) K.frm[f][pl] = frames[f]->p00[pl];
+  for (int f = 0; f < p->num_frames; f++) K.rs[f] = frames[f]->rs00;
   for (int k = 0; k < 2; k++) K.out_pitch[k] = out.g.pitch[k];
   for (int pl = 0; pl < p->num_planes; pl++) K.out[pl] = out.p00[pl];
   K.num_pels = 1024 + (p->num_planes > 1 ? 2 * (1024 >> (g.ss_x + g.ss_y)) : 0);
@@ -1059,6 +1088,7 @@ void tf_gpu_destroy(tf_gpu_ctx *ctx) {
   for (auto &d : ctx->cache) {
     for (int p = 0; p < 3; p++)
       if (d.base[p]) cudaFree(d.base[p]);
+    if (d.rs_base) cudaFree(d.rs_base);
     if (d.ready) cudaEventDestroy(d.ready);
   }
   for (int i = 0; i < 2; i++)
@@ -1191,18 +1221,20 @@ int tf_gpu_device_border(void) { return DEV_BORDER; }
 
 int tf_gpu_debug_read_plane(tf_gpu_ctx *ctx, uint64_t frame_id, int plane, void *dst, int dst_stride, int x0, int y0,
                             int w, int h) {
-  if (!ctx || !dst || plane < 0 || plane > 2 || w <= 0 || h <= 0) return TF_GPU_ERR_INVALID;
+  if (!ctx || !dst || plane < 0 || plane > TF_GPU_DEBUG_ROWSUM_PLANE || w <= 0 || h <= 0) return TF_GPU_ERR_INVALID;
   CU(cudaSetDevice(ctx->device));
   DevFrame *d = find_cached(ctx, frame_id, nullptr);
   if (!d) return fail(ctx, TF_GPU_ERR_INVALID, "frame id %llu is not resident", (unsigned long long)frame_id);
   const Geometry &g = d->g;
-  if (plane >= g.num_planes) return fail(ctx, TF_GPU_ERR_INVALID, "plane not present");
-  const int k = plane > 0;
-  const size_t es = g.is_hbd ? 2 : 1;
+  const bool rowsum = plane == TF_GPU_DEBUG_ROWSUM_PLANE;
+  if (!rowsum && plane >= g.num_planes) return fail(ctx, TF_GPU_ERR_INVALID, "plane not present");
+  const int k = !rowsum && plane > 0;
+  const size_t es = (rowsum || g.is_hbd) ? 2 : 1;
   if (x0 < -g.bx[k] || y0 < -g.by[k] || x0 + w > g.pitch[k] - g.bx[k] || y0 + h > g.rows[k] - g.by[k])
     return fail(ctx, TF_GPU_ERR_INVALID, "rectangle outside the device allocation");
   CU(cudaStreamSynchronize(ctx->copy_stream));
-  const char *src = (const char *)d->p00[plane] + ((long long)y0 * g.pitch[k] + x0) * (long long)es;
+  const void *p00 = rowsum ? (const void *)d->rs00 : d->p00[plane];
+  const char *src = (const char *)p00 + ((long long)y0 * g.pitch[k] + x0) * (long long)es;
   CU(cudaMemcpy2D(dst, (size_t)dst_stride * es, src, (size_t)g.pitch[k] * es, (size_t)w * es, h, cudaMemcpyDeviceToHost));
   return TF_GPU_OK;
 }

@@ -70,6 +70,7 @@ struct KParams {
   double dist_thr;  // max(min(w,h) * 0.1, 1)
   // planes (pointers to pixel (0,0)); pitch in samples
   const void *frm[MAXF][3];
+  const uint16_t *rs[MAXF];  // per frame: luma row sums at pixel (0,0), luma pitch (rowsum16_kernel); 16x16 search
   int pitch[2];
   void *out[3];
   int out_pitch[2];
@@ -154,8 +155,12 @@ struct Search {
   int wpitch;  // bytes; wpitch/4 is odd
   int wshift;  // bytes the window origin was aligned down by
   // optional executed-work counters (bench instrumentation; nullptr in normal runs):
-  // [0] SAD sample pairs read, [1] sub-pel candidate evaluations x block samples, [2] variance samples
+  // [0] SAD sample pairs read, [1] sub-pel candidate evaluations x block samples, [2] variance samples,
+  // [3] diamond sites skipped by the row-sum bound
   unsigned long long *ctr;
+  // Row sums of the reference (16x16 search only): rs[i * stride + j] = sum of ref[i * stride + j + t], t < 16.
+  // nullptr = no row-sum bound.
+  const uint16_t *rs;
 };
 
 constexpr int WIN_BYTES = 9472;  // window capacity per warp, 32x32 search
@@ -549,6 +554,16 @@ __device__ __forceinline__ int var_cost(const Search<T> &S, int r, int c) {
 // iff it beats the incumbent.  That is evaluated here as a warp min-reduction
 // over keys (total << 4 | site index): bit-exact, and without any sequential
 // per-candidate code.
+//
+// Row-sum bound (16x16 search, S.rs set): with S_k the sum of source row k and R_k(mv) the sum of the same W
+// reference samples at the candidate, sum_k |S_k - R_k(mv)| <= SAD(mv) over the rows k the SAD reads (triangle
+// inequality), and sad_post is monotone.  A site with sad_post(bound) + cost >= bestsad can therefore never be
+// accepted, nor be the stage's winning key (a winner beats the stage-start incumbent): it is skipped, exactly as
+// the cost pruning skips sites with cost >= bestsad.  The 16x16 search starts at the rounding of its 32x32 block's
+// MV, usually at or next to the match, so most later sites fall to the bound.  Applied to the far stages, where a
+// skipped site saves its L2 loads.  (Measured and rejected: screening the near stages too and packing their
+// surviving sites into the passes -- the row-sum loads cost more than the shared-memory passes they save: 4K
+// 10-bit 66.0 vs 69.2 frames/s.)
 // ---------------------------------------------------------------------------
 template <typename T, int W, bool SKIP>
 __device__ __forceinline__ unsigned diamond_search(const Search<T> &S_in, MV2 start, int search_step, int *num00,
@@ -570,6 +585,32 @@ __device__ __forceinline__ unsigned diamond_search(const Search<T> &S_in, MV2 st
 #pragma unroll
     for (int it = 0; it < FarL<T, W, SKIP>::IT; it++) sa_far = __dp2a_lo(sf[it], 0x0101u, sa_far);
   }
+  // the bound serves the skip-row SAD only: the full-row pass (small frames, or after a failed skip-row audit)
+  // runs without it
+  constexpr bool RSB = W == 16 && SKIP;
+  constexpr int NPK = RSB ? L::ROWS / 2 : 1;
+  const bool use_rs = RSB && S.rs != nullptr;
+  unsigned srow = sa_near;  // sum of this lane's source row: lanes 0 .. ROWS - 1 hold S_k of the SAD rows in order
+  if (RSB && sizeof(T) == 1) {
+#pragma unroll
+    for (int j = 0; j < L::NW; j++) srow = __vsadu4(sw[j], 0u) + srow;
+  }
+  uint32_t spk[NPK];  // S_k two per register, gathered per far stage (warp-uniform) rather than held: registers
+  auto rs_gather = [&]() {
+#pragma unroll
+    for (int j = 0; j < NPK; j++) spk[j] = __shfl_sync(FULL, srow, 2 * j) | (__shfl_sync(FULL, srow, 2 * j + 1) << 16);
+  };
+  // sad_post of the row-sum bound of the site (r, c) after rs_gather(); only for sites inside the MV limits
+  auto rs_bound = [&](int r, int c) -> unsigned {
+    const uint16_t *p = S.rs + r * S.stride + c;
+    const int step = L::RSTEP * S.stride;
+    unsigned b = 0;
+#pragma unroll
+    for (int j = 0; j < NPK; j++)
+      b = __vsadu2((unsigned)__ldg(p + 2 * j * step) | ((unsigned)__ldg(p + (2 * j + 1) * step) << 16), spk[j]) + b;
+    return sad_post<SKIP>(b, S.hbd_shift);
+  };
+  unsigned npruned = 0;  // sites skipped by the bound (instrumentation)
   // this lane's row / word position inside a far candidate (row-major layout)
   const unsigned char *far_base = reinterpret_cast<const unsigned char *>(
       S.ref + (lane / FarL<T, W, SKIP>::NW) * FarL<T, W, SKIP>::RSTEP * S.stride) + 4 * (lane % FarL<T, W, SKIP>::NW);
@@ -638,7 +679,13 @@ __device__ __forceinline__ unsigned diamond_search(const Search<T> &S_in, MV2 st
       const int sr = best.row + site_row(sidx), sc = best.col + site_col(sidx);
       const unsigned scost = (unsigned)sad_cost(S, sr, sc);
       // exact pruning: sad + cost < bestsad is impossible once cost >= bestsad
-      const bool sok = (lane < nsites) & (all_in | in_range(S.lim, sr, sc)) & (scost < bestsad);
+      bool sok = (lane < nsites) & (all_in | in_range(S.lim, sr, sc)) & (scost < bestsad);
+      if (use_rs) {
+        const unsigned cmask = __ballot_sync(FULL, sok);
+        rs_gather();
+        if (sok) sok = rs_bound(sr, sc) + scost < bestsad;
+        npruned += __popc(cmask & ~__ballot_sync(FULL, sok));
+      }
       const int soff = (sr * S.stride + sc) * (int)sizeof(T);
       const unsigned okmask = __ballot_sync(FULL, sok);
       // (Measured and rejected: reading a quarter of a far candidate's rows first and dropping it when that
@@ -685,7 +732,10 @@ __device__ __forceinline__ unsigned diamond_search(const Search<T> &S_in, MV2 st
       }
     }
   }
-  if (S.ctr && lane == 0) atomicAdd(&S.ctr[0], (unsigned long long)ncand * (L::ROWS * W));
+  if (S.ctr && lane == 0) {
+    atomicAdd(&S.ctr[0], (unsigned long long)ncand * (L::ROWS * W));
+    if (use_rs) atomicAdd(&S.ctr[3], (unsigned long long)npruned);
+  }
   *num00 = n00;
   *best_out = best;
   return bestsad;
@@ -1383,6 +1433,7 @@ __device__ __forceinline__ void search_init(Search<T> &S, const KParams &P, int 
   S.srcs = 0;
   S.wr = S.wc = S.wR = S.wpitch = S.wshift = 0;
   S.ctr = P.ctr;
+  S.rs = nullptr;
   // av1_set_mv_{row,col}_limits (mcomp.h:216-240) + av1_set_mv_search_range (mcomp.c:196-215)
   const int border = P.border, mi_row = mb_row * 8, mi_col = mb_col * 8;
   S.lim.row_min = imax(-(mi_row * 4 + border - 8), -(((mi_row + 8) * 4) + 8));
@@ -1504,6 +1555,7 @@ __device__ __forceinline__ void search16_task(const KParams &P, const int task) 
   search_init(S, P, mb_row, mb_col);
   S.src = reinterpret_cast<const T *>(P.frm[P.filter_idx][0]) + off;
   S.ref = reinterpret_cast<const T *>(P.frm[frame][0]) + off;
+  S.rs = P.rs[frame] + off;
   src_tile_load<T, 16>(S, smem_raw + SearchSmem<T, 16>::WIN);
   const size_t bf = (size_t)blk * P.num_frames + frame;
   const MV2 start = { rawpel((int)P.s_blk_mv[bf * 2 + 0]), rawpel((int)P.s_blk_mv[bf * 2 + 1]) };
@@ -2268,6 +2320,46 @@ __global__ void __launch_bounds__(INGEST_THREADS) ingest_plane_kernel(
       }
     }
     *(uint4 *)(dst + (long long)y * pitch + x0) = make_uint4(w[0], w[1], w[2], w[3]);
+  }
+}
+
+// ---------------------------------------------------------------------------
+// Row sums of a cached luma plane for the lower bound of the 16x16 search (diamond_search):
+// rs[y][x] = sum of plane[y][x + t], t < 16, for the row blockIdx.y - by and columns [-bx, w - bx).  16 * 4095 fits
+// uint16.  One thread per 16 consecutive columns, a running sum along them; with w = aligned_w + 2 bx - 15 every
+// stored sum covers columns the upload defines.
+// ---------------------------------------------------------------------------
+constexpr int ROWSUM_THREADS = 128;
+
+template <typename T>
+__global__ void __launch_bounds__(ROWSUM_THREADS) rowsum16_kernel(const T *__restrict__ p00, int pitch,
+                                                                  uint16_t *__restrict__ rs00, int bx, int by, int w) {
+  const int c0 = (blockIdx.x * ROWSUM_THREADS + threadIdx.x) * 16;  // counted from column -bx
+  if (c0 >= w) return;
+  const long long at = (long long)((int)blockIdx.y - by) * pitch - bx + c0;
+  // samples c0 .. c0 + 31 as 16-byte loads: slot rows start 128-sample aligned at column -bx.  The last group of a
+  // row may read up to 16 samples past the defined columns (pitch padding or the next row, inside the allocation:
+  // the slot has 2 slack rows); they only reach sums that are not stored.
+  constexpr int V = 16 / (int)sizeof(T);
+  T x[32];
+#pragma unroll
+  for (int q = 0; q < 32 / V; q++) *reinterpret_cast<uint4 *>(x + q * V) = __ldg(reinterpret_cast<const uint4 *>(p00 + at) + q);
+  unsigned s = 0;
+#pragma unroll
+  for (int t = 0; t < 16; t++) s += x[t];
+  uint32_t o[8];
+#pragma unroll
+  for (int i = 0; i < 16; i++) {
+    if (i > 0) s += (unsigned)x[i + 15] - (unsigned)x[i - 1];
+    if (i & 1) o[i >> 1] |= s << 16;
+    else o[i >> 1] = s;
+  }
+  uint16_t *dst = rs00 + at;
+  if (w - c0 >= 16) {
+    reinterpret_cast<uint4 *>(dst)[0] = make_uint4(o[0], o[1], o[2], o[3]);
+    reinterpret_cast<uint4 *>(dst)[1] = make_uint4(o[4], o[5], o[6], o[7]);
+  } else {
+    for (int i = 0; i < w - c0; i++) dst[i] = (uint16_t)(o[i >> 1] >> (16 * (i & 1)));
   }
 }
 

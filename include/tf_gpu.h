@@ -184,7 +184,11 @@ int tf_gpu_evict_frame(tf_gpu_ctx *ctx, uint64_t frame_id);
 /* Test hook for the upload path (av1_copy_and_extend_frame, extend.c:113-163): copies the rectangle
  * [x0, x0+w) x [y0, y0+h) of a cached device plane (coordinates relative to pixel (0,0); negative =
  * border) into dst (samples of the frame's container type, dst_stride in samples).  The rectangle
- * must lie inside the device allocation (tf_gpu_device_border() samples of luma border). */
+ * must lie inside the device allocation (tf_gpu_device_border() samples of luma border).
+ * plane TF_GPU_DEBUG_ROWSUM_PLANE reads the slot's luma row sums instead: uint16 values
+ * sum(Y(y, x + t), t < 16), defined for x in [-border, aligned_w + border - 16] and the rows of the
+ * extended luma plane; the 16x16 search bounds its candidates' SAD with them. */
+#define TF_GPU_DEBUG_ROWSUM_PLANE 3
 int tf_gpu_debug_read_plane(tf_gpu_ctx *ctx, uint64_t frame_id, int plane, void *dst, int dst_stride,
                             int x0, int y0, int w, int h);
 int tf_gpu_device_border(void);
