@@ -36,6 +36,7 @@ EXPORTS = [
     "tf_gpu_output_ipc_export", "tf_gpu_output_ipc_import", "tf_gpu_cache_frame_device",
     "tf_gpu_filter_batch_async", "tf_gpu_filter_batch_result", "tf_gpu_download_batch_output",
     "tf_gpu_batch_output_device_plane", "tf_gpu_motion_search_batch", "tf_gpu_motion_search_device",
+    "tf_gpu_predict_device",
 ]
 
 
@@ -102,6 +103,15 @@ assert _MOTION_RESULT_DTYPE.itemsize == C.sizeof(MotionResult) == 16
 TF_GPU_MOTION_REJECTED = -1  # fullpel_var of an item tf_gpu_motion_search_device rejected (tf_gpu.h)
 
 
+class PredictItem(C.Structure):
+    """tf_gpu_predict_item: one block of references[ref] predicted at MV (row, col), 1/8 pel.  The layout of
+    MotionItem, so pack_motion_items packs both."""
+    _fields_ = [("x", C.c_int), ("y", C.c_int), ("row", C.c_int16), ("col", C.c_int16), ("ref", C.c_int32)]
+
+
+assert C.sizeof(PredictItem) == C.sizeof(MotionItem)
+
+
 class Dump(C.Structure):
     _fields_ = [("subblock_mvs", C.c_void_p), ("subblock_mses", C.c_void_p), ("pred", C.c_void_p),
                 ("accum", C.c_void_p), ("count", C.c_void_p)]
@@ -143,6 +153,7 @@ def load_library():
     lib.tf_gpu_motion_search_batch.argtypes = [vp, C.POINTER(Params), u64, C.POINTER(u64), i, i,
                                                C.POINTER(MotionItem), i, C.POINTER(MotionResult)]
     lib.tf_gpu_motion_search_device.argtypes = [vp, C.POINTER(Params), u64, C.POINTER(u64), i, i, vp, i, vp, vp]
+    lib.tf_gpu_predict_device.argtypes = [vp, C.POINTER(Params), C.POINTER(u64), i, i, vp, i, vp, vp, vp]
     lib.tf_gpu_filter_resident.argtypes = [vp, C.POINTER(Params), C.POINTER(u64), C.POINTER(C.c_int64),
                                            C.POINTER(C.c_float)]
     lib.tf_gpu_download_output.argtypes = [vp, C.POINTER(Frame), i, i]
@@ -427,6 +438,15 @@ def motion_search_device_args(ref_ids, block_size, items, device):
     return (C.c_uint64 * len(ids))(*ids), len(ids), items.shape[0]
 
 
+def predict_device_args(ref_ids, block_size, items, device):
+    """Arguments of tf_gpu_predict_device that can be checked without reading the items (which would synchronise):
+    (uint64_t ref_ids[num_refs], num_refs, n).  items: an integer CUDA tensor of shape (n, 5) = x, y, row, col, ref
+    on `device`, the context's torch.device.  Raises ValueError, before anything reaches the library, as
+    motion_search_device_args does: for items that are not such a tensor, 0 or more than TF_GPU_MAX_FRAMES - 1
+    references, and a block size other than 16 or 32.  Positions and refs are checked per item by the kernel."""
+    return motion_search_device_args(ref_ids, block_size, items, device)
+
+
 def pack_motion_items(items):
     """(n, 5) integer tensor (x, y, start_row, start_col, ref) -> (n, 4) int32 tensor whose rows are
     tf_gpu_motion_item, by torch ops on the tensor's device (and current stream).  Values are converted as the C
@@ -691,6 +711,46 @@ class TemporalFilterGpu:
                                                              block_size, packed.data_ptr(), n, res.data_ptr(),
                                                              s.cuda_stream))
             return unpack_motion_results(res[:n])
+
+    def predict_tensors(self, params, ref_ids, block_size, items):
+        """The temporal filter's 12-tap predictor of many blocks of the resident frames ref_ids at caller MVs
+        (tf_gpu_predict_device; see tf_gpu.h for what a 16- or 32-item is and for the far-MV rule).  items: an
+        integer CUDA tensor (n, 5) = x, y, row, col (MV in 1/8 pel, taken as int16), ref on the context's device
+        (see predict_device_args).  Returns (planes, status): planes holds 1 or 3 CUDA tensors (n, bh, bw), luma then
+        the two chroma planes as num_planes of params says, uint8 for 8-bit frames or int16 holding uint16 values for
+        high bit depth (as filter_tensors returns them), all views of one buffer whose item i is laid out as a
+        tf_gpu_dump.pred entry; status is an int32 tensor (n,): 0, or TF_GPU_MOTION_REJECTED for an item whose position
+        or ref the kernel rejects (its samples are 0).  Packing and the kernel run in order on the current torch
+        stream of that device, after what is already enqueued there, and the call does not synchronise: read the
+        result on that stream (or after synchronising it).
+        To predict at the MVs of motion_search_tensors' results `res` for the same blocks and refs, set
+        items[:, 2:4] = res[:, 3:5] on that stream.  Predicting the source itself at MV 0 returns the source block,
+        so a residual is source block minus prediction with nothing else to fetch."""
+        import torch
+        if not isinstance(params, dict):
+            raise ValueError("predict_tensors takes the dict form of params (_params.tf_params): it carries the "
+                             "container type and the subsampling that shape the planes")
+        cp = make_params(params)
+        dev = self._torch_device(torch)
+        ids, num_refs, n = predict_device_args(ref_ids, block_size, items, dev)
+        B = block_size
+        shapes = [(B, B)] + ([(B >> params["ss_y"], B >> params["ss_x"])] * 2 if cp.num_planes == 3 else [])
+        num_pels = sum(h * w for h, w in shapes)
+        with torch.cuda.device(dev):
+            packed = pack_motion_items(items) if n else torch.zeros((1, 4), dtype=torch.int32, device=dev)
+            # two bytes per sample whatever params say, so that frames in a 16-bit container never write past it
+            raw = torch.empty((max(n, 1) * num_pels,), dtype=torch.int16, device=dev)
+            status = torch.empty((max(n, 1),), dtype=torch.int32, device=dev)
+            s = torch.cuda.current_stream(dev)
+            self._check(self.lib.tf_gpu_predict_device(self.h, C.byref(cp), ids, num_refs, block_size,
+                                                       packed.data_ptr(), n, raw.data_ptr(), status.data_ptr(),
+                                                       s.cuda_stream))
+            buf = (raw if params["use_hbd"] else raw.view(torch.uint8))[:n * num_pels].view(n, num_pels)
+            planes, off = [], 0
+            for h, w in shapes:
+                planes.append(buf[:, off:off + h * w].view(n, h, w))
+                off += h * w
+            return planes, status[:n]
 
     def device_border(self):
         return self.lib.tf_gpu_device_border()

@@ -95,8 +95,8 @@ struct tf_gpu_ctx {
   cudaEvent_t ev_async_upload = nullptr;      // last tf_gpu_cache_frame_async upload
   bool async_upload_pending = false;
   cudaEvent_t ev_ingest_src = nullptr;        // producer's stream at a tf_gpu_cache_frame_device call
-  cudaEvent_t ev_search_src = nullptr;        // caller's stream at a tf_gpu_motion_search_device call
-  cudaEvent_t ev_search_done = nullptr;       // that call's search on the main stream
+  cudaEvent_t ev_search_src = nullptr;        // caller's stream at a tf_gpu_motion_search_device / tf_gpu_predict_device call
+  cudaEvent_t ev_search_done = nullptr;       // that call's kernel on the main stream
   cudaEvent_t user_ev[4] = { nullptr, nullptr, nullptr, nullptr };
   std::vector<DevFrame> cache;
   DevFrame out;
@@ -1560,24 +1560,27 @@ int check_item_position(tf_gpu_ctx *ctx, const tf_gpu_params &p, int i, int x, i
   return TF_GPU_OK;
 }
 
-// The checks both motion-search entry points make before anything is enqueued or pinned, short of the items (the
-// synchronous call reads them on the host, the device call leaves them to the kernel) and of where items / results
-// live.  n == 0 passes without the frame checks: the caller returns TF_GPU_OK.  Otherwise *p holds the search
-// params, devf[0] the source slot and devf[1 .. num_refs] the reference slots.
-int check_motion_search(tf_gpu_ctx *ctx, const tf_gpu_params *params, uint64_t src_id, const uint64_t *ref_ids,
-                        int num_refs, int block_size, const void *items, int n, const void *results, tf_gpu_params *p,
-                        DevFrame **devf) {
-  if (!params || !ref_ids || !items || !results) return fail(ctx, TF_GPU_ERR_INVALID, "NULL argument");
+// The checks the motion-search and predictor entry points make before anything is enqueued or pinned, short of the
+// items (the synchronous search reads them on the host, the device calls leave them to the kernel) and of where the
+// item and output buffers live.  src_id: the search's source, NULL for the predictor, whose frames are the
+// references alone.  num_planes: the planes the call reads (the search: 1).  n == 0 passes without the frame checks:
+// the caller returns TF_GPU_OK.  Otherwise *p holds the call's params and devf[0 ..] the slots in frame order (the
+// source first, then the references).
+int check_resident_call(tf_gpu_ctx *ctx, const tf_gpu_params *params, const uint64_t *src_id, const uint64_t *ref_ids,
+                        int num_refs, int block_size, int n, int num_planes, tf_gpu_params *p, DevFrame **devf) {
+  if (!params || !ref_ids) return fail(ctx, TF_GPU_ERR_INVALID, "NULL argument");
   if (block_size != 16 && block_size != 32) return fail(ctx, TF_GPU_ERR_INVALID, "block_size must be 16 or 32");
   if (n < 0) return fail(ctx, TF_GPU_ERR_INVALID, "negative item count");
   if (num_refs < 1 || num_refs > TF_GPU_MAX_FRAMES - 1)
     return fail(ctx, TF_GPU_ERR_INVALID, "num_refs %d out of [1,%d]", num_refs, TF_GPU_MAX_FRAMES - 1);
   if (n == 0) return TF_GPU_OK;
-  *p = search_params(*params, 1 + num_refs);
+  const int nsrc = src_id ? 1 : 0;
+  *p = search_params(*params, nsrc + num_refs);
+  p->num_planes = num_planes;
   int rc = validate_params(ctx, p);
   if (rc) return rc;
-  for (int f = 0; f <= num_refs; f++) {
-    const uint64_t id = f ? ref_ids[f - 1] : src_id;
+  for (int f = 0; f < nsrc + num_refs; f++) {
+    const uint64_t id = f < nsrc ? *src_id : ref_ids[f - nsrc];
     devf[f] = find_cached(ctx, id, nullptr);
     if (!devf[f]) return fail(ctx, TF_GPU_ERR_INVALID, "frame id %llu is not resident", (unsigned long long)id);
     if (!(devf[f]->g == devf[0]->g)) return fail(ctx, TF_GPU_ERR_INVALID, "the source and references must share one geometry");
@@ -1585,17 +1588,60 @@ int check_motion_search(tf_gpu_ctx *ctx, const tf_gpu_params *params, uint64_t s
   return validate_geometry(ctx, p, devf[0]->g);
 }
 
-// The search itself, on the main stream, for both entry points: pins the slots for the current epoch (so that
-// done_ev covers the kernel for a later eviction), waits for each slot's upload or ingest, and makes one launch over
-// items / results in device memory; `timed`: ctx->ev0 / ev1 around the launch.
-int enqueue_motion_search(tf_gpu_ctx *ctx, const tf_gpu_params &p, DevFrame *const *devf, int num_refs, int block_size,
-                          const MotionItem *d_items, MotionResult *d_res, int n, bool timed) {
-  for (int f = 0; f <= num_refs; f++) {
+// One caller buffer of a stream-ordered call: `bytes` from `ptr`, `align`-byte aligned.
+struct DeviceSpan {
+  const void *ptr;
+  size_t bytes, align;
+  const char *what;
+};
+// Each buffer is device or managed memory of the context's device with its extent inside its allocation
+// (check_device_extent), and no two overlap.
+int check_device_spans(tf_gpu_ctx *ctx, const DeviceSpan *s, int count) {
+  for (int i = 0; i < count; i++) {
+    const int rc = check_device_extent(ctx, s[i].ptr, s[i].bytes, s[i].align, s[i].what);
+    if (rc) return rc;
+  }
+  for (int i = 0; i < count; i++)
+    for (int j = i + 1; j < count; j++) {
+      const uintptr_t a = (uintptr_t)s[i].ptr, b = (uintptr_t)s[j].ptr;
+      if (a < b + s[j].bytes && b < a + s[i].bytes) return fail(ctx, TF_GPU_ERR_INVALID, "%s and %s overlap", s[i].what, s[j].what);
+    }
+  return TF_GPU_OK;
+}
+
+// Pins the slots for the current epoch (so that done_ev covers the kernels that read them, for a later eviction)
+// and makes the main stream wait for each slot's upload or ingest.
+int pin_slots(tf_gpu_ctx *ctx, DevFrame *const *devf, int count) {
+  for (int f = 0; f < count; f++) {
     DevFrame *d = devf[f];
     if (d->pinned_epoch != ctx->epoch) CU(cudaStreamWaitEvent(ctx->stream, d->ready, 0));
     d->last_use = ++ctx->use_counter;
     d->pinned_epoch = ctx->epoch;
   }
+  return TF_GPU_OK;
+}
+
+// The body of a stream-ordered call: `enqueue` runs on the main stream after the work already on the caller's
+// `stream`, and `stream` waits for it, so that done_ev covers the call's kernel (see get_frame) and the caller may
+// consume the outputs in its own stream order.  Never blocks the host.
+extern "C++" template <class F>
+int on_caller_stream(tf_gpu_ctx *ctx, void *stream, F &&enqueue) {
+  const cudaStream_t s = (cudaStream_t)stream;
+  CU(cudaEventRecord(ctx->ev_search_src, s));
+  CU(cudaStreamWaitEvent(ctx->stream, ctx->ev_search_src, 0));
+  const int rc = enqueue();
+  if (rc) return rc;
+  CU(cudaEventRecord(ctx->ev_search_done, ctx->stream));
+  CU(cudaStreamWaitEvent(s, ctx->ev_search_done, 0));
+  return TF_GPU_OK;
+}
+
+// The search itself, on the main stream, for both entry points: pins the slots, and makes one launch over
+// items / results in device memory; `timed`: ctx->ev0 / ev1 around the launch.
+int enqueue_motion_search(tf_gpu_ctx *ctx, const tf_gpu_params &p, DevFrame *const *devf, int num_refs, int block_size,
+                          const MotionItem *d_items, MotionResult *d_res, int n, bool timed) {
+  const int rc = pin_slots(ctx, devf, 1 + num_refs);
+  if (rc) return rc;
   const Geometry &g = devf[0]->g;
   KParams K;
   fill_kparams(ctx, &p, g, K);
@@ -1682,9 +1728,10 @@ int tf_gpu_motion_search_batch(tf_gpu_ctx *ctx, const tf_gpu_params *params, uin
                 "ABI structs and device structs must agree");
   if (!ctx) return TF_GPU_ERR_INVALID;
   // every check comes before anything is enqueued or pinned: a rejected call leaves the context as it was
+  if (!items || !results) return fail(ctx, TF_GPU_ERR_INVALID, "NULL argument");
   tf_gpu_params p;
   DevFrame *devf[TF_GPU_MAX_FRAMES];
-  int rc = check_motion_search(ctx, params, src_id, ref_ids, num_refs, block_size, items, n, results, &p, devf);
+  int rc = check_resident_call(ctx, params, &src_id, ref_ids, num_refs, block_size, n, 1, &p, devf);
   if (rc || n == 0) return rc;
   for (int i = 0; i < n; i++) {
     rc = check_item_position(ctx, p, i, items[i].x, items[i].y);
@@ -1718,31 +1765,81 @@ int tf_gpu_motion_search_device(tf_gpu_ctx *ctx, const tf_gpu_params *params, ui
   static_assert(TF_GPU_MOTION_REJECTED == MOTION_REJECTED, "header and kernel must agree on the rejection sentinel");
   if (!ctx) return TF_GPU_ERR_INVALID;
   // every check comes before anything is enqueued or pinned: a rejected call leaves the context as it was
+  if (!items || !results) return fail(ctx, TF_GPU_ERR_INVALID, "NULL argument");
   tf_gpu_params p;
   DevFrame *devf[TF_GPU_MAX_FRAMES];
-  int rc = check_motion_search(ctx, params, src_id, ref_ids, num_refs, block_size, items, n, results, &p, devf);
+  int rc = check_resident_call(ctx, params, &src_id, ref_ids, num_refs, block_size, n, 1, &p, devf);
   if (rc || n == 0) return rc;
   CU(cudaSetDevice(ctx->device));
   const size_t bytes = (size_t)n * sizeof(MotionItem);
-  rc = check_device_extent(ctx, items, bytes, 4, "items");
+  const DeviceSpan spans[2] = { { items, bytes, 4, "items" }, { results, bytes, 4, "results" } };
+  rc = check_device_spans(ctx, spans, 2);
   if (rc) return rc;
-  rc = check_device_extent(ctx, results, bytes, 4, "results");
-  if (rc) return rc;
-  const uintptr_t a = (uintptr_t)items, b = (uintptr_t)results;
-  if (a < b + bytes && b < a + bytes) return fail(ctx, TF_GPU_ERR_INVALID, "items and results overlap");
   CallScope scope(ctx);
   ctx->last_launches = 0;
   ctx->last_kernel_ms = 0.f;  // not timed: the call does not wait for the kernel
-  // on the main stream between the caller's stream and back, so that done_ev covers the search (see get_frame)
-  const cudaStream_t s = (cudaStream_t)stream;
-  CU(cudaEventRecord(ctx->ev_search_src, s));
-  CU(cudaStreamWaitEvent(ctx->stream, ctx->ev_search_src, 0));
-  rc = enqueue_motion_search(ctx, p, devf, num_refs, block_size, (const MotionItem *)items, (MotionResult *)results, n,
-                             false);
+  return on_caller_stream(ctx, stream, [&]() -> int {
+    return enqueue_motion_search(ctx, p, devf, num_refs, block_size, (const MotionItem *)items, (MotionResult *)results,
+                                 n, false);
+  });
+}
+
+// Far MVs (tf_predict_kernel): the origin clamp is exact when every plane's border covers a sub-block's 12-tap
+// footprint plus the load margins: b >= w + 11 + PRED_ML + PRED_MR, w <= 16 >> ss, b = DEV_BORDER >> ss.
+static_assert(DEV_BORDER >= 16 + 11 + PRED_ML + PRED_MR && (DEV_BORDER >> 1) >= 8 + 11 + PRED_ML + PRED_MR,
+              "the device border must hold a far-MV predictor footprint");
+
+int tf_gpu_predict_device(tf_gpu_ctx *ctx, const tf_gpu_params *params, const uint64_t *ref_ids, int num_refs,
+                          int block_size, const tf_gpu_predict_item *items, int n, void *pred, int32_t *status,
+                          void *stream) {
+  static_assert(sizeof(tf_gpu_predict_item) == sizeof(tf_gpu_motion_item) &&
+                    offsetof(tf_gpu_predict_item, row) == offsetof(tf_gpu_motion_item, start_row) &&
+                    offsetof(tf_gpu_predict_item, col) == offsetof(tf_gpu_motion_item, start_col) &&
+                    offsetof(tf_gpu_predict_item, ref) == offsetof(tf_gpu_motion_item, ref),
+                "a predictor item has the layout of a motion-search item");
+  static_assert(sizeof(tf_gpu_predict_item) == sizeof(PredictItem), "ABI struct and device struct must agree");
+  if (!ctx) return TF_GPU_ERR_INVALID;
+  // every check comes before anything is enqueued or pinned: a rejected call leaves the context as it was
+  if (!items || !pred || !status) return fail(ctx, TF_GPU_ERR_INVALID, "NULL argument");
+  tf_gpu_params p;
+  DevFrame *devf[TF_GPU_MAX_FRAMES];
+  int rc = check_resident_call(ctx, params, nullptr, ref_ids, num_refs, block_size, n, params ? params->num_planes : 0,
+                               &p, devf);
+  if (rc || n == 0) return rc;
+  CU(cudaSetDevice(ctx->device));
+  const Geometry &g = devf[0]->g;
+  const size_t es = g.is_hbd ? 2 : 1;
+  const int num_pels =
+      block_size * block_size + (p.num_planes > 1 ? 2 * (block_size >> g.ss_x) * (block_size >> g.ss_y) : 0);
+  const DeviceSpan spans[3] = { { items, (size_t)n * sizeof(PredictItem), 4, "items" },
+                                { pred, (size_t)n * num_pels * es, es, "pred" },
+                                { status, (size_t)n * sizeof(int32_t), 4, "status" } };
+  rc = check_device_spans(ctx, spans, 3);
   if (rc) return rc;
-  CU(cudaEventRecord(ctx->ev_search_done, ctx->stream));
-  CU(cudaStreamWaitEvent(s, ctx->ev_search_done, 0));
-  return TF_GPU_OK;
+  CallScope scope(ctx);
+  ctx->last_launches = 0;
+  ctx->last_kernel_ms = 0.f;  // not timed: the call does not wait for the kernel
+  return on_caller_stream(ctx, stream, [&]() -> int {
+    const int rc2 = pin_slots(ctx, devf, num_refs);
+    if (rc2) return rc2;
+    KParams K;
+    fill_kparams(ctx, &p, g, K);
+    K.num_pels = num_pels;
+    // frames past the references are the first reference's: a wrong ref check could not reach a null pointer
+    for (int f = 0; f < MAXF; f++)
+      for (int pl = 0; pl < p.num_planes; pl++) K.frm[f][pl] = devf[f < num_refs ? f : 0]->p00[pl];
+    const long long grid = block_size == 32 ? n : ((long long)n + FILT_WARPS - 1) / FILT_WARPS;
+    const PredictItem *d_items = (const PredictItem *)items;
+    if (g.is_hbd)
+      tf_predict_kernel<uint16_t><<<(unsigned)grid, FILT_THREADS, 0, ctx->stream>>>(
+          K, d_items, (uint16_t *)pred, status, n, block_size, g.bx[1], g.by[1], g.bx[0]);
+    else
+      tf_predict_kernel<uint8_t><<<(unsigned)grid, FILT_THREADS, 0, ctx->stream>>>(
+          K, d_items, (uint8_t *)pred, status, n, block_size, g.bx[1], g.by[1], g.bx[0]);
+    CU(cudaGetLastError());
+    ctx->last_launches++;
+    return TF_GPU_OK;
+  });
 }
 
 int tf_gpu_host_register(tf_gpu_ctx *ctx, void *ptr, size_t bytes) {

@@ -1884,6 +1884,19 @@ __device__ __noinline__ void convolve12_packed(const KParams &P, const uint16_t 
 constexpr int FILT_WARPS = 4;
 constexpr int FILT_THREADS = FILT_WARPS * 32;
 
+// The scaled source position of one predictor sub-block: init_subpel_params (reconinter.h:131-165) as
+// tf_build_predictor (temporal_filter.c:356-365) calls it for the sub-block at plane position (y, x), with the
+// reference's clamp to [-((288 >> ss) - 4), aligned + 4] samples.  Integer sample: pos >> 10; 1/16 phase:
+// (pos & 1023) >> 6.
+__device__ __forceinline__ void predictor_position(const KParams &P, int k, int y, int x, MV2 mv, int ssy, int ssx,
+                                                   int *py, int *px) {
+  int pos_y = ((y << 4) + mv.row * (1 << (1 - ssy))) * 64 + 32;
+  int pos_x = ((x << 4) + mv.col * (1 << (1 - ssx))) * 64 + 32;
+  const int top = -(((288 >> ssy) - 4) << 10), left = -(((288 >> ssx) - 4) << 10);
+  *py = iclamp(pos_y, top, (P.aligned_h[k] + 4) << 10);
+  *px = iclamp(pos_x, left, (P.aligned_w[k] + 4) << 10);
+}
+
 template <typename T>
 __device__ void build_predictor(const KParams &P, const T *const ref[3], int mb_row, int mb_col, const MV2 *mvs,
                                 T *pred, int16_t *im /* this warp's scratch */) {
@@ -1897,12 +1910,8 @@ __device__ void build_predictor(const KParams &P, const T *const ref[3], int mb_
     const int plane_y = (32 * mb_row) >> ssy, plane_x = (32 * mb_col) >> ssx;
     const int h = plane_h >> 1, w = plane_w >> 1;
     const int i = (q >> 1) * h, j = (q & 1) * w;
-    const int y = plane_y + i, x = plane_x + j;
-    int pos_y = ((y << 4) + mv.row * (1 << (1 - ssy))) * 64 + 32;
-    int pos_x = ((x << 4) + mv.col * (1 << (1 - ssx))) * 64 + 32;
-    const int top = -(((288 >> ssy) - 4) << 10), left = -(((288 >> ssx) - 4) << 10);
-    pos_y = iclamp(pos_y, top, (P.aligned_h[k] + 4) << 10);
-    pos_x = iclamp(pos_x, left, (P.aligned_w[k] + 4) << 10);
+    int pos_y, pos_x;
+    predictor_position(P, k, plane_y + i, plane_x + j, mv, ssy, ssx, &pos_y, &pos_x);
     const T *src = ref[plane] + (pos_y >> 10) * P.pitch[k] + (pos_x >> 10);
     const int sxp = (pos_x & 1023) >> 6, syp = (pos_y & 1023) >> 6;
     if constexpr (sizeof(T) == 2) {
@@ -2202,6 +2211,83 @@ __device__ __forceinline__ void filter_block(const KParams &P, const unsigned bi
 template <typename T>
 __global__ void __launch_bounds__(FILT_THREADS, TF_FILT_MINB) tf_filter_kernel(const __grid_constant__ KParams P) {
   filter_block<T>(P, blockIdx.x);
+}
+
+// ---------------------------------------------------------------------------
+// Predictor at caller MVs (tf_gpu_predict_device): what build_predictor makes of one 16x16 luma unit and its chroma
+// sub-blocks, for an item of size 16 or one quadrant of an item of size 32 (each quadrant at the item's MV, from its
+// own origin, as the filter predicts a block it did not split).  One warp per unit, FILT_WARPS warps per CTA: an item
+// of size 32 is one CTA, warp q its quadrant q; items of size 16 are four to a CTA.  Frame r of P is ref_ids[r].
+//
+// Far MVs: the reference's clamp lets the origin reach 284 samples (luma) above / left of the frame, past the slot's
+// border b.  Each axis of the origin is first clamped to [-b + 5 + PRED_ML, aligned + b - w - 6 - PRED_MR], w the
+// sub-block's extent on that axis.  The 12-tap footprint of origin s is [s - 5, s + w + 6); the convolve routines'
+// loads reach PRED_ML samples before and PRED_MR after it (convolve12_packed's aligned word loads: a row starts at
+// most one sample early, and 8 words from there end at most 3 samples late; convolve12 and the vertical taps read
+// the footprint exactly).  When the clamp moves an origin, both footprints lie in the edge-replicated region of that
+// axis (x <= 0 or x >= aligned - 1 >= crop - 1) because b >= w + 11 + PRED_ML + PRED_MR, so every sample the
+// convolve reads is the one it would read on an unbounded border; every load stays inside the slot, so the __ldg
+// loads only ever see the slot's global memory.
+// Each sub-block is built in shared memory, as in the filter, and then copied out: the convolve routines get the same
+// kinds of pointers from every caller, so adding this caller leaves the filter kernels' code as it was (a direct
+// store to `pred` changed their register allocation).
+// Rejected items (position rule of item_position_ok, or ref outside [0, num_frames)) get MOTION_REJECTED and zeros.
+// ---------------------------------------------------------------------------
+constexpr int PRED_ML = 1, PRED_MR = 3;
+constexpr int PRED_UNIT_PELS = 16 * 16;  // one sub-block of one plane, staged in shared memory
+struct PredictItem {
+  int x, y;
+  int16_t row, col;
+  int32_t ref;
+};
+template <typename T>
+__global__ void __launch_bounds__(FILT_THREADS) tf_predict_kernel(const __grid_constant__ KParams P, const PredictItem *items,
+                                                                  T *pred, int32_t *status, int n, int bsize,
+                                                                  int border_x_uv, int border_y_uv, int border_luma) {
+  __shared__ __align__(16) int16_t im_all[FILT_WARPS * FILT_IM];
+  __shared__ __align__(16) T stage_all[FILT_WARPS * PRED_UNIT_PELS];
+  const int warp = threadIdx.x >> 5, lane = lane_id();
+  const int q = bsize == 32 ? warp : 0;
+  const long long item = bsize == 32 ? (long long)blockIdx.x : (long long)blockIdx.x * FILT_WARPS + warp;
+  if (item >= n) return;
+  const PredictItem it = items[item];
+  const bool ok = item_position_ok(it.x, it.y, P.mi_rows, P.mi_cols) && it.ref >= 0 && it.ref < P.num_frames;
+  if (q == 0 && lane == 0) status[item] = ok ? 0 : MOTION_REJECTED;
+  const MV2 mv = { (int)it.row, (int)it.col };
+  T *out = pred + (size_t)item * P.num_pels;
+  int16_t *im = im_all + warp * FILT_IM;
+  T *stage = stage_all + warp * PRED_UNIT_PELS;
+  int plane_offset = 0;
+  for (int plane = 0; plane < P.num_planes; plane++) {
+    const int ssy = plane ? P.ss_y : 0, ssx = plane ? P.ss_x : 0;
+    const int k = plane > 0;
+    const int plane_h = bsize >> ssy, plane_w = bsize >> ssx;
+    const int h = 16 >> ssy, w = 16 >> ssx;
+    const int i = (q >> 1) * h, j = (q & 1) * w;
+    if (ok) {
+      int pos_y, pos_x;
+      predictor_position(P, k, (it.y >> ssy) + i, (it.x >> ssx) + j, mv, ssy, ssx, &pos_y, &pos_x);
+      const int by = k ? border_y_uv : border_luma, bx = k ? border_x_uv : border_luma;
+      const int oy = iclamp(pos_y >> 10, -by + 5 + PRED_ML, P.aligned_h[k] + by - h - 6 - PRED_MR);
+      const int ox = iclamp(pos_x >> 10, -bx + 5 + PRED_ML, P.aligned_w[k] + bx - w - 6 - PRED_MR);
+      const T *src = reinterpret_cast<const T *>(P.frm[it.ref][plane]) + oy * P.pitch[k] + ox;
+      const int sxp = (pos_x & 1023) >> 6, syp = (pos_y & 1023) >> 6;
+      if constexpr (sizeof(T) == 2) {
+        if (sxp | syp) convolve12_packed(P, src, P.pitch[k], stage, w, w, h, sxp, syp, im);
+        else convolve12<T>(P, src, P.pitch[k], stage, w, w, h, 0, 0, im);
+      } else {
+        convolve12<T>(P, src, P.pitch[k], stage, w, w, h, sxp, syp, im);
+      }
+      __syncwarp();
+    }
+    T *dst = out + plane_offset + i * plane_w + j;
+    const int wsh = 4 - ssx;  // w = 1 << wsh
+#pragma unroll
+    for (int e = lane; e < PRED_UNIT_PELS; e += 32)
+      if (e < h * w) dst[(e >> wsh) * plane_w + (e & (w - 1))] = ok ? stage[e] : (T)0;
+    __syncwarp();
+    plane_offset += plane_h * plane_w;
+  }
 }
 
 // ---------------------------------------------------------------------------

@@ -330,6 +330,53 @@ int tf_gpu_motion_search_device(tf_gpu_ctx *ctx, const tf_gpu_params *params, ui
                                 const tf_gpu_motion_item *items /* device */, int n,
                                 tf_gpu_motion_result *results /* device */, void *stream);
 
+/* The temporal filter's motion-compensated predictor (tf_build_predictor, temporal_filter.c:328-390: MULTITAP_SHARP2
+ * 12-tap kernels, bit-exact) at caller MVs, with items and outputs in DEVICE (or managed) memory of the context's
+ * device: what a block looks like at the MV a motion search returned, for a consumer that weighs, compares or
+ * visualises blocks or computes a residual on the GPU.  Chain from tf_gpu_motion_search_device by copying each
+ * result's row / col into the item (same layout as tf_gpu_motion_item, start_row / start_col -> row / col).
+ * Every item is one block at luma position (x, y) of the resident frame ref_ids[item.ref], MV (row, col) in 1/8 pel;
+ * its prediction is what tf_build_predictor makes with four equal sub-block MVs:
+ *   block_size 16: one 16x16 luma sub-block and its (16 >> ss_x) x (16 >> ss_y) chroma sub-blocks, each built as the
+ *     filter builds one quadrant: init_subpel_params position ((y << 4) + mv * (1 << (1 - ss))) * 64 + 32, clamped to
+ *     [-(((288 >> ss) - 4) << 10), (aligned + 4) << 10], then the 12-tap convolve (copy, 1-D and 2-D rounding at
+ *     8, 10 and 12 bit);
+ *   block_size 32: the four 16x16 quadrants, each at the item's MV and each clamped from its own origin -- the
+ *     filter's predictor of a 32x32 block it did not split.  This differs from one 32x32
+ *     av1_enc_build_one_inter_predictor call only where the position clamp engages, which the MV limits of the motion
+ *     search never allow: for every MV the search returns, the two readings agree.
+ * Every int16 MV is defined: the result equals the reference's predictor on a frame whose edge-replicated border
+ * (av1_copy_and_extend_frame's replication from the crop edge) is wide enough for the read.  The device border is
+ * narrower than the reference clamp lets an origin go (284 luma samples above / left), so the library moves an
+ * origin that lies deeper in the border than the 12-tap footprint needs towards the frame, which changes no sample read.
+ * Output: item i's samples at pred + i * num_pels, num_pels = B^2 + 2 * (B >> ss_x) * (B >> ss_y) (B^2 for
+ * num_planes 1), in the layout of tf_gpu_dump.pred (plane_offset + row * plane_w + col): one item compares directly
+ * with a dump entry.  Samples are the frames' container type: uint8_t for 8-bit frames, uint16_t for high bit depth.
+ * Predicting the source itself at MV 0 gives the source block.
+ * Of `params` the fields bit_depth, num_planes (1 or 3) and mi_rows / mi_cols (the position rule) are read; they
+ * are validated as tf_gpu_motion_search_device validates them.  Ordering and lifetime are those of
+ * tf_gpu_motion_search_device: the kernel runs after the work already on `stream`, on the context's stream (so also
+ * behind a filter call already submitted on this context), and `stream` waits for it before the call returns;
+ * slots read by a queued call keep their frames until it has run.  Never blocks the host.
+ * TF_GPU_ERR_INVALID, with nothing enqueued and the context unchanged, for a NULL pointer, block_size other than 16
+ * or 32, n < 0, num_refs outside [1, TF_GPU_MAX_FRAMES - 1], an id that is not resident, frames of different
+ * geometry, num_planes 3 on frames without chroma, a bit_depth the container cannot hold, items / pred / status
+ * that are not device or managed memory of the context's device, not aligned (4, the sample size, 4), or whose
+ * extent (n * 16 bytes, n * num_pels samples, n * 4 bytes) runs past their allocation, and any two of the three that
+ * overlap.  n == 0 returns TF_GPU_OK with nothing enqueued.  The kernel checks each item against the position rule
+ * of tf_gpu_motion_search_batch (x a multiple of 16, y of 4, inside the mi grid) and 0 <= ref < num_refs: a rejected
+ * item gets status TF_GPU_MOTION_REJECTED and all its samples 0, every other item status 0.  tf_gpu_last_stats
+ * reports one launch and a kernel time of 0. */
+typedef struct {
+  int x, y;          /* luma position of the block's top-left sample */
+  int16_t row, col;  /* MV, 1/8 pel */
+  int32_t ref;       /* index into ref_ids */
+} tf_gpu_predict_item;
+int tf_gpu_predict_device(tf_gpu_ctx *ctx, const tf_gpu_params *params, const uint64_t *ref_ids /* host */,
+                          int num_refs, int block_size, const tf_gpu_predict_item *items /* device */, int n,
+                          void *pred /* device, n * num_pels samples */, int32_t *status /* device, n */,
+                          void *stream);
+
 /* Pinned host memory helpers so lookahead buffers can be DMA'd directly. */
 int tf_gpu_host_register(tf_gpu_ctx *ctx, void *ptr, size_t bytes);
 int tf_gpu_host_unregister(tf_gpu_ctx *ctx, void *ptr);
